@@ -2,7 +2,7 @@
 """Benchmark of the PMR446 receive chain on B200 (BASELINE.json metric: IQ Msamples/s through the
 full chain + roofline fraction).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2]; configs[4] is the same shard per GPU at N = 8): a batch of
 STREAMS = 1024 independent 2.4 Msps cu8 PMR446 captures per GPU, all 16 channels demodulated to s16
@@ -12,7 +12,7 @@ steps).  Filter state carries from step to step exactly as in streaming use.
 
   value     device-resident throughput: inputs already in HBM, s16 audio left in HBM; K steps timed with
             CUDA events on the launch stream between barriers, max over ranks.
-  e2e       the same K steps through the host-buffer C-ABI call pmr446_batch_execute(): pinned host IQ
+  e2e       K more steps through the host-buffer C-ABI call pmr446_batch_execute(): pinned host IQ
             -> H2D -> chain -> D2H of the s16 audio, copies inside the timed region.
   roofline  the kernel with the longest launch, timed live with CUDA events inside the timed steps: algorithmic
             bytes / measured HBM peak and algorithmic flop / measured FP32 FFMA peak, reported for the roofline that
@@ -21,6 +21,9 @@ steps).  Filter state carries from step to step exactly as in streaming use.
 
 --impl reference times the reference's CPU chain (the oracle port -- the reference itself cannot be
 built here, see DESIGN.md) on the host cores with the same config/metric.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned as DIR/<name>.npy in float32
+(see dump_outputs).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -84,16 +87,18 @@ def make_base_captures(count, n):
     return [synth.make_cu8(synth.CaptureSpec(fs=float(FS), carriers=synth.rotated_carriers(s)), n, 446 + s) for s in range(count)]
 
 
-def cpu_chain_rate(threads, seconds_of_signal, active_only=-1):
+def cpu_chain_rate(threads, seconds_of_signal, active_only=-1, last=None):
     """Oracle (CPU port of the reference chain) on `threads` host threads, one stream each.  Returns
-    (Msamples/s aggregate, wall seconds)."""
+    (Msamples/s aggregate, wall seconds); `last`, a dict, receives each thread's s16 audio of its last chunk."""
     from oracle import oracle as orc
     base = make_base_captures(min(threads, 4), CHUNK)
     objs = [orc.PmrOracle(fs_in=FS, in_fmt=1, audio_gain=1.0, chunk=CHUNK, active_only=active_only) for _ in range(threads)]
 
     def work(i):
         for _ in range(seconds_of_signal):
-            objs[i].execute(base[i % len(base)], want=("pcm",))
+            r = objs[i].execute(base[i % len(base)], want=("pcm",))
+        if last is not None:
+            last[i] = r["pcm"]
 
     ths = [threading.Thread(target=work, args=(i,)) for i in range(threads)]
     t0 = time.perf_counter()
@@ -159,7 +164,7 @@ def measured_peaks():
 
 # ------------------------------------------------------------------------------------------------
 def reference_binary_rate(cores):
-    """The UNMODIFIED reference program (oracle/_ref/sdr_pmr446_ref, built by oracle/ref.mk from /root/reference/src with
+    """The UNMODIFIED reference program (oracle/_ref/sdr_pmr446_ref, built by `make -f oracle/ref.mk REF=<checkout>` with
     file-backed SoapySDR / RtAudio stand-ins) on `cores` processes, each on a 10 s capture at the ONE configuration it
     supports: 1.024 Msps hard-coded, one squelch-selected channel demodulated.  Informational (another config than the
     bench line); None when the binary was not built."""
@@ -191,10 +196,13 @@ def run_reference(args, rank, world):
     cores = os.cpu_count() or 1
     secs = 4
     vals = []
+    last = {}
     for it in range(args.warmup + args.steps):
-        v, dt = cpu_chain_rate(cores, secs)
+        v, dt = cpu_chain_rate(cores, secs, last=last)
         if it >= args.warmup:
             vals.append((v, dt))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pcm": np.stack([last[i] for i in range(cores)])})
     value = float(np.mean([v for v, _ in vals]))
     ms = float(np.mean([dt for _, dt in vals]) * 1e3)
     sample = "%d host threads x %d s of one 2.4 Msps stream each per step (all 16 channels demodulated)" % (cores, secs)
@@ -271,6 +279,21 @@ def pcie_topology(local_rank):
     return info
 
 
+DUMP_STREAMS = 64   # the largest dump, 64 streams x 16 channels x 12500 samples of audio in float32, is 51 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array (numpy or torch, one stream per row) as out_dir/<name>.npy in float32, reduced to a fixed sample
+    of DUMP_STREAMS rows drawn with seed 0, in increasing order (every row when there are fewer)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        S = a.shape[0]
+        pick = np.sort(np.random.default_rng(0).choice(S, min(S, DUMP_STREAMS), replace=False))
+        a = a[torch.from_numpy(pick).to(a.device)].cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)[pick]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -314,6 +337,7 @@ def run_ours(args, rank, world, local_rank):
 
     # ---------------- device-resident arm ("value") ----------------
     launches = 0
+    ns = 0
     # ranks finish their set-up (synthetic captures, pinned buffers) seconds apart: meet BEFORE the warm-up, so that no GPU sits idle --
     # and drops its clocks -- between its warm-up steps and the timed region (seen at 8 GPUs: three ranks at 4.2-4.4 ms, five at 4.10)
     barrier()
@@ -326,7 +350,7 @@ def run_ours(args, rank, world, local_rank):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        batch.execute_device(iq_dev, n, outs)
+        _, ns = batch.execute_device(iq_dev, n, outs)
         launches += batch.last_launches
     e1.record()
     barrier()
@@ -334,6 +358,8 @@ def run_ours(args, rank, world, local_rank):
     timings = batch.get_timings()
     batch.timing(False)
     checksum = int(pcm_dev[:, :, :12500].to(torch.int64).abs().sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pcm": pcm_dev[:, :, :ns]})
 
     # ---------------- PCIe probe: what the end-to-end arm can at best reach on this rank, all ranks copying at once ----
     barrier()
@@ -350,7 +376,7 @@ def run_ours(args, rank, world, local_rank):
     o = Outputs()
     o.ld, o.res_ld, o.pcm = ld, batch.max_res, pcm_host.ctypes.data
     ny, ns = C.c_uint(0), C.c_uint(0)
-    e2e_steps = max(1, min(args.steps, 5))
+    e2e_steps = args.steps
 
     def e2e_step():
         check(lib().pmr446_batch_execute(batch.h, iq_np.ctypes.data, iq_np.strides[0], n, C.byref(o), C.byref(ny), C.byref(ns)),
@@ -529,6 +555,7 @@ def run_other(args, name):
             outs.update(ascii=torch.empty((S, 1600), dtype=torch.uint8, device=dev), peak=torch.empty((S, 2), dtype=torch.float32, device=dev))
         view = iq_dev.view(torch.float32).view(S, -1) if kind == "wide" else iq_dev
         dev_step = lambda: obj.execute_device(view, n, outs)
+        dump = lambda r: dict(pcm=outs["pcm"][:, :, :r[1]], **{k: outs[k] for k in ("ascii", "peak") if k in outs})
         pcm_host = torch.zeros((S, M, obj.max_ns), dtype=torch.int16).pin_memory()
         o = _lib.Outputs()
         o.ld, o.res_ld, o.pcm = obj.max_ns, obj.max_res, pcm_host.data_ptr()
@@ -545,6 +572,7 @@ def run_other(args, name):
         obj = chain.DsdBatch(n_streams=S, fs_in=fs, in_fmt=1, max_chunk=n)
         pcm = torch.empty((S, obj.max_out), dtype=torch.int16, device=dev)
         dev_step = lambda: obj.execute_device(iq_dev, n, pcm=pcm)
+        dump = lambda r: {"pcm": pcm[:, :r[1]]}
         pcm_host = torch.zeros((S, obj.max_out), dtype=torch.int16).pin_memory()
         o = _lib.DsdOutputs()
         o.res_ld, o.out_ld, o.pcm = obj.max_res, obj.max_out, pcm_host.data_ptr()
@@ -560,6 +588,13 @@ def run_other(args, name):
               "status": torch.empty((S, C.sizeof(_lib.RxStatus)), dtype=torch.uint8, device=dev),
               "rssi": torch.empty((S, 16), dtype=torch.float32, device=dev)}
         dev_step = lambda: obj.execute_device(iq_dev, n, ro)
+
+        def dump(ns):
+            st = (_lib.RxStatus * S).from_buffer_copy(ro["status"].cpu().numpy().tobytes())
+            fields = {"status_" + k: np.array([getattr(x, k) for x in st]) for k in chain.PmrReceiver.STATUS_FIELDS}
+            pcm = ro["pcm"][:, :ns].cpu().numpy()
+            pcm[np.arange(ns)[None, :] >= fields["status_n_audio"][:, None]] = 0   # a stream's audio ends at its n_audio
+            return dict(pcm=pcm, rssi=ro["rssi"], **fields)
         pcm_host = torch.zeros((S, obj.max_ns), dtype=torch.int16).pin_memory()
         status = (_lib.RxStatus * S)()
         rssi_h = np.zeros((S, 16), np.float32)
@@ -579,12 +614,14 @@ def run_other(args, name):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        dev_step()
+        last = dev_step()
     e1.record()
     torch.cuda.synchronize()
     step_ms = e0.elapsed_time(e1) / args.steps
     launches = getattr(obj, "last_launches", 0) * args.steps
-    e2e_steps = max(1, min(args.steps, 3))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dump(last))
+    e2e_steps = args.steps
     host_step()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
@@ -656,7 +693,13 @@ def main():
                     help="weak (default): 1024 streams per GPU; strong: 8192 streams in total sharded over the GPUs (BASELINE configs[4])")
     ap.add_argument("--config", default="cfg3", choices=["cfg3"] + sorted(OTHER),
                     help="cfg3 (default) = BASELINE configs[2], the judged line; the others are the remaining BASELINE configurations (1 GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (the s16 audio; for --config cfg4 also the waterfall, for "
+                         "--config receiver also the status and RSSI) to DIR/<name>.npy as float32: a fixed sample of %d streams, rank 0's "
+                         "with several GPUs" % DUMP_STREAMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

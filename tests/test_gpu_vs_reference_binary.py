@@ -1,10 +1,10 @@
-"""The CUDA receiver against THE REFERENCE PROGRAM ITSELF: oracle/_ref/sdr_pmr446_ref is the unmodified
-/root/reference/src/sdr_pmr446.c + shared.c (file-backed SoapySDR / RtAudio stand-ins, oracle/ref.mk) -- its played audio,
+"""The CUDA receiver against THE REFERENCE PROGRAM ITSELF: oracle/_ref/sdr_pmr446_ref is the unmodified upstream
+src/sdr_pmr446.c + shared.c (file-backed SoapySDR / RtAudio stand-ins, oracle/ref.mk) -- its played audio,
 tune / detune / channel-change and CTCSS log lines are compared DIRECTLY with pmr446_receiver_execute()'s outputs, without
 oracle/receiver.c in between.  The same for dsd_in: its stdout s16 stream against dsd446_batch_execute().
 
-The binaries are built in the build container (/root/reference is absent on the GPU box; oracle/_ref/ travels with the
-snapshot); the tests skip when they are missing."""
+The repository does not contain the reference's sources: build the binaries with `make -f oracle/ref.mk REF=<checkout>`;
+the tests skip while they are missing."""
 import os
 import re
 import subprocess
@@ -24,7 +24,7 @@ REF = os.path.join(ROOT, "oracle", "_ref")
 def _exe(name):
     path = os.path.join(REF, name)
     if not os.path.exists(path):
-        pytest.skip("oracle/_ref/%s was not built (make -f oracle/ref.mk needs /root/reference)" % name)
+        pytest.skip("oracle/_ref/%s is not built (make -f oracle/ref.mk REF=<checkout of the upstream sdr_pmr446>)" % name)
     return path
 
 

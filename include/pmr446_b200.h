@@ -48,7 +48,8 @@ typedef struct {
   int device;              /* CUDA device ordinal; -1 = current device */
   unsigned fs_in;          /* input sample rate, Hz (SDR_SAMPLERATE, include/sdr_pmr446.h:13) */
   int in_fmt;              /* PMR446_FMT_* */
-  unsigned num_channels;   /* NUM_CHANNELS, src/sdr_pmr446.c:23 (16) */
+  unsigned num_channels;   /* NUM_CHANNELS, src/sdr_pmr446.c:23 (16); any M in [2, 4096] whose generic channelizer
+                              (56 M bytes of shared memory) fits the device's opt-in per-block limit (all of them on a B200) */
   unsigned channel_width;  /* CHANNEL_WIDTH_HZ, :22 (12500) */
   unsigned pfb_m;          /* firpfbch_crcf_create_kaiser semi-length, :437 (13) */
   float pfb_as;            /* ... stop-band attenuation, :437 (80 dB) */
@@ -63,7 +64,9 @@ typedef struct {
   unsigned hp_len;
   const float *lp_taps;    /* audio low-pass FIR, NULL = the reference's 103 taps (:106-119) */
   unsigned lp_len;
-  float deemph_b0, deemph_b1, deemph_a1; /* :461-463 */
+  float deemph_b0, deemph_b1, deemph_a1; /* :461-463; y = b0 x + b1 x[-1] - a1 y[-1].  Any |a1| < 1 whose warm-up
+                              k = ceil(log(2^-30) / log|a1|) fits an audio tile: |a1| <= 0.977 with the low-pass, 0.979
+                              without; create() refuses other poles with PMR446_EINVAL */
   int deemph_fir;          /* APP_FIR_DEEMPH build of the reference: the 101-tap FIR de-emphasis (:122-135, :458, :896)
                               instead of the one-pole filter; served by the fast-convolution audio kernel only
                               (batch API; composite responses up to 1000 taps) */

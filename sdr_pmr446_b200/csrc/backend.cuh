@@ -8,6 +8,7 @@
 // configurations whose composite impulse response does not fit the FFT tile.
 #pragma once
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 
 #include "audio_fft.cuh"   // pcm_sat
@@ -42,6 +43,7 @@ struct AudioParams {
   float* lpcomp;           // optional [rows][out_ld]
   long long out_ld;
   long long lpcomp_ld;     // row stride of lpcomp; 0 = out_ld
+  int de_warm;             // audio_kernel<true>: de-emphasis warm-up per thread (deemph_warmup(de_a1)); lead >= de_warm
 };
 
 constexpr int AU_THREADS = 128;
@@ -49,6 +51,26 @@ constexpr int AU_SPAN = AU_THREADS * 16;   // outputs computed per tile (incl. l
 constexpr int AU_LEAD_LP = 128;            // lead-in with the 103-tap low-pass (>= 112 + 8)
 constexpr int AU_LEAD_MIN = 16;            // lead-in without it (de-emphasis warm-up of 8)
 constexpr int AU_MAXHALO = 384;            // >= padded HP length
+constexpr int AU_MAXLEAD = AU_SPAN / 2;    // longest lead-in a tile may spend on de-emphasis warm-up
+
+// Samples after which the one-pole de-emphasis has forgotten a state dropped at the start of a span to 2^-30 of its value:
+// the least k with |a1|^k <= 2^-30.  -1 if the pole does not decay (|a1| >= 1).
+inline int deemph_warmup(double a1) {
+  const double m = fabs(a1);
+  if (!(m < 1.0)) return -1;
+  if (m < 0x1p-30) return 1;
+  return (int)ceil(log(0x1p-30) / log(m));
+}
+
+// Lead-in of an audio_kernel tile: every stored output sees the low-pass span (16 lp_chunks - 1 with the low-pass) of
+// de-emphasis outputs, each warmed up over `warm` samples inside the tile.  The reference's pole (warm-up 5) keeps
+// AU_LEAD_MIN / AU_LEAD_LP.  -1 if the warm-up does not fit (lead > AU_MAXLEAD).
+inline int audio_lead(bool lowpass, int lp_chunks, int warm) {
+  const int base = lowpass ? AU_LEAD_LP : AU_LEAD_MIN;
+  const int need = ((lowpass ? 16 * lp_chunks - 1 : 0) + warm + 15) / 16 * 16;
+  const int lead = need > base ? need : base;
+  return lead > AU_MAXLEAD ? -1 : lead;
+}
 
 __device__ __forceinline__ int padidx(int i) { return i + (i >> 4); }
 
@@ -90,6 +112,9 @@ __device__ __forceinline__ void fir16(const float* __restrict__ xs, const float*
   if (kb < chunks) step(wa, wb, kb);
 }
 
+// LONG_POLE = false: the de-emphasis state of each thread's 16 outputs is rebuilt from 8 samples of warm-up (pole
+// magnitude up to 0.074 for 2^-30); true: from p.de_warm samples, for poles that decay more slowly.
+template <bool LONG_POLE>
 static __global__ void __launch_bounds__(AU_THREADS) audio_kernel(AudioParams p) {
   extern __shared__ float smem[];
   // layout: xs[padidx(AU_MAXHALO + AU_SPAN + 16)] input tile; ys[...] second buffer (gain*hp, then de-emph)
@@ -171,13 +196,18 @@ static __global__ void __launch_bounds__(AU_THREADS) audio_kernel(AudioParams p)
   }
   __syncthreads();
   {
-    // pole magnitude is 0.0146: eight samples of warm-up reproduce the running state to < 1e-14
     float v1 = 0.0f;
+    if (LONG_POLE) {
+      // outputs before the tile's first one read as zero: start at the later of the warm-up span and the tile start
+      for (int k = min(p.de_warm, 16 * t); k >= 1; k--) v1 = fmaf(-p.de_a1, v1, ys[padidx(AU_LEAD_LP + 16 * t - k)]);
+    } else {
+      // the reference's pole magnitude is 0.0146: eight samples of warm-up reproduce the running state to < 1e-14
 #pragma unroll
-    for (int k = 8; k >= 1; k--) {
-      const int idx = AU_LEAD_LP + 16 * t - k;
-      const float xv = (idx >= AU_LEAD_LP) ? ys[padidx(idx)] : 0.0f;
-      v1 = fmaf(-p.de_a1, v1, xv);
+      for (int k = 8; k >= 1; k--) {
+        const int idx = AU_LEAD_LP + 16 * t - k;
+        const float xv = (idx >= AU_LEAD_LP) ? ys[padidx(idx)] : 0.0f;
+        v1 = fmaf(-p.de_a1, v1, xv);
+      }
     }
 #pragma unroll
     for (int r = 0; r < 16; r++) {

@@ -56,6 +56,8 @@ struct pmr446_batch {
   DevBuf d_out_rssi, d_out_edge;
   int fft_halo = AF_HALO;    // overlap of the FFT audio tile (AF_HALO or AF_HALO_LONG)
   bool fft_audio = false;    // audio / pcm by fast convolution (audio_fft_kernel); the direct-form kernel serves lpcomp
+  int au_lead = AU_LEAD_MIN; // lead-in of the direct-form kernel's tiles (audio_lead)
+  int de_warm = 0;           // de-emphasis warm-up (deemph_warmup); > 8 selects audio_kernel<true>
   DevBuf d_resp, d_aftw;
   // waterfall
   Waterfall wf;
@@ -120,6 +122,8 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
   const int S = b->S;
   const int M = b->M = (int)cfg->num_channels;
   b->generic = !(M == 16 && cfg->pfb_m == 13);   // the register-window kernel is specialised for 16 x 26 taps
+  int smem_cap = 0;                               // per-block shared memory with opt-in (232 448 B on a B200)
+  cudaDeviceGetAttribute(&smem_cap, cudaDevAttrMaxSharedMemoryPerBlockOptin, b->device);
 
   float fs_res = (float)(cfg->num_channels * cfg->channel_width);
   int rc = b->fe.init(S, cfg->in_fmt, fs_res / (float)cfg->fs_in, cfg->resamp_as, true, cfg->dc_alpha, cfg->max_chunk,
@@ -163,9 +167,9 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
     }
     cudaMemcpy(b->d_tw.p, tw.data(), (size_t)M * sizeof(float2), cudaMemcpyHostToDevice);
     const size_t smem = (size_t)M * (3 * sizeof(float2) + CG_FT * sizeof(float));
-    if (smem > 200 * 1024) { pmr446_batch_destroy(b); return fail(PMR446_EINVAL, "num_channels too large for the shared-memory FFT"); }
+    if (smem > (size_t)smem_cap) { pmr446_batch_destroy(b); return fail(PMR446_EINVAL, "num_channels too large for the shared-memory FFT"); }
     cudaFuncSetAttribute(channelize_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    b->generic_tile = cfg->pfb_m == 13 && channelize_generic_tile_smem(M) <= 200 * 1024;
+    b->generic_tile = cfg->pfb_m == 13 && channelize_generic_tile_smem(M) <= (size_t)smem_cap;
     if (b->generic_tile)
       cudaFuncSetAttribute(channelize_generic_tile_kernel<26>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)channelize_generic_tile_smem(M));
   }
@@ -173,7 +177,7 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
   b->max_tiles = (int)(b->max_ns / CH_TL + 3);
   if (!b->generic && (rc = b->d_mag.alloc_zero((size_t)S * b->max_tiles * 16 * sizeof(float)))) { pmr446_batch_destroy(b); return rc; }
   // demod ring: history for the audio FIR halo + one chunk
-  b->demod_cap = next_pow2(b->max_ns + std::max(AU_MAXHALO + AU_LEAD_LP, AF_N) + 64);
+  b->demod_cap = next_pow2(b->max_ns + std::max(AU_MAXHALO + AU_MAXLEAD, AF_N) + 64);
   if ((rc = b->d_demod.alloc_zero((size_t)S * M * b->demod_cap * sizeof(float)))) { pmr446_batch_destroy(b); return rc; }
 
   // audio filters
@@ -191,16 +195,24 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
     pmr446_batch_destroy(b);
     return rc;
   }
+  // de-emphasis pole: its warm-up sets the direct-form kernel's tile lead-in and the length of its impulse response below
+  b->de_warm = cfg->deemph_fir ? 0 : deemph_warmup(cfg->deemph_a1);
+  b->au_lead = b->de_warm < 0 ? -1 : audio_lead(cfg->lowpass != 0, b->lp_chunks, b->de_warm);
+  if (b->au_lead < 0) {
+    pmr446_batch_destroy(b);
+    return fail(PMR446_EINVAL, "deemph_a1 must satisfy |a1| < 1 with a warm-up that fits the audio tile (|a1| <= 0.977)");
+  }
   // fast-convolution response: hp (x gain) * de-emphasis * optional low-pass, as one impulse response < AF_HALO
   {
     const unsigned fir_len = hpn + (cfg->lowpass ? lpn - 1 : 0) + (cfg->deemph_fir ? PMR446_FIR_DEEMPH_TAPS_LEN - 1 : 0);
     const double a1 = cfg->deemph_a1;
-    if (fir_len + 24 <= (unsigned)AF_HALO_LONG && fabs(a1) < 0.1) {
-      b->fft_halo = fir_len + 24 <= (unsigned)AF_HALO ? AF_HALO : AF_HALO_LONG;
+    const unsigned de_len = (unsigned)std::max(24, b->de_warm);   // the pole's response is cut where it is below 2^-30
+    if (fir_len + de_len <= (unsigned)AF_HALO_LONG) {
+      b->fft_halo = fir_len + de_len <= (unsigned)AF_HALO ? AF_HALO : AF_HALO_LONG;
       std::vector<double> h(hpt, hpt + hpn);
       for (auto& x : h) x *= (double)cfg->audio_gain;
       // de-emphasis (A.1): y[n] = b0 x[n] + b1 x[n-1] - a1 y[n-1]
-      std::vector<double> de(24);
+      std::vector<double> de(de_len);
       de[0] = cfg->deemph_b0;
       de[1] = (double)cfg->deemph_b1 - a1 * de[0];
       for (size_t n = 2; n < de.size(); n++) de[n] = -a1 * de[n - 1];
@@ -246,7 +258,8 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
   if (cfg->waterfall > 0) {
     if ((rc = b->wf.init(S, cfg->waterfall))) { pmr446_batch_destroy(b); return rc; }
   }
-  cudaFuncSetAttribute(audio_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(audio_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(audio_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
   CUDA_TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking));
   CUDA_TRY(cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking));
   CUDA_TRY(cudaStreamCreateWithFlags(&b->out_stream, cudaStreamNonBlocking));
@@ -380,10 +393,15 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
     b->timer.mark(st, TM_GATHER);
   }
 
-  if (ns > 0 && b->generic) {
-    // ---- generic-M channelizer: mix once per sample, then FFT-based analysis bank ------------------
+  if (ny > 0 && b->generic) {
+    // generic-M channelizer: mix once per sample -- every new sample, also in a call that completes no frame: the frames
+    // of later calls read it from the mixed ring
     nco_mix_kernel<<<dim3((unsigned)((ny + 255) / 256), S), 256, 0, st>>>((const float2*)b->fe.out.p, (float2*)b->d_mixed.p, b->fe.out_cap,
                                                                           b->fe.out_cap - 1, r0, ny, b->dtheta);
+    b->launches++;
+  }
+  if (ns > 0 && b->generic) {
+    // ---- generic-M channelizer: FFT-based analysis bank over the mixed ring ---------------------------------------------
     ChanGenParams gp;
     memset(&gp, 0, sizeof gp);
     gp.mixed = (const float2*)b->d_mixed.p;
@@ -410,7 +428,7 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
     const size_t smem = (size_t)M * (3 * sizeof(float2) + CG_FT * sizeof(float));
     if (b->generic_tile) channelize_generic_tile_kernel<26><<<(unsigned)((long long)S * gp.tiles), 512, channelize_generic_tile_smem(M), st>>>(gp);
     else channelize_generic_kernel<<<(unsigned)((long long)S * gp.tiles), 256, smem, st>>>(gp);
-    b->launches += 2;
+    b->launches++;
     b->timer.mark(st, TM_CHANNELIZE);
   } else if (ns > 0) {
     // ---- channelizer + discriminator --------------------------------------------------------
@@ -514,7 +532,7 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
       ap.demod_stride = b->demod_cap;
       ap.demod_mask = b->demod_cap - 1;
       ap.rows = S * M;
-      ap.lead = b->cfg.lowpass ? AU_LEAD_LP : AU_LEAD_MIN;
+      ap.lead = b->au_lead;
       const long long own = AU_SPAN - ap.lead;
       ap.tile0 = f0 / own;
       ap.tiles = (int)((f1 + own - 1) / own - ap.tile0);
@@ -535,7 +553,9 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
       ap.pcm = fft_now ? nullptr : out->pcm;
       ap.lpcomp = out->lpcomp;
       ap.out_ld = out->ld;
-      audio_kernel<<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, audio_smem_bytes(), st>>>(ap);
+      ap.de_warm = b->de_warm;
+      if (b->de_warm > 8) audio_kernel<true><<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, audio_smem_bytes(), st>>>(ap);
+      else audio_kernel<false><<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, audio_smem_bytes(), st>>>(ap);
       b->launches++;
       b->timer.mark(st, TM_AUDIO);
     }

@@ -21,6 +21,7 @@ struct pmr446_receiver {
   DevBuf d_chan, d_rssi, d_state, d_u, d_range, d_sel, d_lpcomp, d_hp, d_lp, d_coef, d_freqs, d_edge, d_selchan, d_selrow;
   bool fused = false;        // 16-channel kernel: RSSI and edge samples come out of the channelizer, no [S][M][ns] buffer
   int hp_chunks = 0, lp_chunks = 0, hp_delay = 0;
+  int au_lead = AU_LEAD_MIN, de_warm = 0;   // audio_kernel tile lead-in and de-emphasis warm-up (backend.cuh)
   // staging for the host-buffer call
   DevBuf d_in, d_o_rssi, d_o_status, d_o_audio, d_o_pcm, d_o_ctcss_in, d_o_power, d_o_ascii, d_o_peak;
   cudaStream_t own_stream = nullptr;
@@ -83,7 +84,7 @@ extern "C" int pmr446_receiver_create(const pmr446_rx_config* cfg, pmr446_receiv
   const int S = r->S = cfg->chain.n_streams;
   r->M = (int)M;
   r->max_ns = pmr446_batch_max_ns(r->batch);
-  r->sel_cap = next_pow2(r->max_ns + AU_MAXHALO + AU_LEAD_LP + 64);
+  r->sel_cap = next_pow2(r->max_ns + AU_MAXHALO + AU_MAXLEAD + 64);
   std::vector<float> hp(PMR446_HP_AUDIO_TAPS_LEN), lp(PMR446_LP_AUDIO_TAPS_LEN);
   pmr446_hp_audio_taps_fill(hp.data());
   pmr446_lp_audio_taps_fill(lp.data());
@@ -97,6 +98,8 @@ extern "C" int pmr446_receiver_create(const pmr446_rx_config* cfg, pmr446_receiv
   const double fs_audio = (double)cfg->chain.channel_width;
   for (int j = 0; j < RX_TONES; j++) coef[j] = 2.0f * cosf((float)((2.0 * M_PI * pmr446_ctcss_freqs[j]) / fs_audio));
   r->fused = (M == 16 && cfg->chain.pfb_m == 13);
+  r->de_warm = deemph_warmup(cfg->chain.deemph_a1);   // pmr446_batch_create has refused poles whose warm-up does not fit
+  r->au_lead = audio_lead(cfg->chain.lowpass != 0, (int)((lpn + 15) / 16), r->de_warm);
   if ((rc = r->fused ? (r->d_edge.alloc_zero((size_t)S * M * 2 * sizeof(float2)) || r->d_selchan.alloc_zero((size_t)S * sizeof(int)) ||
                         r->d_selrow.alloc((size_t)S * r->max_ns * sizeof(float)))
                      : (r->d_selchan.alloc_zero((size_t)S * sizeof(int)) || r->d_chan.alloc((size_t)S * M * r->max_ns * sizeof(float2)))) || (rc = r->d_rssi.alloc_zero((size_t)S * M * sizeof(float))) ||
@@ -110,7 +113,8 @@ extern "C" int pmr446_receiver_create(const pmr446_rx_config* cfg, pmr446_receiv
   }
   cudaMemcpy(r->d_coef.p, coef, sizeof coef, cudaMemcpyHostToDevice);
   cudaMemcpy(r->d_freqs.p, pmr446_ctcss_freqs, sizeof pmr446_ctcss_freqs, cudaMemcpyHostToDevice);
-  cudaFuncSetAttribute(audio_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(audio_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(audio_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
   CUDA_TRY(cudaStreamCreateWithFlags(&r->own_stream, cudaStreamNonBlocking));
   if (cudaDeviceSynchronize() != cudaSuccess || cudaGetLastError() != cudaSuccess) {
     pmr446_receiver_destroy(r);
@@ -199,7 +203,7 @@ extern "C" int pmr446_receiver_execute_device(pmr446_receiver* r, const void* iq
     ap.demod_stride = r->sel_cap;
     ap.demod_mask = r->sel_cap - 1;
     ap.rows = S;
-    ap.lead = r->cfg.chain.lowpass ? AU_LEAD_LP : AU_LEAD_MIN;
+    ap.lead = r->au_lead;
     const long long own = AU_SPAN - ap.lead;
     ap.tiles = (int)((ns + own - 1) / own + 1);   // a row's range may straddle one more tile boundary than its length suggests
     ap.row_range = (const long long*)r->d_range.p;
@@ -217,7 +221,9 @@ extern "C" int pmr446_receiver_execute_device(pmr446_receiver* r, const void* iq
     ap.lpcomp = (float*)r->d_lpcomp.p;
     ap.out_ld = out->ld;
     ap.lpcomp_ld = r->max_ns;
-    audio_kernel<<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, rx_audio_smem_bytes(), st>>>(ap);
+    ap.de_warm = r->de_warm;
+    if (r->de_warm > 8) audio_kernel<true><<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, rx_audio_smem_bytes(), st>>>(ap);
+    else audio_kernel<false><<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, rx_audio_smem_bytes(), st>>>(ap);
     r->launches += 2;
   }
   CtcssParams cp;

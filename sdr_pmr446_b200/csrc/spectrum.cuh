@@ -96,18 +96,20 @@ __device__ __forceinline__ void wf_stage_generic(int R, const float2* __restrict
     const int j = idx % nb, q = idx / nb;
     const int k = j % Ns;
     const int j0 = (j - k) * R + k;
-    float2 acc = x[j];
-    int t1 = 0, t2 = 0;   // (r k tstep) mod N and ((q r) mod R) rstep, stepped instead of multiplied
+    // a sum of up to 4096 terms that cancel to a small output in most bins: accumulated in double, so the only float32
+    // rounding left is that of the inputs, the twiddle table and the result (a float32 running sum lost ~p ulp of the
+    // largest terms, e.g. 4e-6 of the stage RMS in the weak bins of a 1828 = 4 x 457 channel bank)
+    double ax = x[j].x, ay = x[j].y;
+    int t = 0;   // (r k tstep + ((q r) mod R) rstep) mod N: the product of the two twiddles is one table entry
     for (int r = 1; r < R; r++) {
-      t1 += k * tstep; if (t1 >= N) t1 -= N;
-      t2 += q * rstep; if (t2 >= N) t2 -= N;
+      t += k * tstep + q * rstep;
+      while (t >= N) t -= N;
       const float2 a = x[j + r * nb];
-      const float2 w1 = tw[t1], w2 = tw[t2];
-      const float2 w = make_float2(w1.x * w2.x - w1.y * w2.y, w1.x * w2.y + w1.y * w2.x);
-      acc.x += a.x * w.x - a.y * w.y;
-      acc.y += a.x * w.y + a.y * w.x;
+      const float2 w = tw[t];
+      ax = fma((double)a.x, (double)w.x, fma(-(double)a.y, (double)w.y, ax));
+      ay = fma((double)a.x, (double)w.y, fma((double)a.y, (double)w.x, ay));
     }
-    y[j0 + q * Ns] = acc;
+    y[j0 + q * Ns] = make_float2((float)ax, (float)ay);
   }
 }
 

@@ -22,8 +22,8 @@ def stronger_later():
     return (synth.Carrier(8, 0.08, 1700.0, 123.0), synth.Carrier(15, 0.25, 2400.0, 250.3, t_on=1.2))
 
 
-def capture(carriers, seed=446, seconds=SECONDS, fs=FS):
-    spec = synth.CaptureSpec(fs=float(fs), carriers=carriers)
+def capture(carriers, seed=446, seconds=SECONDS, fs=FS, num_channels=16):
+    spec = synth.CaptureSpec(fs=float(fs), num_channels=num_channels, carriers=carriers)
     return synth.make_cu8(spec, int(seconds * fs), seed)
 
 

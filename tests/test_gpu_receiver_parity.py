@@ -19,7 +19,7 @@ EXACT = ("state", "active_chan", "n_audio", "tone_detected", "ctcss_index", "eve
 def _pair(carrier_sets, chunk=sc.CHUNK, fs=sc.FS, **kw):
     from oracle import oracle as orc
     from sdr_pmr446_b200 import chain
-    iq = np.stack([sc.capture(c, 446 + s, fs=fs) for s, c in enumerate(carrier_sets)])
+    iq = np.stack([sc.capture(c, 446 + s, fs=fs, num_channels=kw.get("num_channels", 16)) for s, c in enumerate(carrier_sets)])
     rx = chain.PmrReceiver(n_streams=len(carrier_sets), fs_in=fs, in_fmt=1, max_chunk=chunk, audio_gain=1.0, **kw)
     g = rx.run(iq, chunk)
     rx.close()
@@ -115,3 +115,12 @@ def test_receiver_on_2400k_captures():
     g, refs = _pair(sets, chunk=240000, fs=2400000, lock_mode=1)
     _check(g, refs, sets, chunk=240000, fs=2400000)
     assert int(g[-1]["active_chan"][0]) == 6 and int(g[-1]["active_chan"][1]) == 14
+
+
+def test_eight_channel_receiver():
+    """num_channels = 8: the receiver's non-fused path (channel samples of every channel, rssi_kernel, rx_demod_kernel) behind
+    the generic channelizer, on a 100 kHz grid of 8 channels."""
+    sets = (sc.keyed_two_calls(), sc.stronger_later()[:1])
+    g, refs = _pair(sets, num_channels=8)
+    _check(g, refs, sets)
+    assert int(g[0]["active_chan"][0]) == 1 and int(g[-1]["active_chan"][0]) == 6 and int(g[0]["active_chan"][1]) == 7

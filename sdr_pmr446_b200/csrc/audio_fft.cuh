@@ -1,18 +1,20 @@
-// audio_fft_kernel: the audio chain of every channel by fast convolution.  Replaces the same reference lines as
-// audio_kernel (/root/reference/src/sdr_pmr446.c:882-902: 377-tap CTCSS-removal FIR, gain, de-emphasis, optional
-// 103-tap low-pass; SURVEY.md Appendix A.1, A.10, A.11) and the s16 cast of src/dsd_in.c:172-175.
+// Shared pieces of the fast-convolution audio chain (audio_fft4_kernel, audio_fft4.cuh): its constants, its parameter
+// block, the saturating s16 cast, and the radix-4 / radix-16 DFT helpers on (re, im) register pairs that the
+// channelizer, the register DFTs (reg_dft.cuh) and the waterfall (spectrum_fast.cuh) reuse.
 //
-// The three filters in series are one LTI system whose impulse response is shorter than 512 samples (377 + 103 - 1
-// FIR taps followed by the de-emphasis pole 0.0146, below 1e-60 after 32 more samples).  Overlap-save with 4096-point
-// transforms: a block takes TWO channel rows as the real and imaginary part of one complex sequence (the filter is
-// real, so the rows stay separated), runs a forward FFT, multiplies by the precomputed response H (which carries
-// gain and 1/N), runs the inverse FFT and keeps the last 3584 samples.  ~70 flop per audio sample instead of the 759
-// of the direct form.
+// The audio chain replaces the same reference lines as audio_kernel (/root/reference/src/sdr_pmr446.c:882-902:
+// 377-tap CTCSS-removal FIR, gain, de-emphasis, optional 103-tap low-pass; SURVEY.md Appendix A.1, A.10, A.11) and the
+// s16 cast of src/dsd_in.c:172-175.  The three filters in series are one LTI system whose impulse response is shorter
+// than 512 samples (377 + 103 - 1 FIR taps followed by the de-emphasis pole 0.0146, below 1e-60 after 32 more
+// samples).  Overlap-save with 4096-point transforms: forward FFT, multiply by the precomputed response H (which
+// carries gain and 1/N), inverse FFT, keep the last 3584 samples.  ~70 flop per audio sample instead of the 759 of the
+// direct form.
 //
 // FFT layout: 256 threads x 16 points in registers, three radix-16 passes (4096 = 16^3), data exchanged through
 // shared memory between passes (conflict-free: 16-lane groups read consecutive or stride-17 elements); the inter-pass
-// twiddles are powers of one table entry per thread and pass, built by a depth-4 product tree in registers.  The forward transform leaves X[k2 + 16 k1 + 256 k0] in register k0 of thread 16 k2 + k1; H is
-// stored in that order and the inverse transform walks the same exchanges backwards, so no reordering pass exists.
+// twiddles are powers of one table entry per thread and pass, built by a depth-4 product tree in registers.  The
+// forward transform leaves X[k2 + 16 k1 + 256 k0] in register k0 of thread 16 k2 + k1; H is stored in that order and
+// the inverse transform walks the same exchanges backwards, so no reordering pass exists.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -39,8 +41,8 @@ struct AudioFftParams {
   const float* demod;        // ring [rows][demod_stride]
   long long demod_stride, demod_mask;
   int rows;                  // n_streams * num_channels
-  int tiles;                 // tiles per row pair
-  long long tile0;           // tile k covers outputs [k own, (k + 1) own), own = AF_N - HALO
+  int tiles;                 // tiles per group of four rows; tile k covers outputs [f0 + k own, f0 + (k + 1) own), own = AF_N - HALO
+  long long tile0;           // unread, 0: keeps f0 / f1 at the parameter offsets audio_fft4_kernel was scheduled and timed with
   long long f0, f1;          // owned samples; samples >= f1 do not exist yet
   const float2* resp;        // [AF_N] response, element k0 * 256 + t = H[(t >> 4) + 16 (t & 15) + 256 k0] / N
   const float2* tw;          // [AF_N] exp(-2 pi i k / N)
@@ -115,116 +117,6 @@ __device__ __forceinline__ void twiddle_powers(float2* v, float2 w) {
   for (int k = 9; k < 16; k++) pw[k] = cmul(pw[8], pw[k - 8]);
 #pragma unroll
   for (int k = 1; k < 16; k++) v[af_dig(k)] = cmul(v[af_dig(k)], pw[k]);
-}
-
-template <int HALO>   // overlap discarded per tile; the tile keeps AF_N - HALO outputs
-static __global__ void __launch_bounds__(AF_T, 4) audio_fft_kernel(AudioFftParams p) {
-  constexpr int AF_OWN = AF_N - HALO;
-  __shared__ float2 sm[AF_SMEM];
-  const int t = threadIdx.x;
-  const int pair = blockIdx.x / p.tiles;
-  const long long tile = p.tile0 + blockIdx.x % p.tiles;
-  const int row1 = 2 * pair, row2 = 2 * pair + 1;
-  const bool has2 = row2 < p.rows;
-  const long long o0 = tile * AF_OWN - HALO;       // absolute index of tile sample 0
-  const float* d1 = p.demod + (long long)row1 * p.demod_stride;
-  const float* d2 = p.demod + (long long)(has2 ? row2 : row1) * p.demod_stride;
-  // 32-bit window of existing samples, relative to o0
-  const long long lo64 = -o0, hi64 = p.f1 - o0;
-  const int z0 = (int)(lo64 > (1 << 28) ? (1 << 28) : (lo64 < 0 ? 0 : lo64));           // first sample with n >= 0
-  const int z1 = (int)(hi64 > (1 << 28) ? (1 << 28) : (hi64 < 0 ? 0 : hi64));           // one past the last existing one
-  const unsigned base32 = (unsigned)o0, dmask = (unsigned)p.demod_mask;
-
-  float2 v[16], w[16];
-  // thread t holds tile samples t + 256 m: row1 in .x, row2 in .y
-  if (z0 == 0 && z1 >= AF_N && has2) {   // block-uniform: the whole tile exists
-#pragma unroll
-    for (int m = 0; m < 16; m++) {
-      const unsigned idx = (base32 + (unsigned)(t + 256 * m)) & dmask;
-      v[m] = make_float2(d1[idx], d2[idx]);
-    }
-  } else {
-#pragma unroll
-    for (int m = 0; m < 16; m++) {
-      const int i = t + 256 * m;
-      float a = 0.0f, b = 0.0f;
-      if (i >= z0 && i < z1) {
-        const unsigned idx = (base32 + (unsigned)i) & dmask;
-        a = d1[idx];
-        if (has2) b = d2[idx];
-      }
-      v[m] = make_float2(a, b);
-    }
-  }
-  const int hi4 = t >> 4, lo4 = t & 15;
-
-  // ---- forward: over m (-> k2), twiddle W^(t k2) ----
-  dft16<false>(v);
-  twiddle_powers<false>(v, __ldg(p.tw + t));
-#pragma unroll
-  for (int k2 = 0; k2 < 16; k2++) sm[k2 * 256 + t] = v[af_dig(k2)];
-  __syncthreads();
-  // thread (k2 = hi4, a = lo4): over b (-> k1), twiddle W^(16 a k1)
-#pragma unroll
-  for (int m = 0; m < 16; m++) w[m] = sm[hi4 * 256 + lo4 + 16 * m];
-  dft16<false>(w);
-  twiddle_powers<false>(w, __ldg(p.tw + 16 * lo4));
-  __syncthreads();
-#pragma unroll
-  for (int k1 = 0; k1 < 16; k1++) sm[hi4 * 272 + k1 * 17 + lo4] = w[af_dig(k1)];
-  __syncthreads();
-  // thread (k2 = hi4, k1 = lo4): over a (-> k0)
-#pragma unroll
-  for (int a = 0; a < 16; a++) v[a] = sm[hi4 * 272 + lo4 * 17 + a];
-  dft16<false>(v);
-
-  // ---- multiply by the response (includes 1/N and the audio gain) ----
-#pragma unroll
-  for (int k0 = 0; k0 < 16; k0++) w[k0] = cmul(v[af_dig(k0)], __ldg(p.resp + k0 * 256 + t));
-
-  // ---- inverse: over k0 (-> a), twiddle conj W^(a (16 k1 + k2)): the factor conj W^(a k2) belongs to the next pass
-  // but only depends on this thread's k2 and the register index a, so it rides along here ----
-  dft16<true>(w);
-  twiddle_powers<true>(w, __ldg(p.tw + 16 * lo4 + hi4));
-  __syncthreads();
-#pragma unroll
-  for (int a = 0; a < 16; a++) sm[hi4 * 272 + lo4 * 17 + a] = w[af_dig(a)];
-  __syncthreads();
-  // thread (k2 = hi4, a = lo4): over k1 (-> b), twiddle conj W^(16 b k2)
-#pragma unroll
-  for (int k1 = 0; k1 < 16; k1++) v[k1] = sm[hi4 * 272 + k1 * 17 + lo4];
-  dft16<true>(v);
-  twiddle_powers<true>(v, __ldg(p.tw + 16 * hi4));
-  __syncthreads();
-#pragma unroll
-  for (int b = 0; b < 16; b++) sm[hi4 * 256 + lo4 + 16 * b] = v[af_dig(b)];
-  __syncthreads();
-  // thread t: over k2 (-> m): tile samples t + 256 m
-#pragma unroll
-  for (int k2 = 0; k2 < 16; k2++) w[k2] = sm[k2 * 256 + t];
-  dft16<true>(w);
-
-  // ---- keep samples HALO.. of the tile that this call owns ----
-  const long long own_lo = (tile * AF_OWN > p.f0 ? tile * AF_OWN : p.f0) - o0;
-  const long long own_hi = ((tile + 1) * AF_OWN < p.f1 ? (tile + 1) * AF_OWN : p.f1) - o0;
-  const int s_lo = (int)(own_lo < HALO ? HALO : own_lo), s_hi = (int)(own_hi > AF_N ? AF_N : (own_hi < 0 ? 0 : own_hi));
-  const long long col0 = o0 - p.f0;   // column of tile sample 0
-#pragma unroll
-  for (int m = HALO / 256; m < 16; m++) {
-    const int i = t + 256 * m;
-    if (i >= s_lo && i < s_hi) {
-      const float2 y = w[af_dig(m)];
-      const long long col = col0 + i;
-      if (p.audio) {
-        p.audio[(long long)row1 * p.out_ld + col] = y.x;
-        if (has2) p.audio[(long long)row2 * p.out_ld + col] = y.y;
-      }
-      if (p.pcm) {
-        p.pcm[(long long)row1 * p.out_ld + col] = pcm_sat(y.x);
-        if (has2) p.pcm[(long long)row2 * p.out_ld + col] = pcm_sat(y.y);
-      }
-    }
-  }
 }
 
 }  // namespace pmr

@@ -1,16 +1,16 @@
-// audio_fft4_kernel: audio_fft_kernel (same reference lines, same transform layout, same response table) with FOUR channel
-// rows per block instead of two, so that every floating-point instruction is a packed one.
+// audio_fft4_kernel: the audio chain of every channel by fast convolution (method, transform layout and response table:
+// audio_fft.cuh), FOUR channel rows per block, so that every floating-point instruction is a packed one.
 //
-// audio_fft_kernel keeps one complex number (row1 + i row2) per register pair: complex additions are one FADD2, but a
-// multiplication by a twiddle needs the swapped pair and falls back to four scalar FMUL / FFMA, and the +-i rotations of
-// the radix-4 butterflies to two scalar FADDs -- 47 % of its instructions are scalar FP32 and the kernel is bound by issue
-// slots (77 % busy at 60 % FMA pipe, profiles/ncu_r02v_audio_fft.md).  Here a register pair holds the SAME component of TWO
-// sequences (A = row0 + i row1, B = row2 + i row3): C2 = {(re A, re B), (im A, im B)}.  Both sequences go through
-// identical operations with identical twiddles, so a complex multiplication is four packed instructions for two products
-// (twiddle components as scalar-broadcast operands), a rotation by +-i is a pair swap that costs nothing, and the index /
-// predicate / barrier overhead of a tile is shared by four rows.
+// Two rows per block (one complex number row1 + i row2 per register pair, round 1's kernel) make complex additions one
+// FADD2, but a multiplication by a twiddle needs the swapped pair and falls back to four scalar FMUL / FFMA, and the +-i
+// rotations of the radix-4 butterflies to two scalar FADDs -- 47 % of its instructions were scalar FP32 and it was bound
+// by issue slots (77 % busy at 60 % FMA pipe, profiles/ncu_r02v_audio_fft.md).  Here a register pair holds the SAME
+// component of TWO sequences (A = row0 + i row1, B = row2 + i row3): C2 = {(re A, re B), (im A, im B)}.  Both sequences
+// go through identical operations with identical twiddles, so a complex multiplication is four packed instructions for
+// two products (twiddle components as scalar-broadcast operands), a rotation by +-i is a pair swap that costs nothing,
+// and the index / predicate / barrier overhead of a tile is shared by four rows.
 //
-// Two more differences.  (1) The exchange buffer gives every k2 row 272 elements in BOTH layouts, so the rows a 16-thread group
+// Two more differences from round 1's kernel.  (1) The exchange buffer gives every k2 row 272 elements in BOTH layouts, so the rows a 16-thread group
 // (k2 = t >> 4) reads and writes in the middle passes are its own: five of the seven block barriers are __syncwarp() and the
 // eight warps of a block drift apart through the FP-heavy and the shared-memory-heavy phases instead of marching in step
 // (the FMA pipe was 56 % busy with 1.3 warps waiting on it per issue: phases, not capacity).  (2) Tiles are counted from the

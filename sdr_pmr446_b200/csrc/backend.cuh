@@ -3,7 +3,7 @@
 // /root/reference/src/sdr_pmr446.c:882-902 (firfilt_rrrf_execute_block, wdelayf, iirfilt_rrrf;
 // SURVEY.md Appendix A.1, A.10, A.11) for every channel, and the s16 cast of src/dsd_in.c:172-175.
 //
-// Direct form.  Since audio_fft_kernel (fast convolution) took over the audio / s16 outputs of the batched chain, this
+// Direct form.  Since audio_fft4_kernel (fast convolution) took over the audio / s16 outputs of the batched chain, this
 // kernel serves the complementary CTCSS branch (lpcomp), the receiver's squelch-selected rows (per-row sample ranges) and
 // configurations whose composite impulse response does not fit the FFT tile.
 #pragma once

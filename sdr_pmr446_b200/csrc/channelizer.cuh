@@ -25,7 +25,7 @@
 
 #include "audio_fft.cuh"   // dft16 / af_dig
 #include "frontend.cuh"    // Correction
-#include "frontend_fused.cuh"   // packed FP32 helpers
+#include "packed_f32.cuh"
 
 namespace pmr {
 
@@ -139,10 +139,8 @@ template <> struct TapState<false> {};
 
 // TAPS = the selector taps (mag_part / edge) are wanted: a separate instantiation, so that the throughput path carries
 // none of their registers.
-// PIPE = true: the next batch's staging loads sit in registers across phase B + C (168 registers, 3 blocks per SM);
-// PIPE = false: they are only PREFETCHED into L2 a batch ahead and loaded when staged (128 registers, 4 blocks per SM).
-template <bool NCO_CONST, bool TAPS, bool PIPE = false>
-__global__ void __launch_bounds__(128, (PIPE || TAPS) ? 3 : 4) channelize16_kernel(ChanParams p, ChanTaps tp) {
+template <bool NCO_CONST, bool TAPS>
+__global__ void __launch_bounds__(128, TAPS ? 3 : 4) channelize16_kernel(ChanParams p, ChanTaps tp) {
   __shared__ __align__(16) float2 ch_smem[4 * CH_SMEM_WARP];
   const int lane = threadIdx.x & 31;
   const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -243,8 +241,9 @@ __global__ void __launch_bounds__(128, (PIPE || TAPS) ? 3 : 4) channelize16_kern
   if (lane < 16) V[-CH_V_STRIDE + lane] = make_float2(0.0f, 0.0f);
 
   // steady-state staging (warp-uniform per batch): every new sample of the batch exists and they all take the same
-  // correction path.  Then the batch's eight 128-bit loads per lane are issued one batch AHEAD -- after phase A of the
-  // previous batch, when its 33-sample window is dead -- and sit in registers across phase B + C.
+  // correction path.  Then the batch's eight 128-bit loads per lane are issued back to back when it is staged, from L2:
+  // its samples were prefetched there one batch ahead (128 registers, 4 blocks per SM; holding the loads in registers
+  // across the previous batch's phase B + C instead takes 168 registers, 3 blocks per SM).
   auto steady = [&](int b, bool& corr_all) {
     const int jb = 512 * b + CH_HIST * 16, rel_b = seg_rel0 + jb;
     corr_all = vrow && jb >= from_rel && rel_b >= 0 && ((rel_b + 511) >> cr.seg_shift) < cr.nseg;
@@ -288,12 +287,6 @@ __global__ void __launch_bounds__(128, (PIPE || TAPS) ? 3 : 4) channelize16_kern
     }
     return true;
   };
-  float4 t[8];
-  auto issue_loads = [&](int b) {
-    const int jb = 512 * b + CH_HIST * 16;
-#pragma unroll
-    for (int i = 0; i < 8; i++) t[i] = *(const float4*)(res + ((j0_32 + (unsigned)(jb + 2 * lane + 64 * i)) & rmask));
-  };
   auto prefetch_l2 = [&](int b) {
     const int jb = 512 * b + CH_HIST * 16;
 #pragma unroll
@@ -304,7 +297,6 @@ __global__ void __launch_bounds__(128, (PIPE || TAPS) ? 3 : 4) channelize16_kern
   bool ca_next = false, ca_last = false;
   bool fast_next = any && steady(b_first, ca_next);
   const bool tile_steady = fast_next && steady(b_last, ca_last) && ca_last == ca_next;
-  if (fast_next && PIPE) issue_loads(b_first);
   if (any && !stage_history_fast(b_first))
     for (int pp = 2 * lane; pp < CH_HIST * 16; pp += 64) stage_pair(pp, 512 * b_first, 0);   // history of the first batch
 
@@ -330,7 +322,9 @@ __global__ void __launch_bounds__(128, (PIPE || TAPS) ? 3 : 4) channelize16_kern
     }
     // ---- staging: 32 new frames = 512 samples, 8 pairs per lane --------------------------------------------------------------
     if (fast) {
-      if (!PIPE) issue_loads(batch);
+      float4 t[8];
+#pragma unroll
+      for (int i = 0; i < 8; i++) t[i] = *(const float4*)(res + ((j0_32 + (unsigned)(boff + CH_HIST * 16 + 2 * lane + 64 * i)) & rmask));
       if (corr_all) {
         const int rel_b = seg_rel0 + boff + CH_HIST * 16;
         float2 v0[8], e[8];
@@ -356,7 +350,7 @@ __global__ void __launch_bounds__(128, (PIPE || TAPS) ? 3 : 4) channelize16_kern
       for (int i = 0; i < 8; i++) stage_pair(CH_HIST * 16 + 2 * lane + 64 * i, boff, 1);
     }
     __syncwarp();
-    if (!PIPE && batch < b_last) prefetch_l2(batch + 1);
+    if (batch < b_last) prefetch_l2(batch + 1);
     // ---- phase A: branch filters.  Frame kk of the batch sits in X frames kk .. kk + 25 (newest last) --------------------------
 #pragma unroll 1
     for (int pass = 0; pass < 2; pass++) {
@@ -375,7 +369,6 @@ __global__ void __launch_bounds__(128, (PIPE || TAPS) ? 3 : 4) channelize16_kern
     }
     __syncwarp();
     fast_next = batch < b_last && (tile_steady || steady(batch + 1, ca_next));
-    if (fast_next && PIPE) issue_loads(batch + 1);
     // ---- phase B + C: lane = frame kk = 32 batch + lane ------------------------------------------------------------------------
     {
       float2* const row = V + lane * CH_V_STRIDE;

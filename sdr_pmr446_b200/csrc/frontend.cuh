@@ -503,7 +503,7 @@ static __global__ void zir_tail_kernel(float2* ring, long long ring_stride, long
 // Stage list MA,MB,MC,MD = semi-lengths in execution order (highest rate first), 0 = absent.
 // G = input samples per loop iteration (multiple of 2^NST).
 template <int SRC, int DC, int G, int MA, int MB, int MC, int MD, bool ARB>
-__global__ void __launch_bounds__(128, (ARB && (MA > 0) + (MB > 0) >= 2) ? 2 : 3) cascade_kernel(CascadeParams p) {
+__global__ void __launch_bounds__(128, 3) cascade_kernel(CascadeParams p) {
   constexpr int NST = (MA > 0) + (MB > 0) + (MC > 0) + (MD > 0);
   constexpr int D = 1 << NST;
   constexpr int NO = G / D;  // outputs per iteration

@@ -12,7 +12,7 @@
 //    at 600 kHz -> 6 at 300 kHz -> 4 resampler outputs (one 32-byte sector, one 256-bit store).  The resampler phase has
 //    period 2 (step = 1.5): outputs 2q, 2q + 1 come from inputs 3q, 3q + 1 with the two filter-bank rows as
 //    constant-bank operands -- no bank gathers, no phase arithmetic;
-//  * raw bytes are prefetched two sub-blocks ahead (16 registers).
+//  * raw bytes travel global -> shared memory by cp.async FF_CPD sub-blocks ahead of their use (no registers in flight).
 // The DC blocker runs in its zero-state form (DC_ZSR, see frontend.cuh); the zero-input part is added by the consumer of
 // the 200 kHz ring (channelize16_kernel while it stages its tile) or in place by zir_tail_kernel.
 #pragma once
@@ -27,7 +27,6 @@
 namespace pmr {
 
 constexpr int FF_THREADS = 128;
-constexpr int FF_SLOTS = 29 + 13;   // shared-memory history per thread: m = 10 stage (19 even + 10 odd) + resampler window (13)
 
 struct FusedParams {
   CascadeParams c;       // source view, segment grid, DC blocker, destination ring, hb[0..2] = taps of m = 3, 5, 10
@@ -45,15 +44,13 @@ struct HbPair {
 #pragma unroll
     for (int i = 0; i < M; i++) ho[i] = make_float2(0.0f, 0.0f);
   }
-  // SM: the history lives in the thread's shared-memory column (slot k at sm[k * FF_THREADS]) instead of he / ho, which
-  // are then never touched: a stage that runs once per iteration only needs its window in registers while it runs
-  template <bool SCALE, bool SM = false>
-  __device__ __forceinline__ void run(const float* h, const float2* x, float2* y, float scale, float2* sm = nullptr) {
+  template <bool SCALE>
+  __device__ __forceinline__ void run(const float* h, const float2* x, float2* y, float scale) {
     float2 e[2 * M - 1 + B], o[M + B];
 #pragma unroll
-    for (int i = 0; i < 2 * M - 1; i++) e[i] = SM ? sm[i * FF_THREADS] : he[i];
+    for (int i = 0; i < 2 * M - 1; i++) e[i] = he[i];
 #pragma unroll
-    for (int i = 0; i < M; i++) o[i] = SM ? sm[(2 * M - 1 + i) * FF_THREADS] : ho[i];
+    for (int i = 0; i < M; i++) o[i] = ho[i];
 #pragma unroll
     for (int b = 0; b < B; b++) { e[2 * M - 1 + b] = x[2 * b]; o[M + b] = x[2 * b + 1]; }
 #pragma unroll
@@ -63,28 +60,12 @@ struct HbPair {
       for (int j = 0; j < 2 * M; j++) acc = fma_tap(h[j], e[2 * M - 1 + b - j], acc);   // h points into the kernel parameters
       y[b] = SCALE ? fmul2(acc, make_float2(scale, scale)) : acc;
     }
-    if (SM) {
 #pragma unroll
-      for (int i = 0; i < 2 * M - 1; i++) sm[i * FF_THREADS] = e[B + i];
+    for (int i = 0; i < 2 * M - 1; i++) he[i] = e[B + i];
 #pragma unroll
-      for (int i = 0; i < M; i++) sm[(2 * M - 1 + i) * FF_THREADS] = o[B + i];
-    } else {
-#pragma unroll
-      for (int i = 0; i < 2 * M - 1; i++) he[i] = e[B + i];
-#pragma unroll
-      for (int i = 0; i < M; i++) ho[i] = o[B + i];
-    }
+    for (int i = 0; i < M; i++) ho[i] = o[B + i];
   }
 };
-
-// cu8 -> pair, exactly fl((u8 - fl(127.4)) / 128) like the scalar loader: PRMT drops the byte into the mantissa of 2^23,
-// one packed FADD removes the 2^23, one packed FFMA scales and offsets
-__device__ __forceinline__ float2 cu8_pair(unsigned w, int k) {
-  const float2 raw = make_float2(__uint_as_float(__byte_perm(w, 0x4B000000u, 0x7540u + (unsigned)(2 * k))),
-                                 __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7540u + (unsigned)(2 * k + 1))));
-  const float2 u = fadd2(raw, make_float2(-8388608.0f, -8388608.0f));
-  return ffma2(u, make_float2(1.0f / 128.0f, 1.0f / 128.0f), make_float2(-127.4f / 128.0f, -127.4f / 128.0f));
-}
 
 // cu8 -> X = u8 - 127 as an exact small integer (one PRMT per byte + one packed FADD2 per sample).  The sample itself is
 // x = X / 128 + c0' with c0' = -(fl(127.4) - 127) / 128, both exactly representable, and everything after it is linear:
@@ -93,7 +74,7 @@ __device__ __forceinline__ float2 cu8_pair(unsigned w, int k) {
 // that starts at the head of a stream starts (FusedParams::w0); every other segment starts from zero state as before and
 // the affine scan carries the difference.  With V_X(0) = w0 the true state is exactly v = V_X / 128 + c0' / alpha, so the
 // zero-input term the consumers add is -alpha (V_X / 128) E[k]: DcScanParams::unit_scale, nothing else changes.
-// One FMA-pipe instruction per sample less than cu8_pair (7.5 % of the fused kernel's FMA work).
+// One FMA-pipe instruction per sample less than converting to x itself (7.5 % of the fused kernel's FMA work).
 constexpr float CU8_XBIAS = 127.40000152587890625f - 127.0f;   // X of a zero-valued ("no sample") x
 __device__ __forceinline__ float2 cu8_pair_x(unsigned w, int k) {
   const float2 raw = make_float2(__uint_as_float(__byte_perm(w, 0x4B000000u, 0x7540u + (unsigned)(2 * k))),
@@ -101,36 +82,18 @@ __device__ __forceinline__ float2 cu8_pair_x(unsigned w, int k) {
   return fadd2(raw, make_float2(-8388735.0f, -8388735.0f));    // -(2^23 + 127)
 }
 
-// The same conversion as a table look-up: 256 entries, each replicated for the 32 lanes at a 256-byte pitch, so ONE PRMT
-// builds the shared-memory byte offset (byte 1 = the sample byte, byte 0 = 4 * lane) and the load is conflict-free (bank =
-// lane).  Takes the FADD2 + FFMA2 per sample (15 % of the kernel's FMA-pipe work) off the FMA pipe and puts two LDS.32 on
-// the otherwise idle load/store pipe.  64 KB of shared memory per block.
-constexpr int FF_LUT_BYTES = 256 * 256;
-__device__ __forceinline__ float2 cu8_pair_lut(const char* lut, unsigned lane4, unsigned w, int k) {
-  const unsigned o0 = __byte_perm(w, lane4, 0x5504u + ((unsigned)(2 * k) << 4));
-  const unsigned o1 = __byte_perm(w, lane4, 0x5504u + ((unsigned)(2 * k + 1) << 4));
-  return make_float2(*(const float*)(lut + o0), *(const float*)(lut + o1));
-}
-
 constexpr int FF_G = 48;        // input samples per iteration
 constexpr int FF_SUB = 16;      // ... in three sub-blocks of 16 (32 bytes of cu8)
 constexpr int FF_D = 8;         // decimation of the three half-bands
 constexpr int FF_NO = 4;        // resampler outputs per iteration
-constexpr int FF_PF = 8;        // L1 prefetch distance in sub-blocks
 
-__device__ __forceinline__ void ldg256_nc(const void* p, unsigned* w) {
-  asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]), "=r"(w[4]), "=r"(w[5]), "=r"(w[6]), "=r"(w[7]) : "l"(p));
-}
-
-// SMH = false (shipped): every history in registers, ~250 registers, 2 blocks per SM.  SMH = true: the histories of the two
-// stages that run once per iteration (m = 10 half-band, resampler) live in shared memory (42 slots x 128 threads x 8 B =
-// 43 KB, thread-private columns: a warp's access to one slot is 256 contiguous bytes), 167 registers, 3 blocks per SM --
-// measured 2.75 ms against 2.68 ms (1024 streams), so occupancy is not what limits this kernel.
-// CPA = true: the raw bytes travel global -> shared memory with cp.async, FF_CPD sub-blocks ahead (thread-private 32-byte
-// slots, no registers in flight), instead of register loads two sub-blocks ahead behind an L1 prefetch: ptxas sinks those
-// loads to within ~300 instructions of their use and the profile shows them arriving late (5 % of the kernel's stall samples on
-// the first PRMT of a sub-block; l1tex hit rate 10 %: the L1 prefetch does not hold).
+// Every history lives in registers (~250 registers, 2 blocks per SM); keeping the m = 10 and resampler histories in shared
+// memory instead (167 registers, 3 blocks per SM) measured 2.75 ms against 2.68 ms (1024 streams): occupancy is not what
+// limits this kernel.
+// The raw bytes travel global -> shared memory with cp.async, FF_CPD sub-blocks ahead (thread-private 32-byte slots, no
+// registers in flight).  Register loads two sub-blocks ahead behind an L1 prefetch arrived late: ptxas sinks them to
+// within ~300 instructions of their use (5 % of the kernel's stall samples on the first PRMT of a sub-block; l1tex hit
+// rate 10 %: the L1 prefetch does not hold).
 constexpr int FF_CPD = 6;
 // src_bytes = 0 reads nothing and zero-fills: the guard costs no branch, the iteration stays ONE basic block
 __device__ __forceinline__ void cp_async16(unsigned smem, const void* gmem, int src_bytes) {
@@ -141,24 +104,9 @@ __device__ __forceinline__ uint4 lds128_v(unsigned smem) {   // volatile: stays 
   asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(smem));
   return v;
 }
-template <int DC, int NB = 2, bool SMH = false, bool LUT = false, bool CPA = false>
-__global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedParams fp) {
-  extern __shared__ __align__(16) char ff_lut[];   // LUT only: FF_LUT_BYTES of dynamic shared memory
-  const unsigned lane4 = (threadIdx.x & 31u) * 4u;
-  if (LUT) {
-    for (int i = threadIdx.x; i < 256 * 32; i += blockDim.x) {
-      const int b = i >> 5, ln = i & 31;
-      *(float*)(ff_lut + b * 256 + ln * 4) = fmaf((float)b, 1.0f / 128.0f, -127.4f / 128.0f);   // exact, as cu8_pair
-    }
-    __syncthreads();
-  }
-  __shared__ float2 ff_hist[SMH ? FF_SLOTS * FF_THREADS : 1];
-  float2* const smc = ff_hist + (SMH ? threadIdx.x : 0);
-  float2* const sma = smc + (SMH ? 29 * FF_THREADS : 0);
-  if (SMH) {
-#pragma unroll
-    for (int i = 0; i < FF_SLOTS; i++) smc[i * FF_THREADS] = make_float2(0.0f, 0.0f);
-  }
+// The DC blocker always runs, in X units (cu8_pair_x): the host folds 1 / 128 into p.scale.
+static __global__ void __launch_bounds__(FF_THREADS, 2) fused_frontend_kernel(FusedParams fp) {
+  extern __shared__ __align__(16) char ff_stage[];   // FF_CPD x 32 bytes per thread
   const CascadeParams& p = fp.c;
   long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (gid >= (long long)p.n_streams * p.nseg) return;
@@ -169,17 +117,17 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
   if (i_hi > p.out1) i_hi = p.out1;
   long long qb = T0 - p.halo;
   long long q_cap = qb + p.seg_len;                               // where this segment's local DC sum is complete
-  if (DC == DC_ZSR && q_cap > p.dc_end) q_cap = p.dc_end;
+  if (q_cap > p.dc_end) q_cap = p.dc_end;
   if (qb < 0) qb = 0;
   long long q_end = i_hi > i_lo ? i_hi * FF_D : qb;
-  if (DC == DC_ZSR && q_cap > q_end) q_end = q_cap;
+  if (q_cap > q_end) q_end = q_cap;
   if (q_end <= qb) {
-    if (DC == DC_ZSR) p.sums[gid] = make_float2(0.0f, 0.0f);
+    p.sums[gid] = make_float2(0.0f, 0.0f);
     return;
   }
   // everything below is 32-bit and relative to qb (a multiple of 48: every iteration starts at resampler phase 0)
   const int n_it = (int)((q_end - qb + FF_G - 1) / FF_G);
-  const int cap_it = (DC == DC_ZSR) ? (q_cap > qb ? (int)((q_cap - qb) / FF_G) : 0) : -1;
+  const int cap_it = q_cap > qb ? (int)((q_cap - qb) / FF_G) : 0;
   const long long ob = qb / FF_D;                                  // absolute 300 kHz index of local sample 0
   int own_lo = (int)(i_lo - ob), own_hi = (int)(i_hi - ob);
   if (i_hi <= i_lo) own_lo = own_hi = 0;
@@ -192,7 +140,7 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
 #pragma unroll
   for (int i = 0; i < 13; i++) aw[i] = make_float2(0.0f, 0.0f);
   float2 v = make_float2(0.0f, 0.0f);                              // DC blocker state (zero-state response)
-  if ((DC == DC_ZSR) && !LUT && T0 - p.halo <= 0) v = make_float2(fp.w0, fp.w0);   // head of the stream: see cu8_pair_x
+  if (T0 - p.halo <= 0) v = make_float2(fp.w0, fp.w0);             // head of the stream: see cu8_pair_x
 
   float2* dst = p.dst + (long long)s * p.dst_stride;
   const unsigned dmask = (unsigned)p.dst_mask;
@@ -202,22 +150,11 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
 
   Loader<SRC_CU8> ld;
   ld.template init<FF_SUB>(p.src, s, qb);
-  constexpr bool XU = (DC == DC_ZSR) && !LUT;   // integer-unit recurrence (cu8_pair_x); the host folds 1 / 128 into p.scale
-  const int n_sub = 3 * n_it;
   Raw<SRC_CU8, FF_SUB> raw[3];
-  // Loads go through L1 here (unlike cascade_kernel's no-allocate loads): with ~250 registers per thread ptxas sinks the
-  // register loads towards their use, so the DRAM latency is taken by a register-free L1 prefetch issued FF_PF
-  // sub-blocks ahead and the load proper, two sub-blocks ahead, hits L1.  256 threads x 8 sectors in flight = 64 KB of L1.
-  auto fetch = [&](int sbi, Raw<SRC_CU8, FF_SUB>& r) {
-    if (sbi >= ld.fast_lo && sbi < ld.fast_hi) ldg256_nc(ld.fp + (size_t)sbi * (2 * FF_SUB), r.w);
-  };
-  auto prefetch = [&](int sbi) {
-    if (sbi >= ld.fast_lo && sbi < ld.fast_hi) asm volatile("prefetch.global.L1 [%0];" ::"l"(ld.fp + (size_t)sbi * (2 * FF_SUB)));
-  };
-  // CPA: slot k of the thread = two 16-byte pieces at stage[(2 k + h) * blockDim.x + threadIdx.x]; sub-block sbi uses slot
+  // slot k of the thread = two 16-byte pieces at stage[(2 k + h) * blockDim.x + threadIdx.x]; sub-block sbi uses slot
   // sbi mod FF_CPD = 3 (it & 1) + sub.  One commit group per sub-block step (empty when the sub-block is not a whole aligned
   // group of the chunk), so "all but the newest FF_CPD - 1 groups" is always the group of the sub-block about to be read.
-  const unsigned stage = (unsigned)__cvta_generic_to_shared(ff_lut) + 16u * threadIdx.x, spitch = 16u * blockDim.x;
+  const unsigned stage = (unsigned)__cvta_generic_to_shared(ff_stage) + 16u * threadIdx.x, spitch = 16u * blockDim.x;
   const uint8_t* const cp_dummy = (const uint8_t*)((uintptr_t)ld.cur & ~(uintptr_t)31);
   auto cp_issue = [&](int sbi, int slot) {
     const bool ok = sbi >= ld.fast_lo && sbi < ld.fast_hi;
@@ -231,15 +168,8 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
     const uint4 a = lds128_v(stage + (unsigned)(2 * slot) * spitch), b = lds128_v(stage + (unsigned)(2 * slot + 1) * spitch);
     r.w[0] = a.x; r.w[1] = a.y; r.w[2] = a.z; r.w[3] = a.w; r.w[4] = b.x; r.w[5] = b.y; r.w[6] = b.z; r.w[7] = b.w;
   };
-  if (CPA) {
 #pragma unroll
-    for (int i = 0; i < FF_CPD; i++) cp_issue(i, i);
-  } else {
-#pragma unroll
-    for (int i = 2; i < FF_PF; i++) prefetch(i);
-    fetch(0, raw[0]);
-    if (n_sub > 1) fetch(1, raw[1]);
-  }
+  for (int i = 0; i < FF_CPD; i++) cp_issue(i, i);
   const float2 cpole = make_float2(1.0f - p.alpha, 1.0f - p.alpha);   // exact: alpha is 1 - fl(1 - alpha_nominal)
 
   // One iteration = 48 input samples.  FAST: all three sub-blocks are whole aligned 32-byte groups of the current chunk --
@@ -252,36 +182,29 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
     for (int sub = 0; sub < 3; sub++) {
       const int sbi = 3 * it + sub;
       const int slot = 3 * (it & 1) + sub;
-      if (CPA) {
-        cp_take(sbi, slot, raw[sub]);
-      } else {
-        if (sbi + FF_PF < n_sub) prefetch(sbi + FF_PF);
-        if (sbi + 2 < n_sub) fetch(sbi + 2, raw[(sub + 2) % 3]);   // two sub-blocks ahead
-      }
+      cp_take(sbi, slot, raw[sub]);
       float2 x[FF_SUB];
       if (FAST) {
 #pragma unroll
         for (int j = 0; j < FF_SUB / 2; j++) {
-          x[2 * j] = LUT ? cu8_pair_lut(ff_lut, lane4, raw[sub].w[j], 0) : (XU ? cu8_pair_x(raw[sub].w[j], 0) : cu8_pair(raw[sub].w[j], 0));
-          x[2 * j + 1] = LUT ? cu8_pair_lut(ff_lut, lane4, raw[sub].w[j], 1) : (XU ? cu8_pair_x(raw[sub].w[j], 1) : cu8_pair(raw[sub].w[j], 1));
+          x[2 * j] = cu8_pair_x(raw[sub].w[j], 0);
+          x[2 * j + 1] = cu8_pair_x(raw[sub].w[j], 1);
         }
       } else {
         float xr[FF_SUB], xi[FF_SUB];
         ld.template convert<FF_SUB>(p.src, qb + (long long)sbi * FF_SUB, sbi, raw[sub], xr, xi);
 #pragma unroll
         for (int i = 0; i < FF_SUB; i++)   // X = (x - c0') * 128, exact (a sample) or CU8_XBIAS (a zero: before the stream start)
-          x[i] = XU ? make_float2(fmaf(xr[i], 128.0f, CU8_XBIAS), fmaf(xi[i], 128.0f, CU8_XBIAS)) : make_float2(xr[i], xi[i]);
+          x[i] = make_float2(fmaf(xr[i], 128.0f, CU8_XBIAS), fmaf(xi[i], 128.0f, CU8_XBIAS));
       }
-      if (CPA) cp_issue(sbi + FF_CPD, slot);   // refill the slot just emptied (its words are in x by now)
-      if (DC != DC_NONE) {
-        // A.1 dc blocker, zero-state part: y = x - alpha v[n-1], v[n] = (1 - alpha) v[n-1] + x.  Only the one-FFMA2
-        // recurrence of v is serial; the outputs hang off it.
+      cp_issue(sbi + FF_CPD, slot);   // refill the slot just emptied (its words are in x by now)
+      // A.1 dc blocker, zero-state part: y = x - alpha v[n-1], v[n] = (1 - alpha) v[n-1] + x.  Only the one-FFMA2
+      // recurrence of v is serial; the outputs hang off it.
 #pragma unroll
-        for (int i = 0; i < FF_SUB; i++) {
-          const float2 y = ffma2(nalpha, v, x[i]);
-          v = ffma2(cpole, v, x[i]);
-          x[i] = y;
-        }
+      for (int i = 0; i < FF_SUB; i++) {
+        const float2 y = ffma2(nalpha, v, x[i]);
+        v = ffma2(cpole, v, x[i]);
+        x[i] = y;
       }
       float2 a[FF_SUB / 2], b[FF_SUB / 4];
       sa.template run<false>(p.hb[0], x, a, 1.0f);
@@ -290,11 +213,11 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
       for (int i = 0; i < 4; i++) cin[4 * sub + i] = b[i];
     }
     float2 c[6];                                                   // 300 kHz, scaled by 2^-3 like msresamp2 does
-    sc.template run<true, SMH>(p.hb[2], cin, c, scale, smc);
+    sc.template run<true>(p.hb[2], cin, c, scale);
     // arbitrary resampler (A.5), phase period 2: outputs 4 it + {0, 1, 2, 3} sit at local inputs 6 it + {0, 1, 3, 4}
     float2 w[13 + 6];
 #pragma unroll
-    for (int i = 0; i < 13; i++) w[i] = SMH ? sma[i * FF_THREADS] : aw[i];
+    for (int i = 0; i < 13; i++) w[i] = aw[i];
 #pragma unroll
     for (int i = 0; i < 6; i++) w[13 + i] = c[i];
     float2 o[4];
@@ -307,10 +230,7 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
       o[r] = acc;
     }
 #pragma unroll
-    for (int i = 0; i < 13; i++) {
-      if (SMH) sma[i * FF_THREADS] = w[6 + i];
-      else aw[i] = w[6 + i];
-    }
+    for (int i = 0; i < 13; i++) aw[i] = w[6 + i];
 
     const int lo = own_lo - 6 * it, hi = own_hi - 6 * it;          // owned local inputs of this iteration are [lo, hi)
     float2* d4 = dst + ((jb32 + 4u * (unsigned)it) & dmask);       // 32-byte aligned, never straddles the ring's end
@@ -326,15 +246,11 @@ __global__ void __launch_bounds__(FF_THREADS, NB) fused_frontend_kernel(FusedPar
     }
   };
   for (int it = 0; it < n_it; it++) {
-    if (DC == DC_ZSR) {
-      if (it == cap_it) p.sums[gid] = v;
-    }
+    if (it == cap_it) p.sums[gid] = v;
     if (3 * it >= ld.fast_lo && 3 * it + 2 < ld.fast_hi) iteration(it, std::true_type());
     else iteration(it, std::false_type());
   }
-  if (DC == DC_ZSR) {
-    if (cap_it >= n_it) p.sums[gid] = v;
-  }
+  if (cap_it >= n_it) p.sums[gid] = v;
 }
 
 // ---- front6_kernel: the first SIX half-band stages of a deep plan in one pass (dsd_in: 2.4 Msps -> 37.5 kHz, /root/reference/
@@ -349,10 +265,10 @@ struct Front6Params {
 };
 constexpr int F6_G = 64, F6_D = 64;
 
-constexpr int F6_CPD = 8;   // cp.async depth in sub-blocks (two iterations), see fused_frontend_kernel<..., CPA>
-template <int DC, int ME, int MF, bool CPA = false>
+constexpr int F6_CPD = 8;   // cp.async depth in sub-blocks (two iterations), see fused_frontend_kernel
+template <int ME, int MF>
 __global__ void __launch_bounds__(FF_THREADS, 2) front6_kernel(Front6Params fp) {
-  extern __shared__ __align__(16) char f6_stage[];   // CPA: F6_CPD x 32 bytes per thread
+  extern __shared__ __align__(16) char f6_stage[];   // F6_CPD x 32 bytes per thread
   const CascadeParams& p = fp.c;
   long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (gid >= (long long)p.n_streams * p.nseg) return;
@@ -363,16 +279,16 @@ __global__ void __launch_bounds__(FF_THREADS, 2) front6_kernel(Front6Params fp) 
   if (i_hi > p.out1) i_hi = p.out1;
   long long qb = T0 - p.halo;
   long long q_cap = qb + p.seg_len;
-  if (DC == DC_ZSR && q_cap > p.dc_end) q_cap = p.dc_end;
+  if (q_cap > p.dc_end) q_cap = p.dc_end;
   if (qb < 0) qb = 0;
   long long q_end = i_hi > i_lo ? i_hi * F6_D : qb;
-  if (DC == DC_ZSR && q_cap > q_end) q_end = q_cap;
+  if (q_cap > q_end) q_end = q_cap;
   if (q_end <= qb) {
-    if (DC == DC_ZSR) p.sums[gid] = make_float2(0.0f, 0.0f);
+    p.sums[gid] = make_float2(0.0f, 0.0f);
     return;
   }
   const int n_it = (int)((q_end - qb + F6_G - 1) / F6_G);
-  const int cap_it = (DC == DC_ZSR) ? (q_cap > qb ? (int)((q_cap - qb) / F6_G) : 0) : -1;
+  const int cap_it = q_cap > qb ? (int)((q_cap - qb) / F6_G) : 0;
   const long long ob = qb / F6_D;
   int own_lo = (int)(i_lo - ob), own_hi = (int)(i_hi - ob);
   if (i_hi <= i_lo) own_lo = own_hi = 0;
@@ -382,9 +298,8 @@ __global__ void __launch_bounds__(FF_THREADS, 2) front6_kernel(Front6Params fp) 
   HbPair<ME, 2> se;
   HbPair<MF, 1> sf;
   sa.reset(); sb.reset(); se.reset(); sf.reset();
-  float2 v = make_float2(0.0f, 0.0f);
-  constexpr bool XU = (DC == DC_ZSR);   // integer-unit recurrence, see cu8_pair_x
-  if (XU && T0 - p.halo <= 0) v = make_float2(fp.w0, fp.w0);
+  float2 v = make_float2(0.0f, 0.0f);   // DC blocker state in X units, see cu8_pair_x
+  if (T0 - p.halo <= 0) v = make_float2(fp.w0, fp.w0);
   float2* dst = p.dst + (long long)s * p.dst_stride;
   const unsigned dmask = (unsigned)p.dst_mask, ob32 = (unsigned)ob;
   const float scale = p.scale;
@@ -392,14 +307,7 @@ __global__ void __launch_bounds__(FF_THREADS, 2) front6_kernel(Front6Params fp) 
 
   Loader<SRC_CU8> ld;
   ld.template init<FF_SUB>(p.src, s, qb);
-  const int n_sub = 4 * n_it;
   Raw<SRC_CU8, FF_SUB> raw[4];
-  auto fetch = [&](int sbi, Raw<SRC_CU8, FF_SUB>& r) {
-    if (sbi >= ld.fast_lo && sbi < ld.fast_hi) ldg256_nc(ld.fp + (size_t)sbi * (2 * FF_SUB), r.w);
-  };
-  auto prefetch = [&](int sbi) {
-    if (sbi >= ld.fast_lo && sbi < ld.fast_hi) asm volatile("prefetch.global.L1 [%0];" ::"l"(ld.fp + (size_t)sbi * (2 * FF_SUB)));
-  };
   const unsigned stage = (unsigned)__cvta_generic_to_shared(f6_stage) + 16u * threadIdx.x, spitch = 16u * blockDim.x;
   const uint8_t* const cp_dummy = (const uint8_t*)((uintptr_t)ld.cur & ~(uintptr_t)31);
   auto cp_issue = [&](int sbi, int slot) {
@@ -414,15 +322,8 @@ __global__ void __launch_bounds__(FF_THREADS, 2) front6_kernel(Front6Params fp) 
     const uint4 a = lds128_v(stage + (unsigned)(2 * slot) * spitch), b = lds128_v(stage + (unsigned)(2 * slot + 1) * spitch);
     r.w[0] = a.x; r.w[1] = a.y; r.w[2] = a.z; r.w[3] = a.w; r.w[4] = b.x; r.w[5] = b.y; r.w[6] = b.z; r.w[7] = b.w;
   };
-  if (CPA) {
 #pragma unroll
-    for (int i = 0; i < F6_CPD; i++) cp_issue(i, i);
-  } else {
-#pragma unroll
-    for (int i = 2; i < FF_PF; i++) prefetch(i);
-    fetch(0, raw[0]);
-    if (n_sub > 1) fetch(1, raw[1]);
-  }
+  for (int i = 0; i < F6_CPD; i++) cp_issue(i, i);
 
   HbPair<3, 4> sc4;   // stages 3 and 4 run per HALF iteration (32 inputs): shorter live ranges than 16-sample staging arrays
   HbPair<3, 2> sd2;
@@ -438,34 +339,27 @@ __global__ void __launch_bounds__(FF_THREADS, 2) front6_kernel(Front6Params fp) 
         const int sub = 2 * half + s2;
         const int sbi = 4 * it + sub;
         const int slot = 4 * (it & 1) + sub;
-        if (CPA) {
-          cp_take(slot, raw[sub]);
-        } else {
-          if (sbi + FF_PF < n_sub) prefetch(sbi + FF_PF);
-          if (sbi + 2 < n_sub) fetch(sbi + 2, raw[(sub + 2) % 4]);
-        }
+        cp_take(slot, raw[sub]);
         float2 x[FF_SUB];
         if (FAST) {
 #pragma unroll
           for (int j = 0; j < FF_SUB / 2; j++) {
-            x[2 * j] = XU ? cu8_pair_x(raw[sub].w[j], 0) : cu8_pair(raw[sub].w[j], 0);
-            x[2 * j + 1] = XU ? cu8_pair_x(raw[sub].w[j], 1) : cu8_pair(raw[sub].w[j], 1);
+            x[2 * j] = cu8_pair_x(raw[sub].w[j], 0);
+            x[2 * j + 1] = cu8_pair_x(raw[sub].w[j], 1);
           }
         } else {
           float xr[FF_SUB], xi[FF_SUB];
           ld.template convert<FF_SUB>(p.src, qb + (long long)sbi * FF_SUB, sbi, raw[sub], xr, xi);
 #pragma unroll
           for (int i = 0; i < FF_SUB; i++)
-            x[i] = XU ? make_float2(fmaf(xr[i], 128.0f, CU8_XBIAS), fmaf(xi[i], 128.0f, CU8_XBIAS)) : make_float2(xr[i], xi[i]);
+            x[i] = make_float2(fmaf(xr[i], 128.0f, CU8_XBIAS), fmaf(xi[i], 128.0f, CU8_XBIAS));
         }
-        if (CPA) cp_issue(sbi + F6_CPD, slot);
-        if (DC != DC_NONE) {
+        cp_issue(sbi + F6_CPD, slot);
 #pragma unroll
-          for (int i = 0; i < FF_SUB; i++) {
-            const float2 y = ffma2(nalpha, v, x[i]);
-            v = ffma2(cpole, v, x[i]);
-            x[i] = y;
-          }
+        for (int i = 0; i < FF_SUB; i++) {
+          const float2 y = ffma2(nalpha, v, x[i]);
+          v = ffma2(cpole, v, x[i]);
+          x[i] = y;
         }
         float2 a[8], b[4];
         sa.template run<false>(p.hb[0], x, a, 1.0f);
@@ -485,15 +379,11 @@ __global__ void __launch_bounds__(FF_THREADS, 2) front6_kernel(Front6Params fp) 
     if (it >= own_lo && it < own_hi) dst[(ob32 + (unsigned)it) & dmask] = f[0];
   };
   for (int it = 0; it < n_it; it++) {
-    if (DC == DC_ZSR) {
-      if (it == cap_it) p.sums[gid] = v;
-    }
+    if (it == cap_it) p.sums[gid] = v;
     if (4 * it >= ld.fast_lo && 4 * it + 3 < ld.fast_hi) iteration(it, std::true_type());
     else iteration(it, std::false_type());
   }
-  if (DC == DC_ZSR) {
-    if (cap_it >= n_it) p.sums[gid] = v;
-  }
+  if (cap_it >= n_it) p.sums[gid] = v;
 }
 
 }  // namespace pmr

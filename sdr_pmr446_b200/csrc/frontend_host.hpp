@@ -65,11 +65,6 @@ inline cascade_fn pick_cascade(int src, int dc, bool arb, const int* ms, int* G)
   } else {
     if (dc == DC_NONE && src == SRC_RING && is(10, 0, 0, 0)) { *G = 8; return cfn<SRC_RING, DC_NONE, 8, 10, 0, 0, 0, true>(); }
     if (dc == DC_NONE && src == SRC_RING && is(0, 0, 0, 0)) { *G = 8; return cfn<SRC_RING, DC_NONE, 8, 0, 0, 0, 0, true>(); }
-    // [5, 10] + dynamic-phase resampler in ONE launch (1.024 Msps -> 200 kHz, the reference's own plan): the DC blocker's
-    // state per segment comes from a pre-pass over the raw input (DC_SCAN: +2 GB read), which is cheaper than the 256 kHz
-    // ring round trip and the second launch it replaces
-    if (dc == DC_SCAN && src == SRC_CU8 && is(5, 10, 0, 0)) return cfn<SRC_CU8, DC_SCAN, 16, 5, 10, 0, 0, true>();
-    if (dc == DC_SCAN && src == SRC_CF32 && is(5, 10, 0, 0)) return cfn<SRC_CF32, DC_SCAN, 16, 5, 10, 0, 0, true>();
     if (dc == DC_SCAN && src == SRC_CU8 && is(0, 0, 0, 0)) return cfn<SRC_CU8, DC_SCAN, 16, 0, 0, 0, 0, true>();
     if (dc == DC_SCAN && src == SRC_CF32 && is(0, 0, 0, 0)) return cfn<SRC_CF32, DC_SCAN, 16, 0, 0, 0, 0, true>();
     if (dc == DC_NONE && src == SRC_CF32 && is(0, 0, 0, 0)) return cfn<SRC_CF32, DC_NONE, 16, 0, 0, 0, 0, true>();
@@ -100,8 +95,7 @@ inline bool cut_groups(std::vector<int> order, std::vector<std::vector<int>>* gr
 struct Frontend {
   // How a plan is cut into launches (pure host logic, also exported through pmr446_describe_frontend for the CPU tests):
   // groups[0 .. n-2] are half-band groups, groups[n-1] is the resampler's launch (with the last half-band, or empty).
-  static int plan_groups(const design::MsresampPlan& plan, int in_fmt, std::vector<std::vector<int>>* groups, bool* fused, bool* front6 = nullptr,
-                         bool with_dc_hint = true) {
+  static int plan_groups(const design::MsresampPlan& plan, int in_fmt, std::vector<std::vector<int>>* groups, bool* fused, bool* front6 = nullptr) {
     if (front6) *front6 = false;
     // execution-order stage list: plan.m[stages-1] runs first
     std::vector<int> order;
@@ -112,25 +106,16 @@ struct Frontend {
     // the lowest rate (half the traffic) and the per-lane filter-bank gathers no longer share a kernel with the 58-register
     // m = 10 window.  A single half-band also runs on its own (the resampler kernel with a half-band only reads a ring).
     // Otherwise the last half-band goes with the resampler (tiled kernel when the phase has period 2).
+    // (The two launches measured 1.35 + 1.14 ms at 1024 x 1.024 Msps against 0.57 + 2.34 ms for ONE launch of [5, 10] +
+    // resampler behind a DC pre-pass over the raw input.)
     const bool split_arb = (order.size() == 2 && order[0] == 5 && order[1] == 10 && plan.step != (3u << 23)) || order.size() == 1;
-    // PMR446_FRONTEND=one runs that plan as ONE launch instead (DC pre-pass + [5, 10] + resampler, see pick_cascade): measured
-    // 0.57 + 2.34 ms against 1.35 + 1.14 ms for the two launches at 1024 x 1.024 Msps, so it is not the default
-    const char* fe_env0 = getenv("PMR446_FRONTEND");
-    const bool one_launch = order.size() == 2 && order[0] == 5 && order[1] == 10 && plan.step != (3u << 23) && with_dc_hint &&
-                            fe_env0 && strcmp(fe_env0, "one") == 0;
-    // 2.4 Msps cu8 -> 200 kHz ([3, 5, 10] + rate 2/3): everything in ONE launch, no intermediate ring (frontend_fused.cuh).
-    // PMR446_FRONTEND=split keeps round 1's two launches (cascade -> 600 kHz ring -> tiled half-band + resampler) for A/B runs.
-    const char* fe_env = getenv("PMR446_FRONTEND");
-    *fused = in_fmt == PMR446_FMT_CU8 && order.size() == 3 && order[0] == 3 && order[1] == 5 && order[2] == 10 &&
-             plan.step == (3u << 23) && !(fe_env && strcmp(fe_env, "split") == 0);
+    // 2.4 Msps cu8 -> 200 kHz ([3, 5, 10] + rate 2/3): everything in ONE launch, no intermediate ring (frontend_fused.cuh)
+    *fused = in_fmt == PMR446_FMT_CU8 && order.size() == 3 && order[0] == 3 && order[1] == 5 && order[2] == 10 && plan.step == (3u << 23);
     // deep cu8 plans (dsd_in: 3,3,3,3,3,5,10 at 2.4 Msps, 3,3,3,3,5,10 at 1.024 Msps): the first six stages in one launch
     const bool six = front6 && in_fmt == PMR446_FMT_CU8 && (order.size() == 6 || order.size() == 7) && order[0] == 3 && order[1] == 3 &&
-                     order[2] == 3 && order[3] == 3 && ((order[4] == 3 && order[5] == 5) || (order[4] == 5 && order[5] == 10)) &&
-                     !(fe_env && strcmp(fe_env, "split") == 0);
+                     order[2] == 3 && order[3] == 3 && ((order[4] == 3 && order[5] == 5) || (order[4] == 5 && order[5] == 10));
     if (*fused) {
       groups->push_back(order);
-    } else if (one_launch) {
-      groups->push_back(order);   // the only level: [5, 10] + resampler, DC_SCAN
     } else if (six) {
       *front6 = true;
       groups->emplace_back(order.begin(), order.begin() + 6);
@@ -231,7 +216,9 @@ struct Frontend {
     if (plan.bits > 8) return fail(PMR446_EINVAL, "resampler filter bank larger than 256 rows");
     std::vector<std::vector<int>> groups;   // pre-launch groups, then the arb launch
     bool want_fused = false, want_front6 = false;
-    if (int rc = plan_groups(plan, in_fmt, &groups, &want_fused, &want_front6, dc)) return rc;
+    if (int rc = plan_groups(plan, in_fmt, &groups, &want_fused, &want_front6)) return rc;
+    // the fused and front6 kernels always run the DC blocker (every caller that passes cu8 asks for it)
+    if ((want_fused || want_front6) && !dc) return fail(PMR446_EINVAL, "internal: cu8 front end planned without the DC blocker");
     levels.resize(groups.size());
     long long max_in = max_chunk;
     int stage_cursor = (int)plan.stages - 1;  // index into plan.m / plan.hb of the next stage to place
@@ -281,7 +268,6 @@ struct Frontend {
         L.halo = (halo + L.D + FF_G - 1) / FF_G * FF_G;
         int sl = 6144;
         while (sl > 1536 && (long long)S * ((max_in + sl - 1) / sl) < 148LL * 256) sl >>= 1;
-        if (getenv("PMR446_FF_SEG")) sl = atoi(getenv("PMR446_FF_SEG"));   // tuning probe: 1536 / 3072 / 6144 / 12288
         L.seg_len = sl;
         for (int r = 0; r < 2; r++) {
           const unsigned row = (unsigned)((((unsigned long long)r * plan.step) & ((1u << 24) - 1)) >> (24 - plan.bits));
@@ -375,11 +361,7 @@ struct Frontend {
   // Consumes n raw samples per stream ([n_in, n_in + n)); afterwards n_out is the absolute
   // number of output samples in the `out` ring.
   // the cu8 kernels that run the DC recurrence on X = u8 - 127 (cu8_pair_x): sums / v_lag in X units, 1 / 128 in the scale
-  static bool integer_units(const Level& L) { return L.dc == DC_ZSR && ((L.fused && !fused_lut()) || L.front6); }
-  static bool fused_lut() {   // tuning probe: table look-up conversion (x units) instead of the integer-unit recurrence
-    static const bool on = getenv("PMR446_FF_CVT") && strcmp(getenv("PMR446_FF_CVT"), "lut") == 0;
-    return on;
-  }
+  static bool integer_units(const Level& L) { return L.dc == DC_ZSR && (L.fused || L.front6); }
   // few streams with many segments: one block per stream; otherwise one warp per stream
   void launch_dc_scan(const DcScanParams& sp, cudaStream_t st) const {
     if (S <= 64 && sp.nseg > 128) dc_scan_block_kernel<<<S, 256, 0, st>>>(sp);
@@ -524,15 +506,10 @@ struct Frontend {
           memcpy(cp.hb, L.hb, sizeof cp.hb);
           memcpy(fp.hb5, L.hb[4], sizeof fp.hb5);
           memcpy(fp.hb6, L.hb[5], sizeof fp.hb6);
-          const bool e3 = L.ms[4] == 3;
-          static const bool f6_cpa = !(getenv("PMR446_F6_CPA") && atoi(getenv("PMR446_F6_CPA")) == 0);   // cp.async staging as in the fused kernel (2.90 -> 2.87 ms per dsd_in step); 0: register loads
+          // cp.async staging as in the fused kernel (2.87 ms per dsd_in step against 2.90 ms with register loads)
           const size_t f6_smem = (size_t)F6_CPD * 32 * FF_THREADS;
-          if (L.dc == DC_ZSR && e3 && f6_cpa) front6_kernel<DC_ZSR, 3, 5, true><<<blocks, FF_THREADS, f6_smem, st>>>(fp);
-          else if (L.dc == DC_ZSR && f6_cpa) front6_kernel<DC_ZSR, 5, 10, true><<<blocks, FF_THREADS, f6_smem, st>>>(fp);
-          else if (L.dc == DC_ZSR && e3) front6_kernel<DC_ZSR, 3, 5><<<blocks, FF_THREADS, 0, st>>>(fp);
-          else if (L.dc == DC_ZSR) front6_kernel<DC_ZSR, 5, 10><<<blocks, FF_THREADS, 0, st>>>(fp);
-          else if (e3) front6_kernel<DC_NONE, 3, 5><<<blocks, FF_THREADS, 0, st>>>(fp);
-          else front6_kernel<DC_NONE, 5, 10><<<blocks, FF_THREADS, 0, st>>>(fp);
+          if (L.ms[4] == 3) front6_kernel<3, 5><<<blocks, FF_THREADS, f6_smem, st>>>(fp);
+          else front6_kernel<5, 10><<<blocks, FF_THREADS, f6_smem, st>>>(fp);
           *launches += 1;
           tm->mark(st, TM_CASCADE0);
           if (out1 > out0) new_out = out1;
@@ -560,23 +537,11 @@ struct Frontend {
           memcpy(cp.hb, L.hb, sizeof cp.hb);
           memcpy(fp.arb, L.arb_rows, sizeof fp.arb);   // (folding cp.scale into these taps saves 6 FMUL2 of 590 and ran 3 % slower)
           fp.w0 = (float)((double)CU8_XBIAS / (double)alpha_eff);
-          static const bool smem3 = getenv("PMR446_FF_VARIANT") && strcmp(getenv("PMR446_FF_VARIANT"), "smem3") == 0;   // tuning probe
-          static const bool lut_cvt = [] {
-            const bool on = fused_lut();
-            if (on) cudaFuncSetAttribute(fused_frontend_kernel<DC_ZSR, 2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FF_LUT_BYTES);
-            return on;
-          }();
-          // raw bytes staged global -> shared memory by cp.async six sub-blocks ahead (2.456 vs 2.486 ms); PMR446_FF_CPA=0: register loads behind an L1 prefetch
-          static const bool cpa = !(getenv("PMR446_FF_CPA") && atoi(getenv("PMR446_FF_CPA")) == 0);
-          static const int thr_env = getenv("PMR446_FF_THREADS") ? atoi(getenv("PMR446_FF_THREADS")) : 0;   // tuning probe: 32 / 64
+          // raw bytes staged global -> shared memory by cp.async six sub-blocks ahead (2.456 ms against 2.486 ms with register loads).
           // 32-thread blocks: the same 8 warps per SM, but the 10.6 "waves" of 128-thread blocks end in a shorter tail (2.62 vs 2.68 ms)
-          const int thr = smem3 ? FF_THREADS : ((thr_env == 64 || thr_env == 128) ? thr_env : 32);
+          const int thr = 32;
           const unsigned fblocks = (unsigned)((threads + thr - 1) / thr);
-          if (L.dc != DC_ZSR) fused_frontend_kernel<DC_NONE><<<fblocks, thr, 0, st>>>(fp);
-          else if (smem3) fused_frontend_kernel<DC_ZSR, 3, true><<<blocks, FF_THREADS, 0, st>>>(fp);
-          else if (lut_cvt) fused_frontend_kernel<DC_ZSR, 2, false, true><<<fblocks, thr, FF_LUT_BYTES, st>>>(fp);
-          else if (cpa) fused_frontend_kernel<DC_ZSR, 2, false, false, true><<<fblocks, thr, (size_t)FF_CPD * 32 * thr, st>>>(fp);
-          else fused_frontend_kernel<DC_ZSR><<<fblocks, thr, 0, st>>>(fp);
+          fused_frontend_kernel<<<fblocks, thr, (size_t)FF_CPD * 32 * thr, st>>>(fp);
           *launches += 1;
           tm->mark(st, TM_CASCADE0);
           if (out1 > out0) new_out = (long long)design::arb_outputs_after((uint64_t)out1, plan.step);

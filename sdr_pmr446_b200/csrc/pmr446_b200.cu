@@ -55,7 +55,7 @@ struct pmr446_batch {
   long long last_f0 = 0, last_ns = 0;   // frame range of the last execute call (pmr446_batch_gather_channel)
   DevBuf d_out_rssi, d_out_edge;
   int fft_halo = AF_HALO;    // overlap of the FFT audio tile (AF_HALO or AF_HALO_LONG)
-  bool fft_audio = false;    // audio / pcm by fast convolution (audio_fft_kernel); the direct-form kernel serves lpcomp
+  bool fft_audio = false;    // audio / pcm by fast convolution (audio_fft4_kernel); the direct-form kernel serves lpcomp
   int au_lead = AU_LEAD_MIN; // lead-in of the direct-form kernel's tiles (audio_lead)
   int de_warm = 0;           // de-emphasis warm-up (deemph_warmup); > 8 selects audio_kernel<true>
   DevBuf d_resp, d_aftw;
@@ -260,6 +260,8 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
   }
   cudaFuncSetAttribute(audio_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
   cudaFuncSetAttribute(audio_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(audio_fft4_kernel<AF_HALO>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF4_SMEM_BYTES);
+  cudaFuncSetAttribute(audio_fft4_kernel<AF_HALO_LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF4_SMEM_BYTES);
   CUDA_TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking));
   CUDA_TRY(cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking));
   CUDA_TRY(cudaStreamCreateWithFlags(&b->out_stream, cudaStreamNonBlocking));
@@ -459,9 +461,7 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
     long long warps = (long long)S * cp.tiles;   // one warp per (stream, frame tile)
     unsigned blocks = (unsigned)((warps * 32 + 127) / 128);
     const bool taps = tp.mag_part || tp.edge;
-    static const bool pipe_regs = getenv("PMR446_CH_PIPE") && atoi(getenv("PMR446_CH_PIPE")) == 1;   // tuning probe
-    if (b->nco_lut && !taps && pipe_regs) channelize16_kernel<true, false, true><<<blocks, 128, 0, st>>>(cp, tp);
-    else if (b->nco_lut && !taps) channelize16_kernel<true, false><<<blocks, 128, 0, st>>>(cp, tp);
+    if (b->nco_lut && !taps) channelize16_kernel<true, false><<<blocks, 128, 0, st>>>(cp, tp);
     else if (b->nco_lut) channelize16_kernel<true, true><<<blocks, 128, 0, st>>>(cp, tp);
     else if (!taps) channelize16_kernel<false, false><<<blocks, 128, 0, st>>>(cp, tp);
     else channelize16_kernel<false, true><<<blocks, 128, 0, st>>>(cp, tp);
@@ -492,9 +492,11 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
       fp.demod_stride = b->demod_cap;
       fp.demod_mask = b->demod_cap - 1;
       fp.rows = S * M;
+      // tiles anchored at the call's first sample: ceil(ns / own) transforms per row instead of one more whenever the call
+      // straddles the absolute grid (3.49 tiles' worth of a 1 s step: 4 instead of 4.49 on average)
       const long long af_own = AF_N - b->fft_halo;
-      fp.tile0 = f0 / af_own;
-      fp.tiles = (int)((f1 + af_own - 1) / af_own - fp.tile0);
+      fp.tiles = (int)((f1 - f0 + af_own - 1) / af_own);
+      fp.tile0 = 0;
       fp.f0 = f0;
       fp.f1 = f1;
       fp.resp = (const float2*)b->d_resp.p;
@@ -502,27 +504,9 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
       fp.audio = out->audio;
       fp.pcm = out->pcm;
       fp.out_ld = out->ld;
-      // four rows per block, all-packed arithmetic (audio_fft4.cuh); PMR446_AUDIO_FFT=2 keeps round 1's two-row kernel (tuning probe)
-      static const bool four = [] {
-        const char* e = getenv("PMR446_AUDIO_FFT");
-        if (e && strcmp(e, "2") == 0) return false;
-        cudaFuncSetAttribute(audio_fft4_kernel<AF_HALO>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF4_SMEM_BYTES);
-        cudaFuncSetAttribute(audio_fft4_kernel<AF_HALO_LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF4_SMEM_BYTES);
-        return true;
-      }();
-      if (four) {
-        // tiles anchored at the call's first sample: ceil(ns / own) transforms per row instead of one more whenever the call
-        // straddles the absolute grid (3.49 tiles' worth of a 1 s step: 4 instead of 4.49 on average)
-        fp.tile0 = 0;
-        fp.tiles = (int)((f1 - f0 + af_own - 1) / af_own);
-        const unsigned fgrid = (unsigned)((long long)((fp.rows + 3) / 4) * fp.tiles);
-        if (b->fft_halo == AF_HALO) audio_fft4_kernel<AF_HALO><<<fgrid, AF_T, AF4_SMEM_BYTES, st>>>(fp);
-        else audio_fft4_kernel<AF_HALO_LONG><<<fgrid, AF_T, AF4_SMEM_BYTES, st>>>(fp);
-      } else {
-        const unsigned fgrid = (unsigned)((long long)((fp.rows + 1) / 2) * fp.tiles);
-        if (b->fft_halo == AF_HALO) audio_fft_kernel<AF_HALO><<<fgrid, AF_T, 0, st>>>(fp);
-        else audio_fft_kernel<AF_HALO_LONG><<<fgrid, AF_T, 0, st>>>(fp);
-      }
+      const unsigned fgrid = (unsigned)((long long)((fp.rows + 3) / 4) * fp.tiles);   // four rows per block (audio_fft4.cuh)
+      if (b->fft_halo == AF_HALO) audio_fft4_kernel<AF_HALO><<<fgrid, AF_T, AF4_SMEM_BYTES, st>>>(fp);
+      else audio_fft4_kernel<AF_HALO_LONG><<<fgrid, AF_T, AF4_SMEM_BYTES, st>>>(fp);
       b->launches++;
       b->timer.mark(st, TM_AUDIO);
     }
@@ -792,7 +776,7 @@ extern "C" int pmr446_describe_frontend(float rate, float as, int in_fmt, int wi
   design::MsresampPlan p = design::msresamp_plan(rate, as);
   std::vector<std::vector<int>> groups;
   bool fused = false, front6 = false;
-  if (int rc = Frontend::plan_groups(p, in_fmt, &groups, &fused, &front6, with_dc != 0)) return rc;
+  if (int rc = Frontend::plan_groups(p, in_fmt, &groups, &fused, &front6)) return rc;
   std::string out;
   for (size_t l = 0; l < groups.size(); l++) {
     const bool arb = l + 1 == groups.size();

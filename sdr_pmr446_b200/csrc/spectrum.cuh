@@ -471,9 +471,8 @@ struct Waterfall {
     // enough (stream, part) blocks to fill the GPU: one block needs nfft * 20 bytes of shared memory (block-per-transform
     // kernel) or nfft * 8 * (1 + 2 * 8 warps) bytes (warp-per-transform kernel, nfft <= 1024)
     {
-      const char* env = getenv("PMR446_WATERFALL");   // "generic" keeps round 1's shared-memory kernels (A/B runs)
       const unsigned P = W / 8;
-      if (W % 8 == 0 && (P == 8 || P == 10 || P == 12 || P == 15 || P == 16 || P == 20) && !(env && strcmp(env, "generic") == 0)) {
+      if (W % 8 == 0 && (P == 8 || P == 10 || P == 12 || P == 15 || P == 16 || P == 20)) {
         fast_p = (int)P;
         for (unsigned m = 0; m < P; m++) {
           const double a = -2.0 * M_PI * (double)m / (double)P;

@@ -188,3 +188,15 @@ def test_makefile_lists_every_kernel_header():
     hdrs = set(re.search(r"^HDRS\s*=\s*(.*)$", mk, re.M).group(1).split())
     have = {os.path.basename(p) for p in glob.glob(os.path.join(root, "*.cuh")) + glob.glob(os.path.join(root, "*.hpp"))}
     assert have <= hdrs, sorted(have - hdrs)
+
+
+def test_library_reads_no_environment_variables():
+    """The library's behaviour is a function of its configuration struct alone, not of the environment of the process that loads it."""
+    import glob
+    import os
+    import re
+    root = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "sdr_pmr446_b200", "csrc")
+    srcs = [p for ext in ("*.cu", "*.cuh", "*.hpp") for p in glob.glob(os.path.join(root, ext))]
+    assert srcs
+    hits = [os.path.basename(p) for p in srcs if re.search(r"\bgetenv\b", open(p).read())]
+    assert not hits, hits

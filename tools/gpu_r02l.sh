@@ -1,17 +1,16 @@
 #!/bin/bash
-# round 2 evidence run: GPU suite, bench (fused and split front end), other configs, launch list, ncu captures of the step's kernels
+# round 2 evidence run: GPU suite, bench, other configs, launch list, ncu captures of the step's kernels
 T=${1:-r02l}
 mkdir -p gpurun_out
 python -m pytest tests -m gpu -x -q > gpurun_out/pytest_gpu_$T.log 2>&1; echo "pytest exit $?" >> gpurun_out/pytest_gpu_$T.log
 python bench.py --steps 10 --warmup 3 > gpurun_out/bench_$T.json 2> gpurun_out/bench_$T.err
-PMR446_FRONTEND=split python bench.py --steps 10 --warmup 3 > gpurun_out/bench_${T}_split.json 2> gpurun_out/bench_${T}_split.err
 for c in cfg1 cfg2 cfg4 receiver; do python bench.py --config $c --steps 5 --warmup 3 > gpurun_out/bench_${T}_$c.json 2> gpurun_out/bench_${T}_$c.err; done
 ncu --metrics gpu__time_duration.sum --clock-control none -s 40 -c 60 --csv --log-file gpurun_out/launches_$T.csv python bench.py --steps 2 --warmup 1 > gpurun_out/bench_under_ncu_$T.log 2>&1
 bash tools/gpu_prof6.sh fused_frontend ff_$T python tools/quick_bench.py --streams 1024 --steps 1
 bash tools/gpu_prof6.sh channelize16 ch_$T python tools/quick_bench.py --streams 1024 --steps 1
 bash tools/gpu_prof6.sh audio_fft af_$T python tools/quick_bench.py --streams 1024 --steps 1
 tail -3 gpurun_out/pytest_gpu_$T.log
-for f in bench_$T bench_${T}_split bench_${T}_cfg1 bench_${T}_cfg2 bench_${T}_cfg4 bench_${T}_receiver; do python - <<PY
+for f in bench_$T bench_${T}_cfg1 bench_${T}_cfg2 bench_${T}_cfg4 bench_${T}_receiver; do python - <<PY
 import json
 try:
     d=json.load(open('gpurun_out/$f.json'))

@@ -3,8 +3,8 @@
  * (/root/reference/src/sdr_pmr446.c:795-823, :881-902, :910-913) replaced by ONE coarse call per
  * chunk, pmr446_batch_execute(), for any number of capture files processed side by side.
  *
- * usage: pmr446_batch_file [-r fs_in] [-8] [-g gain] [-l] [-n chunk] -o out_prefix capture0 [capture1 ...]
- *   -8  captures are cu8 (default cf32);  writes <out_prefix>.<stream>.<channel>.s16 for all 16 channels
+ * usage: pmr446_batch_file [-r fs_in] [-8 | -16 | -s8] [-g gain] [-l] [-n chunk] -o out_prefix capture0 [capture1 ...]
+ *   -8 / -16 / -s8  captures are cu8 / cs16 / cs8 (default cf32);  writes <out_prefix>.<stream>.<channel>.s16 for all 16 channels
  */
 #include <stdint.h>
 #include <stdio.h>
@@ -23,17 +23,19 @@ int main(int argc, char **argv) {
   for (int i = 1; i < argc; i++) {
     if (!strcmp(argv[i], "-r") && i + 1 < argc) cfg.fs_in = (unsigned)atol(argv[++i]);
     else if (!strcmp(argv[i], "-8")) cfg.in_fmt = PMR446_FMT_CU8;
+    else if (!strcmp(argv[i], "-16")) cfg.in_fmt = PMR446_FMT_CS16;
+    else if (!strcmp(argv[i], "-s8")) cfg.in_fmt = PMR446_FMT_CS8;
     else if (!strcmp(argv[i], "-g") && i + 1 < argc) cfg.audio_gain = (float)atof(argv[++i]);
     else if (!strcmp(argv[i], "-l")) cfg.lowpass = 1;
     else if (!strcmp(argv[i], "-n") && i + 1 < argc) cfg.max_chunk = (unsigned)atol(argv[++i]);
     else if (!strcmp(argv[i], "-o") && i + 1 < argc) prefix = argv[++i];
     else if (nfiles < 256) files[nfiles++] = argv[i];
   }
-  if (!prefix || nfiles == 0) { fprintf(stderr, "usage: %s [-r fs] [-8] [-g gain] [-l] [-n chunk] -o prefix capture...\n", argv[0]); return 1; }
+  if (!prefix || nfiles == 0) { fprintf(stderr, "usage: %s [-r fs] [-8 | -16 | -s8] [-g gain] [-l] [-n chunk] -o prefix capture...\n", argv[0]); return 1; }
   cfg.n_streams = nfiles;
   pmr446_batch *b = NULL;
   if (pmr446_batch_create(&cfg, &b) != PMR446_OK) { fprintf(stderr, "pmr446_batch_create: %s\n", pmr446_last_error()); return 2; }
-  const size_t bps = cfg.in_fmt == PMR446_FMT_CU8 ? 2 : 8;
+  const size_t bps = (size_t)pmr446_bytes_per_sample(cfg.in_fmt);
   const long long ld = pmr446_batch_max_ns(b);
   uint8_t *iq = (uint8_t *)calloc((size_t)nfiles * cfg.max_chunk, bps);
   int16_t *pcm = (int16_t *)calloc((size_t)nfiles * 16 * ld, 2);

@@ -5,13 +5,14 @@
  * queueing audio (/root/reference/src/sdr_pmr446.c:795-913) is ONE call, pmr446_receiver_execute().
  *
  * Replaces around that call:
- *   SoapySDR readStream (src/shared.c, :788-793)      -> fread of a cu8 / cf32 capture (or stdin) into pinned memory
+ *   SoapySDR readStream (src/shared.c, :788-793)      -> fread of a cu8 / cs16 / cs8 / cf32 capture (or stdin) into pinned memory
  *   RtAudio output callback (:520-593)                -> WAV writer (s16 or float32, 12.5 kHz mono)
  *   LOG lines (:613-626, :838, :852, :861)            -> the same messages from pmr446_rx_status.events
  *   waterfall row + footer (:630-666, :914-918)       -> printed from the ascii row and the status
  *
- * usage: pmr446_rx_file [-r fs_in] [-8] [-g audio_gain] [-s squelch_dB] [-m excluded,channels] [-L] [-l]
+ * usage: pmr446_rx_file [-r fs_in] [-8 | -16 | -s8] [-g audio_gain] [-s squelch_dB] [-m excluded,channels] [-L] [-l]
  *                       [-w W] [-n chunk] [-f] -o out.wav capture|-
+ *   -8 cu8, -16 cs16, -s8 cs8 capture (default cf32)
  */
 #include <math.h>
 #include <stdint.h>
@@ -72,6 +73,8 @@ int main(int argc, char **argv) {
   for (int i = 1; i < argc; i++) {
     if (!strcmp(argv[i], "-r") && i + 1 < argc) cfg.chain.fs_in = (unsigned)atol(argv[++i]);
     else if (!strcmp(argv[i], "-8")) cfg.chain.in_fmt = PMR446_FMT_CU8;
+    else if (!strcmp(argv[i], "-16")) cfg.chain.in_fmt = PMR446_FMT_CS16;
+    else if (!strcmp(argv[i], "-s8")) cfg.chain.in_fmt = PMR446_FMT_CS8;
     else if (!strcmp(argv[i], "-g") && i + 1 < argc) cfg.chain.audio_gain = (float)atof(argv[++i]);
     else if (!strcmp(argv[i], "-s") && i + 1 < argc) cfg.squelch_level = (float)atof(argv[++i]);
     else if (!strcmp(argv[i], "-m") && i + 1 < argc) {   /* comma-separated 1-based channels to exclude (:283-297) */
@@ -88,7 +91,7 @@ int main(int argc, char **argv) {
     else in_path = argv[i];
   }
   if (!out_path || !in_path) {
-    fprintf(stderr, "usage: %s [-r fs] [-8] [-g gain] [-s squelch] [-m ch,ch] [-L] [-l] [-w W] [-n chunk] [-f] -o out.wav capture|-\n", argv[0]);
+    fprintf(stderr, "usage: %s [-r fs] [-8 | -16 | -s8] [-g gain] [-s squelch] [-m ch,ch] [-L] [-l] [-w W] [-n chunk] [-f] -o out.wav capture|-\n", argv[0]);
     return 1;
   }
   pmr446_receiver *rx = NULL;
@@ -96,7 +99,7 @@ int main(int argc, char **argv) {
   FILE *fi = strcmp(in_path, "-") ? fopen(in_path, "rb") : stdin;
   FILE *fo = fopen(out_path, "wb");
   if (!fi || !fo) { perror(fi ? out_path : in_path); return 2; }
-  const size_t bps = cfg.chain.in_fmt == PMR446_FMT_CU8 ? 2 : 8;
+  const size_t bps = (size_t)pmr446_bytes_per_sample(cfg.chain.in_fmt);
   const unsigned W = cfg.chain.waterfall, M = cfg.chain.num_channels;
   const long long ld = pmr446_receiver_max_ns(rx);
   void *iq = NULL;

@@ -42,12 +42,20 @@ extern "C" {
 
 #define PMR446_FMT_CF32 0      /* interleaved float32 I,Q  (SOAPY_SDR_CF32, src/shared.c:62) */
 #define PMR446_FMT_CU8 1       /* interleaved uint8 I,Q, converted as (u8 - 127.4)/128 */
+#define PMR446_FMT_CS16 2      /* interleaved little-endian int16 I,Q, converted as x / 32768 (exact) */
+#define PMR446_FMT_CS8 3       /* interleaved int8 I,Q, converted as x / 128 (exact) */
+
+/* Bytes per IQ sample of an in_fmt (2, 8, 4, 2 for the formats above): the unit of n and the layout of iq / iq_stride in
+ * every execute call.  Any other value is read as cf32 (8). */
+int pmr446_bytes_per_sample(int in_fmt);
 
 typedef struct {
   int n_streams;           /* independent IQ streams processed per call */
   int device;              /* CUDA device ordinal; -1 = current device */
   unsigned fs_in;          /* input sample rate, Hz (SDR_SAMPLERATE, include/sdr_pmr446.h:13) */
-  int in_fmt;              /* PMR446_FMT_* */
+  int in_fmt;              /* PMR446_FMT_*; any other value is read as cf32.  cs16 and cs8 run the cf32 front end on
+                              the exactly converted samples, so their results are bitwise those of cf32 input x / 32768
+                              or x / 128 */
   unsigned num_channels;   /* NUM_CHANNELS, src/sdr_pmr446.c:23 (16); any M in [2, 4096] whose generic channelizer
                               (56 M bytes of shared memory) fits the device's opt-in per-block limit (all of them on a B200) */
   unsigned channel_width;  /* CHANNEL_WIDTH_HZ, :22 (12500) */
@@ -199,7 +207,7 @@ typedef struct {
   int n_streams;
   int device;
   unsigned fs_in;          /* SDR_SAMPLERATE, include/dsd_in.h:11 */
-  int in_fmt;
+  int in_fmt;              /* PMR446_FMT_*, as in pmr446_config */
   unsigned fs_sig;         /* SIG_SAMPLERATE, src/dsd_in.c:23 (12500) */
   unsigned fs_audio;       /* AUDIO_SAMPLERATE, :22 (48000) */
   unsigned max_chunk;      /* SDR_INPUT_CHUNK, :25 (200000) */
@@ -244,7 +252,9 @@ int pmr446_design_asgram_window(unsigned W, float *w);
 unsigned pmr446_design_nco_dtheta(float dtheta);
 /* How msresamp_crcf_create(rate, as) (src/sdr_pmr446.c:425-426, src/dsd_in.c:100) is cut into kernel launches for the
  * given input format, e.g. "fused[3,5,10]+arb" or "cascade[3,3,3,3] | cascade[3,5] | tile[10]+arb"; every decimating
- * rate liquid accepts (0 < rate <= 1) has a plan.  buf receives the NUL-terminated description. */
+ * rate liquid accepts (0 < rate <= 1) has a plan.  buf receives the NUL-terminated description.  With with_dc = 1 (every
+ * chain runs the DC blocker) PMR446_FMT_CS16 and PMR446_FMT_CS8 get the same plan as PMR446_FMT_CF32; the stand-alone
+ * resampler without the DC blocker (with_dc = 0) exists for cf32 only. */
 int pmr446_describe_frontend(float rate, float as, int in_fmt, int with_dc, char *buf, int len);
 /* Total msresamp outputs after n_in inputs since stream start (decimating rates). */
 long long pmr446_count_resampled(float rate, float as, long long n_in);

@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(_HERE, "libpmr446_b200.so")
 _LIB = None
 
 OK, EINVAL, ENODEV, ECUDA, ERANGE, ENOMEM = 0, -1, -2, -3, -4, -5
-FMT_CF32, FMT_CU8 = 0, 1
+FMT_CF32, FMT_CU8, FMT_CS16, FMT_CS8 = 0, 1, 2, 3
 
 
 class Config(C.Structure):
@@ -75,7 +75,7 @@ EXPORTS = [
     "dsd446_default_config", "dsd446_batch_create", "dsd446_batch_destroy", "dsd446_batch_max_res",
     "dsd446_batch_max_out", "dsd446_batch_last_launches", "dsd446_batch_execute", "dsd446_batch_execute_device", "dsd446_batch_reset",
     "pmr446_design_msresamp", "pmr446_design_pfbch", "pmr446_design_asgram_window", "pmr446_design_nco_dtheta",
-    "pmr446_count_resampled", "pmr446_describe_frontend",
+    "pmr446_count_resampled", "pmr446_describe_frontend", "pmr446_bytes_per_sample",
 ]
 
 
@@ -150,8 +150,14 @@ def lib():
         L.pmr446_count_resampled.argtypes = [C.c_float, C.c_float, C.c_longlong]
         L.pmr446_count_resampled.restype = C.c_longlong
         L.pmr446_describe_frontend.argtypes = [C.c_float, C.c_float, C.c_int, C.c_int, C.c_char_p, C.c_int]
+        L.pmr446_bytes_per_sample.argtypes = [C.c_int]
         _LIB = L
     return _LIB
+
+
+def bytes_per_sample(in_fmt):
+    """Bytes per IQ sample of an in_fmt, as the library reads it (cu8 and cs8 2, cs16 4, anything else cf32, 8)."""
+    return lib().pmr446_bytes_per_sample(int(in_fmt))
 
 
 class Pmr446Error(RuntimeError):

@@ -13,9 +13,19 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import FMT_CF32, FMT_CU8, Config, Outputs, check, lib
+from ._lib import FMT_CF32, FMT_CS8, FMT_CS16, FMT_CU8, Config, Outputs, bytes_per_sample, check, lib  # noqa: F401 (formats re-exported)
 
 PMR_OUTPUTS = ("res", "chan", "demod", "lpcomp", "audio", "pcm")
+
+
+def _samples(iq, bps):
+    """IQ samples per row of a host array in the handle's format (any dtype: the row is read as bytes)."""
+    return iq.shape[1] * iq.itemsize // bps
+
+
+def _columns(chunk, iq, bps):
+    """Array columns that hold `chunk` IQ samples."""
+    return chunk * bps // iq.itemsize
 
 
 def default_config(**kw):
@@ -39,7 +49,7 @@ class PmrBatch:
         self.M = self.cfg.num_channels
         self.max_res = lib().pmr446_batch_max_res(self.h)
         self.max_ns = lib().pmr446_batch_max_ns(self.h)
-        self.bytes_per_sample = 2 if self.cfg.in_fmt == FMT_CU8 else 8
+        self.bytes_per_sample = bytes_per_sample(self.cfg.in_fmt)
 
     def close(self):
         if getattr(self, "h", None) and lib is not None:
@@ -74,12 +84,12 @@ class PmrBatch:
 
     # ---- host buffers ------------------------------------------------------------------------
     def execute(self, iq, want=PMR_OUTPUTS):
-        """iq: [S, n*2] uint8 (cu8) or [S, n] complex64 (cf32).  Returns dict of numpy arrays."""
+        """iq: [S, n*2] uint8 (cu8), int16 (cs16) or int8 (cs8), or [S, n] complex64 (cf32).  Returns dict of numpy arrays."""
         iq = np.ascontiguousarray(iq)
         if iq.ndim == 1:
             iq = iq[None, :]
         assert iq.shape[0] == self.S
-        n = iq.shape[1] // 2 if self.cfg.in_fmt == FMT_CU8 else iq.shape[1]
+        n = _samples(iq, self.bytes_per_sample)
         S, M, ld, rld = self.S, self.M, self.max_ns, self.max_res
         bufs = {}
         out = Outputs()
@@ -122,7 +132,7 @@ class PmrBatch:
         chunk = chunk or self.cfg.max_chunk
         if iq.ndim == 1:
             iq = iq[None, :]
-        step = 2 * chunk if self.cfg.in_fmt == FMT_CU8 else chunk
+        step = _columns(chunk, iq, self.bytes_per_sample)
         parts = [self.execute(iq[:, o:o + step], want) for o in range(0, iq.shape[1], step)]
         r = {"ny": sum(p["ny"] for p in parts), "ns": sum(p["ns"] for p in parts)}
         for k in parts[0]:
@@ -178,6 +188,7 @@ class PmrReceiver:
         self.S = self.cfg.chain.n_streams
         self.M = self.cfg.chain.num_channels
         self.max_ns = lib().pmr446_receiver_max_ns(self.h)
+        self.bytes_per_sample = bytes_per_sample(self.cfg.chain.in_fmt)
 
     def close(self):
         if getattr(self, "h", None) and lib is not None:
@@ -203,7 +214,7 @@ class PmrReceiver:
         if iq.ndim == 1:
             iq = iq[None, :]
         assert iq.shape[0] == self.S
-        n = iq.shape[1] // 2 if self.cfg.chain.in_fmt == FMT_CU8 else iq.shape[1]
+        n = _samples(iq, self.bytes_per_sample)
         S, M, ld = self.S, self.M, self.max_ns
         status = (_lib.RxStatus * S)()
         bufs = {"rssi": np.zeros((S, M), np.float32), "audio": np.zeros((S, ld), np.float32), "pcm": np.zeros((S, ld), np.int16),
@@ -248,7 +259,7 @@ class PmrReceiver:
         chunk = chunk or self.cfg.chain.max_chunk
         if iq.ndim == 1:
             iq = iq[None, :]
-        step = 2 * chunk if self.cfg.chain.in_fmt == FMT_CU8 else chunk
+        step = _columns(chunk, iq, self.bytes_per_sample)
         return [self.execute(iq[:, o:o + step]) for o in range(0, iq.shape[1], step)]
 
 
@@ -273,6 +284,7 @@ class DsdBatch:
         self.S = self.cfg.n_streams
         self.max_res = lib().dsd446_batch_max_res(self.h)
         self.max_out = lib().dsd446_batch_max_out(self.h)
+        self.bytes_per_sample = bytes_per_sample(self.cfg.in_fmt)
 
     def close(self):
         if getattr(self, "h", None) and lib is not None:
@@ -296,7 +308,7 @@ class DsdBatch:
         if iq.ndim == 1:
             iq = iq[None, :]
         assert iq.shape[0] == self.S
-        n = iq.shape[1] // 2 if self.cfg.in_fmt == FMT_CU8 else iq.shape[1]
+        n = _samples(iq, self.bytes_per_sample)
         S = self.S
         res = np.zeros((S, self.max_res), np.complex64)
         fm = np.zeros((S, self.max_res), np.float32)
@@ -313,7 +325,7 @@ class DsdBatch:
         chunk = chunk or self.cfg.max_chunk
         if iq.ndim == 1:
             iq = iq[None, :]
-        step = 2 * chunk if self.cfg.in_fmt == FMT_CU8 else chunk
+        step = _columns(chunk, iq, self.bytes_per_sample)
         parts = [self.execute(iq[:, o:o + step]) for o in range(0, iq.shape[1], step)]
         r = {"ny": sum(p["ny"] for p in parts), "nz": sum(p["nz"] for p in parts)}
         for k in ("res", "fm", "audio", "pcm"):

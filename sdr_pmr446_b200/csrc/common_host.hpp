@@ -45,6 +45,25 @@ inline int select_device(int device) {
   return 0;
 }
 
+// The input formats (pmr446_config::in_fmt): bytes per IQ sample and the loader of the front end's first launch.  Every
+// value that is not one of the integer formats is read as cf32.
+inline int fmt_bytes_per_sample(int in_fmt) {
+  switch (in_fmt) {
+    case PMR446_FMT_CU8: return 2;
+    case PMR446_FMT_CS8: return 2;
+    case PMR446_FMT_CS16: return 4;
+    default: return 8;
+  }
+}
+inline int fmt_source(int in_fmt) {
+  switch (in_fmt) {
+    case PMR446_FMT_CU8: return SRC_CU8;
+    case PMR446_FMT_CS8: return SRC_CS8;
+    case PMR446_FMT_CS16: return SRC_CS16;
+    default: return SRC_CF32;
+  }
+}
+
 inline long long next_pow2(long long v) {
   long long p = 1;
   while (p < v) p <<= 1;

@@ -188,7 +188,7 @@ extern "C" int dsd446_batch_execute(dsd446_batch* b, const void* iq, long long i
   cudaSetDevice(b->device);
   cudaStream_t st = b->own_stream;
   const int S = b->S;
-  const size_t bps = b->cfg.in_fmt == PMR446_FMT_CU8 ? 2 : 8;
+  const size_t bps = (size_t)fmt_bytes_per_sample(b->cfg.in_fmt);
   const long long in_row = (long long)((b->cfg.max_chunk * bps + 63) / 64 * 64);
   int rc;
   if ((rc = b->d_in.ensure((size_t)S * in_row))) return rc;

@@ -1,4 +1,4 @@
-// Front-end kernels: cu8/cf32 load -> DC blocker -> half-band decimator cascade -> arbitrary
+// Front-end kernels: cu8/cf32/cs16/cs8 load -> DC blocker -> half-band decimator cascade -> arbitrary
 // resampler.  Replaces iirfilt_crcf_execute_block + msresamp_crcf_execute of the reference
 // (/root/reference/src/sdr_pmr446.c:795-796, /root/reference/src/dsd_in.c:167-168; algorithm:
 // SURVEY.md Appendix A.1-A.5).
@@ -29,7 +29,7 @@
 
 namespace pmr {
 
-enum { SRC_CU8 = 0, SRC_CF32 = 1, SRC_RING = 2 };
+enum { SRC_CU8 = 0, SRC_CF32 = 1, SRC_RING = 2, SRC_CS16 = 3, SRC_CS8 = 4 };
 enum { DC_NONE = 0, DC_SCAN = 1, DC_ZSR = 2 };
 
 // Zero-input-response correction applied while loading a ring written by a DC_ZSR launch.
@@ -46,7 +46,7 @@ struct Correction {
 };
 
 // Per-launch view of the input signal of all streams.
-//  two-source (SRC_CU8 / SRC_CF32): samples [hist_base, n0) live in `hist`, [n0, n1) in `cur`.
+//  two-source (SRC_CU8 / SRC_CF32 / SRC_CS16 / SRC_CS8): samples [hist_base, n0) live in `hist`, [n0, n1) in `cur`.
 //  ring (SRC_RING): sample n lives at cur[n & ring_mask]; samples with n < 0 read as zero.
 struct SrcView {
   const void* hist;
@@ -96,6 +96,10 @@ template <int G>
 struct Raw<SRC_CF32, G> { unsigned w[2 * G]; };  // 8 bytes per sample
 template <int G>
 struct Raw<SRC_RING, G> { unsigned w[2 * G]; };
+template <int G>
+struct Raw<SRC_CS16, G> { unsigned w[G]; };      // 4 bytes per sample
+template <int G>
+struct Raw<SRC_CS8, G> { unsigned w[G / 2]; };   // 2 bytes per sample
 
 // 256-bit global accesses (LDG/STG.E.ENL2.256 on sm_100): a lane's 32-byte piece is one DRAM sector and,
 // with every lane on a different cache line, costs one L1 wavefront instead of two 128-bit ones.
@@ -123,6 +127,18 @@ __device__ __forceinline__ float u8f(unsigned w, int k) {
   return __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7540u + (unsigned)k)) - 8388608.0f;
 }
 
+// Iterations [lo, hi) of a thread whose groups of G samples start at qb that lie wholly inside the current chunk
+// [n0, n1) and can therefore be read with aligned vector loads (none unless the chunk is aligned, see SrcView).
+template <int G>
+__device__ __forceinline__ void fast_iters(const SrcView& v, long long qb, int* lo_out, int* hi_out) {
+  *lo_out = *hi_out = 0;
+  if (v.cur_aligned) {
+    const long long lo = (v.n0 - qb + G - 1) / G, hi = (v.n1 - qb) / G;
+    *lo_out = (int)(lo < 0 ? 0 : (lo > (1 << 30) ? (1 << 30) : lo));
+    *hi_out = (int)(hi < 0 ? 0 : (hi > (1 << 30) ? (1 << 30) : hi));
+  }
+}
+
 // ---- cu8 two-source --------------------------------------------------------------------
 template <>
 struct Loader<SRC_CU8> {
@@ -134,12 +150,7 @@ struct Loader<SRC_CU8> {
   __device__ __forceinline__ void init(const SrcView& v, int s, long long qb) {
     hist = (const uint8_t*)v.hist + (long long)s * v.hist_stride;
     cur = (const uint8_t*)v.cur + (long long)s * v.cur_stride;
-    fast_lo = fast_hi = 0;
-    if (v.cur_aligned) {
-      const long long lo = (v.n0 - qb + G - 1) / G, hi = (v.n1 - qb) / G;
-      fast_lo = (int)(lo < 0 ? 0 : (lo > (1 << 30) ? (1 << 30) : lo));
-      fast_hi = (int)(hi < 0 ? 0 : (hi > (1 << 30) ? (1 << 30) : hi));
-    }
+    fast_iters<G>(v, qb, &fast_lo, &fast_hi);
     fp = cur + 2 * (qb - v.n0);
   }
   template <int G>
@@ -190,12 +201,7 @@ struct Loader<SRC_CF32> {
   __device__ __forceinline__ void init(const SrcView& v, int s, long long qb) {
     hist = (const float2*)((const char*)v.hist + (long long)s * v.hist_stride);
     cur = (const float2*)((const char*)v.cur + (long long)s * v.cur_stride);
-    fast_lo = fast_hi = 0;
-    if (v.cur_aligned) {
-      const long long lo = (v.n0 - qb + G - 1) / G, hi = (v.n1 - qb) / G;
-      fast_lo = (int)(lo < 0 ? 0 : (lo > (1 << 30) ? (1 << 30) : lo));
-      fast_hi = (int)(hi < 0 ? 0 : (hi > (1 << 30) ? (1 << 30) : hi));
-    }
+    fast_iters<G>(v, qb, &fast_lo, &fast_hi);
     fp = cur + (qb - v.n0);
   }
   template <int G>
@@ -221,6 +227,111 @@ struct Loader<SRC_CF32> {
         }
         xr[i] = w.x;
         xi[i] = w.y;
+      }
+    }
+  }
+};
+
+// ---- cs16 / cs8 two-source ---------------------------------------------------------------
+// x 2^-15 (cs16) and x 2^-7 (cs8) exactly, without the I2F unit: x with its sign bit flipped is the unsigned x + 2^15
+// (x + 2^7); dropped into the mantissa of 2^23 it reads as 2^23 + 2^15 + x, and one FFMA by the power of two with the
+// scaled bias as addend leaves x 2^-15 (the product is exact, and so is the sum: it is representable).
+// s16f: half h (0 = I, the low half; 1 = Q) of a cs16 word.  s8f: byte k of a cs8 word already XORed with 0x80808080.
+__device__ __forceinline__ float s16f(unsigned w, int h) {
+  return fmaf(__uint_as_float((h ? (w >> 16) : (w & 0xFFFFu)) ^ 0x4B008000u), 0x1p-15f, -257.0f);
+}
+__device__ __forceinline__ float s8f(unsigned wb, int k) {
+  return fmaf(__uint_as_float(__byte_perm(wb, 0x4B000000u, 0x7540u + (unsigned)k)), 0x1p-7f, -65537.0f);
+}
+
+template <>
+struct Loader<SRC_CS16> {
+  const unsigned* hist;   // one 32-bit word per sample: I in the low half, Q in the high half
+  const unsigned* cur;
+  const unsigned* fp;
+  int fast_lo, fast_hi;
+  template <int G>
+  __device__ __forceinline__ void init(const SrcView& v, int s, long long qb) {
+    hist = (const unsigned*)((const char*)v.hist + (long long)s * v.hist_stride);
+    cur = (const unsigned*)((const char*)v.cur + (long long)s * v.cur_stride);
+    fast_iters<G>(v, qb, &fast_lo, &fast_hi);
+    fp = cur + (qb - v.n0);
+  }
+  template <int G>
+  __device__ __forceinline__ void fetch(int it, Raw<SRC_CS16, G>& r) const {
+    static_assert(G % 8 == 0, "cs16 groups are loaded 32 bytes at a time");
+    if (it >= fast_lo && it < fast_hi) {
+#pragma unroll
+      for (int i = 0; i < G / 8; i++) ldg256_stream(fp + (size_t)it * G + 8 * i, r.w + 8 * i);
+    }
+  }
+  template <int G>
+  __device__ __forceinline__ void convert(const SrcView& v, long long q, int it, const Raw<SRC_CS16, G>& r, float* xr, float* xi) const {
+    if (it >= fast_lo && it < fast_hi) {
+#pragma unroll
+      for (int i = 0; i < G; i++) { xr[i] = s16f(r.w[i], 0); xi[i] = s16f(r.w[i], 1); }
+    } else {
+#pragma unroll
+      for (int i = 0; i < G; i++) {
+        const long long n = q + i;
+        float re = 0.0f, im = 0.0f;
+        if (n >= 0 && n < v.n1 && (n >= v.n0 || n >= v.hist_base)) {
+          const unsigned w = (n >= v.n0) ? cur[n - v.n0] : hist[n - v.hist_base];
+          re = s16f(w, 0);
+          im = s16f(w, 1);
+        }
+        xr[i] = re;
+        xi[i] = im;
+      }
+    }
+  }
+};
+
+template <>
+struct Loader<SRC_CS8> {
+  const uint8_t* hist;
+  const uint8_t* cur;
+  const uint8_t* fp;
+  int fast_lo, fast_hi;
+  template <int G>
+  __device__ __forceinline__ void init(const SrcView& v, int s, long long qb) {
+    hist = (const uint8_t*)v.hist + (long long)s * v.hist_stride;
+    cur = (const uint8_t*)v.cur + (long long)s * v.cur_stride;
+    fast_iters<G>(v, qb, &fast_lo, &fast_hi);
+    fp = cur + 2 * (qb - v.n0);
+  }
+  template <int G>
+  __device__ __forceinline__ void fetch(int it, Raw<SRC_CS8, G>& r) const {
+    static_assert(G % 16 == 0, "cs8 groups are loaded 32 bytes at a time");
+    if (it >= fast_lo && it < fast_hi) {
+#pragma unroll
+      for (int i = 0; i < G / 16; i++) ldg256_stream(fp + (size_t)it * (2 * G) + 32 * i, r.w + 8 * i);
+    }
+  }
+  template <int G>
+  __device__ __forceinline__ void convert(const SrcView& v, long long q, int it, const Raw<SRC_CS8, G>& r, float* xr, float* xi) const {
+    if (it >= fast_lo && it < fast_hi) {
+#pragma unroll
+      for (int j = 0; j < G / 2; j++) {   // one 32-bit word = two samples
+        const unsigned wb = r.w[j] ^ 0x80808080u;
+        xr[2 * j] = s8f(wb, 0);
+        xi[2 * j] = s8f(wb, 1);
+        xr[2 * j + 1] = s8f(wb, 2);
+        xi[2 * j + 1] = s8f(wb, 3);
+      }
+    } else {
+#pragma unroll
+      for (int i = 0; i < G; i++) {
+        const long long n = q + i;
+        float re = 0.0f, im = 0.0f;
+        if (n >= 0 && n < v.n1 && (n >= v.n0 || n >= v.hist_base)) {
+          const uint8_t* b = (n >= v.n0) ? cur + 2 * (n - v.n0) : hist + 2 * (n - v.hist_base);
+          const unsigned wb = ((unsigned)b[0] | ((unsigned)b[1] << 8)) ^ 0x8080u;
+          re = s8f(wb, 0);
+          im = s8f(wb, 1);
+        }
+        xr[i] = re;
+        xi[i] = im;
       }
     }
   }

@@ -60,6 +60,8 @@ inline cascade_fn pick_cascade(int src, int dc, bool arb, const int* ms, int* G)
   if (!arb) {
     if (dc == DC_ZSR && src == SRC_CU8) { PMR_GROUPS(SRC_CU8, DC_ZSR) }
     if (dc == DC_ZSR && src == SRC_CF32) { PMR_GROUPS(SRC_CF32, DC_ZSR) }
+    if (dc == DC_ZSR && src == SRC_CS16) { PMR_GROUPS(SRC_CS16, DC_ZSR) }
+    if (dc == DC_ZSR && src == SRC_CS8) { PMR_GROUPS(SRC_CS8, DC_ZSR) }
     if (dc == DC_NONE && src == SRC_CF32) { PMR_GROUPS(SRC_CF32, DC_NONE) }   // stand-alone msresamp_crcf (liquid shim): no DC blocker
     if (dc == DC_NONE && src == SRC_RING) { PMR_GROUPS(SRC_RING, DC_NONE) }
   } else {
@@ -67,6 +69,8 @@ inline cascade_fn pick_cascade(int src, int dc, bool arb, const int* ms, int* G)
     if (dc == DC_NONE && src == SRC_RING && is(0, 0, 0, 0)) { *G = 8; return cfn<SRC_RING, DC_NONE, 8, 0, 0, 0, 0, true>(); }
     if (dc == DC_SCAN && src == SRC_CU8 && is(0, 0, 0, 0)) return cfn<SRC_CU8, DC_SCAN, 16, 0, 0, 0, 0, true>();
     if (dc == DC_SCAN && src == SRC_CF32 && is(0, 0, 0, 0)) return cfn<SRC_CF32, DC_SCAN, 16, 0, 0, 0, 0, true>();
+    if (dc == DC_SCAN && src == SRC_CS16 && is(0, 0, 0, 0)) return cfn<SRC_CS16, DC_SCAN, 16, 0, 0, 0, 0, true>();
+    if (dc == DC_SCAN && src == SRC_CS8 && is(0, 0, 0, 0)) return cfn<SRC_CS8, DC_SCAN, 16, 0, 0, 0, 0, true>();
     if (dc == DC_NONE && src == SRC_CF32 && is(0, 0, 0, 0)) return cfn<SRC_CF32, DC_NONE, 16, 0, 0, 0, 0, true>();
   }
 #undef PMR_GROUPS
@@ -109,6 +113,7 @@ struct Frontend {
     // (The two launches measured 1.35 + 1.14 ms at 1024 x 1.024 Msps against 0.57 + 2.34 ms for ONE launch of [5, 10] +
     // resampler behind a DC pre-pass over the raw input.)
     const bool split_arb = (order.size() == 2 && order[0] == 5 && order[1] == 10 && plan.step != (3u << 23)) || order.size() == 1;
+    // cs16 and cs8 take the cf32 plans below: the fused and front6 kernels read cu8 only.
     // 2.4 Msps cu8 -> 200 kHz ([3, 5, 10] + rate 2/3): everything in ONE launch, no intermediate ring (frontend_fused.cuh)
     *fused = in_fmt == PMR446_FMT_CU8 && order.size() == 3 && order[0] == 3 && order[1] == 5 && order[2] == 10 && plan.step == (3u << 23);
     // deep cu8 plans (dsd_in: 3,3,3,3,3,5,10 at 2.4 Msps, 3,3,3,3,5,10 at 1.024 Msps): the first six stages in one launch
@@ -208,7 +213,7 @@ struct Frontend {
     c_pole = 1.0f - alpha;
     alpha_eff = 1.0f - c_pole;
     max_chunk = max_chunk_;
-    bps = (in_fmt == PMR446_FMT_CU8) ? 2 : 8;
+    bps = fmt_bytes_per_sample(in_fmt);
     if (rate > 1.0f) return fail(PMR446_EINVAL, "front end only decimates (rate <= 1)");
     plan = design::msresamp_plan(rate, as);
     if (plan.sub_len != 14) return fail(PMR446_EINVAL, "arbitrary resampler kernel is specialised for 14 taps");
@@ -224,7 +229,7 @@ struct Frontend {
     int stage_cursor = (int)plan.stages - 1;  // index into plan.m / plan.hb of the next stage to place
     for (size_t l = 0; l < groups.size(); l++) {
       Level& L = levels[l];
-      L.src = (l == 0) ? (in_fmt == PMR446_FMT_CU8 ? SRC_CU8 : SRC_CF32) : SRC_RING;
+      L.src = (l == 0) ? fmt_source(in_fmt) : SRC_RING;
       L.fused = want_fused;
       L.front6 = want_front6 && l == 0;
       L.dc = (l == 0 && dc) ? ((groups.size() >= 2 || L.fused) ? DC_ZSR : DC_SCAN) : DC_NONE;
@@ -450,6 +455,8 @@ struct Frontend {
         dp.c = c_pole;
         dp.sums = (float2*)sums.p;
         if (L.src == SRC_CU8) dc_local_kernel<SRC_CU8><<<blocks, 128, 0, st>>>(dp);
+        else if (L.src == SRC_CS16) dc_local_kernel<SRC_CS16><<<blocks, 128, 0, st>>>(dp);
+        else if (L.src == SRC_CS8) dc_local_kernel<SRC_CS8><<<blocks, 128, 0, st>>>(dp);
         else dc_local_kernel<SRC_CF32><<<blocks, 128, 0, st>>>(dp);
         launch_dc_scan(sp, st);
         *launches += 2;
@@ -619,6 +626,7 @@ struct Frontend {
       dim3 grid((count + 127) / 128, S);
       if (count > 0) {
         if (bps == 2) hist_update_kernel<uint16_t><<<grid, 128, 0, st>>>(v0, (uint16_t*)dst.p, hist_cap, new_base, count);
+        else if (bps == 4) hist_update_kernel<uint32_t><<<grid, 128, 0, st>>>(v0, (uint32_t*)dst.p, hist_cap, new_base, count);
         else hist_update_kernel<float2><<<grid, 128, 0, st>>>(v0, (float2*)dst.p, hist_cap, new_base, count);
         *launches += 1;
         tm->mark(st, TM_HIST);

@@ -563,7 +563,7 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
   cudaSetDevice(b->device);
   cudaStream_t st = b->own_stream, cs = b->copy_stream;
   const int S = b->S, M = b->M;
-  const size_t bps = b->cfg.in_fmt == PMR446_FMT_CU8 ? 2 : 8;
+  const size_t bps = (size_t)fmt_bytes_per_sample(b->cfg.in_fmt);
   const unsigned W = b->cfg.waterfall;
   if (iq_stride < (long long)(n * bps)) {   // a single stream may pass stride 0
     if (S > 1) return fail(PMR446_EINVAL, "iq_stride smaller than one stream's chunk");
@@ -780,7 +780,7 @@ extern "C" int pmr446_describe_frontend(float rate, float as, int in_fmt, int wi
   std::string out;
   for (size_t l = 0; l < groups.size(); l++) {
     const bool arb = l + 1 == groups.size();
-    const int src = l == 0 ? (in_fmt == PMR446_FMT_CU8 ? SRC_CU8 : SRC_CF32) : SRC_RING;
+    const int src = l == 0 ? fmt_source(in_fmt) : SRC_RING;
     const int dc = (l == 0 && with_dc) ? ((groups.size() >= 2 || fused) ? DC_ZSR : DC_SCAN) : DC_NONE;
     int ms[4] = {0, 0, 0, 0}, G = 0;
     for (size_t k = 0; k < groups[l].size() && k < 4; k++) ms[k] = groups[l][k];
@@ -811,6 +811,8 @@ extern "C" int pmr446_design_asgram_window(unsigned W, float* w) {
 }
 
 extern "C" unsigned pmr446_design_nco_dtheta(float dtheta) { return design::nco_dtheta(dtheta); }
+
+extern "C" int pmr446_bytes_per_sample(int in_fmt) { return fmt_bytes_per_sample(in_fmt); }
 
 // Outputs of the decimating msresamp after n_in input samples in total (closed form, SURVEY.md A.2/A.5).
 extern "C" long long pmr446_count_resampled(float rate, float as, long long n_in) {

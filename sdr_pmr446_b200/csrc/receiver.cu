@@ -253,7 +253,7 @@ extern "C" int pmr446_receiver_execute(pmr446_receiver* r, const void* iq, long 
   cudaSetDevice(r->device);
   cudaStream_t st = r->own_stream;
   const int S = r->S, M = r->M;
-  const size_t bps = r->cfg.chain.in_fmt == PMR446_FMT_CU8 ? 2 : 8;
+  const size_t bps = (size_t)fmt_bytes_per_sample(r->cfg.chain.in_fmt);
   const unsigned W = r->cfg.chain.waterfall;
   if (iq_stride < (long long)(n * bps)) {
     if (S > 1) return fail(PMR446_EINVAL, "iq_stride smaller than one stream's chunk");

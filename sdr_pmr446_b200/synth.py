@@ -4,7 +4,7 @@ The reference has no recorded captures or fixtures (SURVEY.md §4), so tests and
 use seeded synthetic captures: narrow-band FM carriers on the 12.5 kHz PMR446 grid
 (/root/reference/src/sdr_pmr446.c:22-28) with an audio tone plus a CTCSS sub-tone
 (tone table :138-141), complex AWGN and a DC offset, quantised to RTL-SDR style cu8 with the
-inverse of the SoapyRTLSDR conversion (u8 - 127.4)/128.
+inverse of the SoapyRTLSDR conversion (u8 - 127.4)/128, or to signed cs16 / cs8 (x 32768 / x 128).
 
 All phases are closed-form in the absolute sample index, so a capture generated in pieces
 (`start=`) is identical to one generated in one go (noise aside, which is drawn per call).
@@ -93,8 +93,34 @@ def make_cu8(spec: CaptureSpec, n: int, seed: int = 446, start: int = 0) -> np.n
     return to_cu8(make_cf64(spec, n, seed, start))
 
 
+def _to_signed(x: np.ndarray, bits: int, dtype) -> np.ndarray:
+    full = float(1 << (bits - 1))
+    out = np.empty(2 * x.shape[0], dtype=dtype)
+    out[0::2] = np.clip(np.rint(full * x.real), -full, full - 1).astype(dtype)
+    out[1::2] = np.clip(np.rint(full * x.imag), -full, full - 1).astype(dtype)
+    return out
+
+
+def to_cs16(x: np.ndarray) -> np.ndarray:
+    """Interleaved I,Q int16 (Airspy, SDRplay, LimeSDR, USRP, PlutoSDR): clip(round(32768 x), -32768, 32767)."""
+    return _to_signed(x, 16, np.int16)
+
+
+def to_cs8(x: np.ndarray) -> np.ndarray:
+    """Interleaved I,Q int8 (HackRF): clip(round(128 x), -128, 127)."""
+    return _to_signed(x, 8, np.int8)
+
+
 def make_cf32(spec: CaptureSpec, n: int, seed: int = 446, start: int = 0) -> np.ndarray:
     return make_cf64(spec, n, seed, start).astype(np.complex64)
+
+
+def make_cs16(spec: CaptureSpec, n: int, seed: int = 446, start: int = 0) -> np.ndarray:
+    return to_cs16(make_cf64(spec, n, seed, start))
+
+
+def make_cs8(spec: CaptureSpec, n: int, seed: int = 446, start: int = 0) -> np.ndarray:
+    return to_cs8(make_cf64(spec, n, seed, start))
 
 
 def cfg1_capture(n: int = 10_240_000, fs: float = 1024000.0, seed: int = 446, stream_id: int = 0) -> np.ndarray:

@@ -15,12 +15,100 @@ liquid-dsp:
               floor(W / 2) samples of the call, 4 W-point zero-padded DFT, power averaged over the call's
               transforms, FFT-shifted, 10 log10(max(p, 1e-12)); row characters from the maximum of 4 bins against
               the levels -40 + 2 j dB (asgramcf_set_scale(-40, 2)).
+  convert     raw IQ -> the float32 value the chain works on: cu8 (u8 - 127.4f) * (1 / 128) in float32 (the subtraction
+              is exact), cs16 x 2^-15, cs8 x 2^-7, cf32 as is.
+  dc_block    iirfilt_crcf_create_dc_blocker(alpha): y[n] = v[n] - v[n-1], v[n] = x[n] + c v[n-1] from zero state, with
+              the effective feedback c = fl32(1 - alpha) (liquid stores a1 = -1 + alpha in float32; DESIGN 4).
+  msresamp    msresamp_crcf / msresamp_rrrf with the plan of pmr446_design_msresamp (stages, m, step, npfb, hb[16][20]
+              newest-first, pfb[npfb][14] newest-first), all state zero at stream start.
+              decimation: half-band stages from the highest index down, each output o = sum_j hb[g][j] x[2 (o - j)] +
+              x[2 (o - m) + 1] (resamp2_decim: even samples into the filter branch, odd ones into the delay branch),
+              then the scale 2^-stages, then the arbitrary resampler.
+              arbitrary resampler: output j = sum_k pfb[row_j][k] u[pos_j - k], pos_j = (j step) >> 24, row_j = ((j step)
+              mod 2^24) >> (24 - log2 npfb), in exact integers; after n inputs there are ceil(n 2^24 / step) outputs.
+              interpolation (rate > 1): the arbitrary resampler first, then the half-band stages from index 0 up, each
+              input n giving y[2 n] = x[n - m] (delay branch) and y[2 n + 1] = sum_j hb[g][j] x[n - j] (filter branch;
+              resamp2_interp, msresamp2_interp), no scale.
 """
 import numpy as np
 from scipy import signal
 
 LEVEL_CHARS = b" .,-+*&NM#"
 ASGRAM_REF, ASGRAM_DIV = -40.0, 2.0
+FMT_CF32, FMT_CU8, FMT_CS16, FMT_CS8 = 0, 1, 2, 3
+
+
+def convert(iq, fmt):
+    """Raw capture (interleaved I, Q for the integer formats, complex64 for cf32) -> complex128 of the float32 values."""
+    if fmt == FMT_CF32:
+        return np.asarray(iq, np.complex64).astype(np.complex128)
+    iq = np.asarray(iq)
+    if fmt == FMT_CU8:
+        v = (iq.astype(np.float32) - np.float32(127.4)) * np.float32(1.0 / 128.0)
+    elif fmt == FMT_CS16:
+        v = iq.astype(np.float64) * 2.0 ** -15
+    elif fmt == FMT_CS8:
+        v = iq.astype(np.float64) * 2.0 ** -7
+    else:
+        raise ValueError("unknown input format %r" % (fmt,))
+    v = v.astype(np.float64)
+    return v[0::2] + 1j * v[1::2]
+
+
+def dc_block(x, alpha):
+    c = float(np.float32(1.0) - np.float32(alpha))
+    return signal.lfilter([1.0, -1.0], [1.0, -c], np.asarray(x, np.complex128))
+
+
+def _arb(x, plan):
+    """The arbitrary resampler over x from stream start (zero history)."""
+    step, pfb = int(plan["step"]), np.asarray(plan["pfb"], np.float64)
+    bits = int(plan["npfb"]).bit_length() - 1
+    taps = pfb.shape[1]
+    n = x.shape[0]
+    J = (n * (1 << 24) + step - 1) // step
+    ph = np.arange(J, dtype=np.uint64) * np.uint64(step)
+    pos = (ph >> np.uint64(24)).astype(np.int64)
+    row = ((ph & np.uint64((1 << 24) - 1)) >> np.uint64(24 - bits)).astype(np.int64)
+    xp = np.concatenate([np.zeros(taps - 1, x.dtype), x])
+    out = np.zeros(J, x.dtype)
+    for k in range(taps):
+        out += pfb[row, k] * xp[pos - k + taps - 1]
+    return out
+
+
+def msresamp_decim(x, plan):
+    """msresamp_crcf (rate <= 1) over x from stream start."""
+    x = np.asarray(x, np.complex128)
+    stages = int(plan["stages"])
+    for g in range(stages - 1, -1, -1):
+        m = int(plan["m"][g])
+        h = np.asarray(plan["hb"][g][:2 * m], np.float64)
+        n = x.shape[0] // 2
+        ev, od = x[0:2 * n:2], x[1:2 * n:2]
+        y = signal.lfilter(h, [1.0], ev)
+        y[m:] += od[:max(n - m, 0)]
+        x = y
+    return _arb(x * 2.0 ** -stages, plan)
+
+
+def msresamp_interp_real(x, plan):
+    """msresamp_rrrf (rate > 1) over x from stream start."""
+    y = _arb(np.asarray(x, np.float64), plan)
+    for g in range(int(plan["stages"])):
+        m = int(plan["m"][g])
+        h = np.asarray(plan["hb"][g][:2 * m], np.float64)
+        out = np.zeros(2 * y.shape[0])
+        out[2 * m::2] = y[:max(y.shape[0] - m, 0)]
+        out[1::2] = signal.lfilter(h, [1.0], y)
+        y = out
+    return y
+
+
+def front_end(iq, fmt, plan, alpha, with_dc=True):
+    """Raw capture -> the front end's output `res` (conversion, DC blocker, msresamp_crcf)."""
+    x = convert(iq, fmt)
+    return msresamp_decim(dc_block(x, alpha) if with_dc else x, plan)
 
 
 def nco_phase(n, dtheta, j0=0):
@@ -143,6 +231,21 @@ def check_demod(demod, chan_used, chan_ref, kf, tol_rad):
     dd = np.abs(wrapped((demod.astype(np.float64) - ref_d) * k))
     assert np.all(dd[good] <= 2 * cone[good] + tol_rad), float(np.max(dd[good] - 2 * cone[good]))
     return float(np.max(d[ok]))
+
+
+def check_res(out, ref, tol_rms, tol_max):
+    """A resampler output (complex or real) against its float64 reference: error RMS <= tol_rms of the reference RMS over
+    the whole output, and EVERY sample's |error| <= tol_max of that RMS (an RMS over N samples lets k sparse errors of
+    tol_rms sqrt(N / k) through: segment starts, tile and chunk edges are where such errors come from).  Returns both
+    measured ratios (error RMS, worst sample) over the reference RMS."""
+    out, ref = np.asarray(out), np.asarray(ref)
+    assert out.shape == ref.shape, (out.shape, ref.shape)
+    stage = np.sqrt(np.mean(np.abs(ref) ** 2))
+    e = np.abs(out.astype(np.complex128 if np.iscomplexobj(out) else np.float64) - ref)
+    rms, worst = float(np.sqrt(np.mean(e ** 2)) / stage), float(np.max(e, initial=0.0) / stage)
+    assert rms <= tol_rms, ("rms", rms)
+    assert worst <= tol_max, ("sample", int(np.argmax(e)), worst)
+    return rms, worst
 
 
 def check_pcm(pcm, audio64, max_abs_err):

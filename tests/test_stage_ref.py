@@ -68,3 +68,101 @@ def test_asgram_matches_oracle(W):
             assert np.all(p["ascii"] == ord(" ")) and np.all(p["peak"] == 0)
             continue
         stage_ref.check_asgram(p["psd"], p["peak"], p["ascii"], psd, peak, 1e-3)
+
+
+# ---- front end and dsd_in back end --------------------------------------------------------------------------------------
+FE_TOL_RMS, FE_TOL_MAX = 2e-5, 6e-5      # ~3x the float32 oracle's own distance from float64 (1.4e-6 .. 6.3e-6 / 1.8e-5)
+ALPHA = 0.0005
+
+
+def _capture(fs, fmt, n, seed, dsd=False):
+    from sdr_pmr446_b200 import synth
+    if dsd:   # dsd_in: one carrier at 0 Hz
+        spec = synth.CaptureSpec(fs=float(fs), carriers=(synth.Carrier(1, 0.3, 1000.0, 0.0),), offset_hz=-synth.channel_offset_hz(1))
+    else:
+        spec = synth.CaptureSpec(fs=float(fs), carriers=synth.rotated_carriers(seed))
+    return synth.make_cu8(spec, n, seed) if fmt == stage_ref.FMT_CU8 else synth.make_cf32(spec, n, seed)
+
+
+def _uneven(n, chunk):
+    """Chunk sizes (at most `chunk`) covering n samples: a long call, 1 and 7 samples, one off a multiple of 16, the rest."""
+    sizes = [chunk - 5, 1, 7, 4095, 333]
+    while sum(sizes) < n:
+        sizes.append(min(chunk, n - sum(sizes)))
+    sizes[-1] -= sum(sizes) - n
+    return [k for k in sizes if k > 0]
+
+
+def _oracle_calls(o, iq, sizes, bps, **kw):
+    parts, p = [], 0
+    for k in sizes:
+        parts.append(o.execute(iq[p * bps:(p + k) * bps], **kw))
+        p += k
+    return parts
+
+
+@pytest.mark.parametrize("fs,fmt,fs_out", [(2400000, 1, 200000), (1024000, 1, 200000), (3200000, 0, 200000), (4800000, 0, 200000),
+                                           (20000000, 0, 200000), (500000, 0, 200000), (250000, 0, 200000), (200000, 0, 200000),
+                                           (2400000, 1, 12500), (1024000, 0, 12500)])
+def test_front_end_matches_oracle(fs, fmt, fs_out):
+    """stage_ref.front_end (conversion, DC blocker, half-band cascade, arbitrary resampler) against the oracle's `res`, fed
+    in uneven chunks; every sample, not only the RMS."""
+    from oracle import oracle as orc
+    from util import design_msresamp
+    n, chunk = fs // 2, fs // 10
+    iq = _capture(fs, fmt, n, 600 + fmt, dsd=fs_out == 12500)
+    bps = 2 if fmt == stage_ref.FMT_CU8 else 1
+    if fs_out == 12500:   # the dsd_in chain is the oracle's only front end into 12.5 kHz
+        o = orc.DsdOracle(fs_in=fs, in_fmt=fmt, chunk=chunk)
+        parts = _oracle_calls(o, iq, _uneven(n, chunk), bps)
+    else:
+        o = orc.PmrOracle(fs_in=fs, in_fmt=fmt, num_channels=fs_out // 12500, chunk=chunk)
+        parts = _oracle_calls(o, iq, _uneven(n, chunk), bps, want=("res",))
+    o.close()
+    res = np.concatenate([p["res"] for p in parts])
+    ref = stage_ref.front_end(iq, fmt, design_msresamp(np.float32(fs_out) / np.float32(fs)), ALPHA)
+    stage_ref.check_res(res, ref, FE_TOL_RMS, FE_TOL_MAX)
+
+
+@pytest.mark.parametrize("fmt", [0, 1])
+def test_dc_block_matches_oracle(fmt):
+    from oracle import oracle as orc
+    n, chunk = 300000, 100000
+    iq = _capture(1024000, fmt, n, 610 + fmt)
+    bps = 2 if fmt == stage_ref.FMT_CU8 else 1
+    o = orc.PmrOracle(fs_in=1024000, in_fmt=fmt, chunk=chunk)
+    parts = _oracle_calls(o, iq, _uneven(n, chunk), bps, want=("dcblocked",))
+    o.close()
+    ref = stage_ref.dc_block(stage_ref.convert(iq, fmt), ALPHA)
+    stage_ref.check_res(np.concatenate([p["dcblocked"] for p in parts]), ref, FE_TOL_RMS, FE_TOL_MAX)
+
+
+def test_convert_integer_formats():
+    """cs16 x 2^-15 and cs8 x 2^-7 at the extremes; cu8 (u8 - 127.4f) / 128 rounded as float32 arithmetic rounds it."""
+    v16 = np.array([-32768, 32767, 0, 1, -1, 12345], np.int16)
+    assert np.array_equal(stage_ref.convert(v16, stage_ref.FMT_CS16), (v16[0::2] + 1j * v16[1::2]) / 32768.0)
+    v8 = np.array([-128, 127, 0, -1], np.int8)
+    assert np.array_equal(stage_ref.convert(v8, stage_ref.FMT_CS8), (v8[0::2] + 1j * v8[1::2]) / 128.0)
+    u8 = np.arange(256, dtype=np.uint8)
+    x = stage_ref.convert(u8, stage_ref.FMT_CU8)
+    want = ((u8.astype(np.float32) - np.float32(127.4)) * np.float32(1 / 128)).astype(np.float64)
+    assert np.array_equal(x.real, want[0::2]) and np.array_equal(x.imag, want[1::2])
+
+
+@pytest.mark.parametrize("fs,fmt", [(2400000, 1), (1024000, 0)])
+def test_msresamp_interp_matches_oracle(fs, fmt):
+    """stage_ref.msresamp_interp_real (msresamp_rrrf x 3.84) against the dsd_in oracle's audio given its own discriminator
+    output, and its s16 cast (dsd_in truncates and does not saturate: only samples inside +-1 are compared)."""
+    from oracle import oracle as orc
+    from util import design_msresamp
+    n, chunk = 600000, 200000
+    iq = _capture(fs, fmt, n, 620 + fmt, dsd=True)
+    o = orc.DsdOracle(fs_in=fs, in_fmt=fmt, chunk=chunk)
+    parts = _oracle_calls(o, iq, _uneven(n, chunk), 2 if fmt == stage_ref.FMT_CU8 else 1)
+    o.close()
+    fm, audio, pcm = (np.concatenate([p[k] for p in parts]) for k in ("fm", "audio", "pcm"))
+    au = stage_ref.msresamp_interp_real(fm, design_msresamp(np.float32(48000) / np.float32(12500)))
+    stage_ref.check_res(audio, au, 1e-6, 1e-5)
+    inside = np.abs(au) < 0.999
+    assert np.mean(inside) > 0.95
+    stage_ref.check_pcm(pcm[inside], au[inside], float(np.max(np.abs(audio - au))))

@@ -45,6 +45,29 @@ def design_dtheta(M):
     return int(lib().pmr446_design_nco_dtheta(nco_offset(M)))
 
 
+def design_msresamp(rate, as_db=60.0):
+    """msresamp_crcf_create(rate, as) / msresamp_rrrf_create as the library plans it: dict of stages, m, step, npfb,
+    hb [16][20] and pfb [npfb][14] (the form tests/stage_ref.py takes)."""
+    import ctypes as C
+
+    from sdr_pmr446_b200._lib import check, lib
+    st, m, step, npfb = C.c_uint(), (C.c_uint * 16)(), C.c_uint(), C.c_uint()
+    hb, pfb = np.zeros((16, 20), np.float32), np.zeros((256, 14), np.float32)
+    check(lib().pmr446_design_msresamp(np.float32(rate), as_db, C.byref(st), m, C.byref(step), C.byref(npfb), hb.ctypes.data,
+                                       pfb.ctypes.data), "pmr446_design_msresamp")
+    return dict(stages=st.value, m=list(m)[:st.value], step=step.value, npfb=npfb.value, hb=hb, pfb=pfb[:npfb.value])
+
+
+def describe_frontend(rate, fmt, with_dc=1, as_db=60.0):
+    """pmr446_describe_frontend: the plan string of the front end ("fused[3,5,10]+arb", "cascade[3,5] | tile[10]+arb", ...)."""
+    import ctypes as C
+
+    from sdr_pmr446_b200._lib import check, lib
+    buf = C.create_string_buffer(256)
+    check(lib().pmr446_describe_frontend(np.float32(rate), as_db, fmt, with_dc, buf, 256), "pmr446_describe_frontend")
+    return buf.value.decode()
+
+
 def design_asgram_window(W):
     from sdr_pmr446_b200._lib import check, lib
     w = np.zeros(W, np.float32)

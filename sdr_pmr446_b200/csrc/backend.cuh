@@ -11,7 +11,9 @@
 #include <math.h>
 #include <stdint.h>
 
+#include "../../include/pmr446_taps.h"
 #include "audio_fft.cuh"   // pcm_sat
+#include "common_host.hpp"
 
 namespace pmr {
 
@@ -243,5 +245,73 @@ static __global__ void __launch_bounds__(AU_THREADS) audio_kernel(AudioParams p)
     if (prow) prow[i - f0r] = pcm_sat(v);
   }
 }
+
+// Host side of the direct-form audio chain: the high-pass and low-pass taps a configuration selects, the tile lead-in
+// and de-emphasis warm-up they and the pole need, and the launch.  In an unnamed namespace because audio_kernel is
+// static: each translation unit sets up and launches its own instantiations.
+namespace {
+struct DirectAudio {
+  std::vector<float> hp, lp;   // the caller's taps, or the reference's
+  DevBuf d_hp, d_lp;           // the same, zero-padded to whole 16-tap chunks
+  int hp_chunks = 0, lp_chunks = 0, hp_delay = 0;
+  int de_warm = 0;             // de-emphasis warm-up (deemph_warmup); > 8 selects audio_kernel<true>
+  int lead = AU_LEAD_MIN;      // lead-in of a tile (audio_lead)
+  pmr446_config cfg{};         // gain, de-emphasis, low-pass switch
+
+  static int upload_padded(const std::vector<float>& h, DevBuf& d, int* chunks) {
+    std::vector<float> t((h.size() + 15) / 16 * 16, 0.0f);
+    std::copy(h.begin(), h.end(), t.begin());
+    *chunks = (int)(t.size() / 16);
+    if (int rc = d.alloc(t.size() * sizeof(float))) return rc;
+    CUDA_TRY(cudaMemcpy(d.p, t.data(), t.size() * sizeof(float), cudaMemcpyHostToDevice));
+    return 0;
+  }
+
+  int init(const pmr446_config& c) {
+    const unsigned hpn = c.hp_taps ? c.hp_len : PMR446_HP_AUDIO_TAPS_LEN, lpn = c.lp_taps ? c.lp_len : PMR446_LP_AUDIO_TAPS_LEN;
+    if (hpn < 1 || hpn > (unsigned)AU_MAXHALO || (hpn & 1) == 0) return fail(PMR446_EINVAL, "hp_len must be odd and <= 383");
+    if (lpn < 1 || lpn > (unsigned)AU_LEAD_LP - 16) return fail(PMR446_EINVAL, "lp_len must be <= 112");
+    hp.resize(hpn);
+    lp.resize(lpn);
+    if (c.hp_taps) std::copy(c.hp_taps, c.hp_taps + hpn, hp.begin());
+    else pmr446_hp_audio_taps_fill(hp.data());
+    if (c.lp_taps) std::copy(c.lp_taps, c.lp_taps + lpn, lp.begin());
+    else pmr446_lp_audio_taps_fill(lp.data());
+    hp_delay = (int)(hpn - 1) / 2;   // wdelayf_create((HP_AUDIO_FILT_TAPS - 1) / 2), :447
+    if (int rc = upload_padded(hp, d_hp, &hp_chunks)) return rc;
+    if (int rc = upload_padded(lp, d_lp, &lp_chunks)) return rc;
+    // the de-emphasis pole's warm-up sets the tile lead-in; deemph_fir replaces the pole (fast-convolution path only)
+    de_warm = c.deemph_fir ? 0 : deemph_warmup(c.deemph_a1);
+    lead = de_warm < 0 ? -1 : audio_lead(c.lowpass != 0, lp_chunks, de_warm);
+    if (lead < 0) return fail(PMR446_EINVAL, "deemph_a1 must satisfy |a1| < 1 with a warm-up that fits the audio tile (|a1| <= 0.977)");
+    cfg = c;
+    cudaFuncSetAttribute(audio_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+    cudaFuncSetAttribute(audio_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+    return 0;
+  }
+
+  // Fills the parameters the chain does not own (taps, gain, de-emphasis, lead-in, warm-up) and launches p.rows x p.tiles
+  // blocks.  The caller sets the ring, rows, tiles, sample ranges and outputs; it reads `lead` to lay out the tiles.
+  void launch(AudioParams& p, cudaStream_t st) const {
+    p.lead = lead;
+    p.hp_taps = (const float*)d_hp.p;
+    p.hp_chunks = hp_chunks;
+    p.hp_delay = hp_delay;
+    p.lp_taps = cfg.lowpass ? (const float*)d_lp.p : nullptr;
+    p.lp_chunks = lp_chunks;
+    p.gain = cfg.audio_gain;
+    p.de_b0 = cfg.deemph_b0;
+    p.de_b1 = cfg.deemph_b1;
+    p.de_a1 = cfg.deemph_a1;
+    p.de_warm = de_warm;
+    // the padded input tile, the second buffer and the taps of audio_kernel
+    const size_t xn = AU_MAXHALO + AU_SPAN + 16, yn = AU_LEAD_LP + AU_SPAN + 16;
+    const size_t smem = ((xn + xn / 16 + 1) + (yn + yn / 16 + 1) + 384 + 128 + 8) * sizeof(float);
+    const unsigned grid = (unsigned)((long long)p.rows * p.tiles);
+    if (de_warm > 8) audio_kernel<true><<<grid, AU_THREADS, smem, st>>>(p);
+    else audio_kernel<false><<<grid, AU_THREADS, smem, st>>>(p);
+  }
+};
+}  // namespace
 
 }  // namespace pmr

@@ -106,6 +106,40 @@ struct DevBuf {
   int ensure(size_t n) { return (p && bytes >= n) ? 0 : alloc(n); }
 };
 
+// Row stride of a host-buffer call's input, or PMR446_EINVAL: a single stream may pass a stride smaller than its chunk
+// (0, say), several streams may not.
+inline long long host_iq_stride(long long iq_stride, unsigned n, size_t bytes_per_sample, int streams) {
+  const long long row = (long long)(n * bytes_per_sample);
+  if (iq_stride >= row) return iq_stride;
+  if (streams > 1) return fail(PMR446_EINVAL, "iq_stride smaller than one stream's chunk");
+  return row;
+}
+
+// stage(host, buf, bytes): the device buffer, grown to `bytes`, that stages a host-buffer call's output the caller
+// requested (host != nullptr); nullptr for one not requested.  A failed allocation must fail the call, not silently
+// drop the output: the first one is kept in rc.
+struct Staging {
+  int rc = 0;
+  template <typename T>
+  T* operator()(T* host, DevBuf& buf, size_t bytes) {
+    if (!host || rc) return nullptr;
+    rc = buf.ensure(bytes);
+    return rc ? nullptr : (T*)buf.p;
+  }
+};
+
+// Device -> host copy of columns [col0, col0 + cols) of `rows` rows of elt-byte elements; nothing if the output was not
+// requested (host == nullptr) or the range is empty.
+inline void copy_back(cudaStream_t st, void* host, const void* dev, long long host_ld, long long dev_ld, size_t elt, long long rows,
+                      long long col0, long long cols) {
+  if (host && cols > 0)
+    cudaMemcpy2DAsync((char*)host + col0 * elt, host_ld * elt, (const char*)dev + col0 * elt, dev_ld * elt, cols * elt, rows,
+                      cudaMemcpyDeviceToHost, st);
+}
+
+// Frames (channelizer outputs per channel) that the next n input samples complete in a batch chain (closed form).
+long long batch_frames_after(const pmr446_batch* b, unsigned n);
+
 // out[row][k] = ring[row][(start + k) & mask], k < count
 template <typename T>
 __global__ void gather_ring_kernel(const T* ring, long long ring_stride, long long mask, long long start, long long count, T* out, long long out_ld) {

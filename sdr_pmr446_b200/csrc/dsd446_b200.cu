@@ -6,6 +6,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <memory>
 #include <vector>
 
 #include "../../include/pmr446_b200.h"
@@ -60,21 +61,16 @@ extern "C" int dsd446_batch_create(const dsd446_config* cfg, dsd446_batch** out)
   if (cfg->n_streams < 1 || cfg->max_chunk < 1 || cfg->fs_in == 0 || cfg->fs_sig == 0) return fail(PMR446_EINVAL, "bad configuration");
   if (int rc = select_device(cfg->device)) return rc;
   cudaGetLastError();   // clean slate for the check at the end
-  dsd446_batch* b = new dsd446_batch();
+  std::unique_ptr<dsd446_batch, int (*)(dsd446_batch*)> b(new dsd446_batch(), dsd446_batch_destroy);   // freed on every early return
   b->cfg = *cfg;
   b->S = cfg->n_streams;
   cudaGetDevice(&b->device);
   int rc = b->fe.init(b->S, cfg->in_fmt, ((float)cfg->fs_sig) / cfg->fs_in, cfg->resamp_as, true, cfg->dc_alpha, cfg->max_chunk, 64);
-  if (rc) { dsd446_batch_destroy(b); return rc; }
+  if (rc) return rc;
   b->up = design::msresamp_plan(((float)cfg->fs_audio) / cfg->fs_sig, cfg->resamp_as);
-  if (!b->up.interp || b->up.stages != 1 || b->up.sub_len != 14 || b->up.m[0] > 10) {
-    dsd446_batch_destroy(b);
+  if (!b->up.interp || b->up.stages != 1 || b->up.sub_len != 14 || b->up.m[0] > 10)
     return fail(PMR446_EINVAL, "up-sampler plan not built: need one half-band stage after the arbitrary resampler (2 < rate <= 4)");
-  }
-  if (b->up.step < (1u << 23) || b->up.step > (1u << 24)) {
-    dsd446_batch_destroy(b);
-    return fail(PMR446_EINVAL, "up-sampler plan not built: arbitrary stage outside (1, 2]");
-  }
+  if (b->up.step < (1u << 23) || b->up.step > (1u << 24)) return fail(PMR446_EINVAL, "up-sampler plan not built: arbitrary stage outside (1, 2]");
   {  // smallest P <= DSB_T after which the 24-bit phase is back within 1/16 of a bank row: a thread that computes outputs k, k + P,
      // k + 2P, ... keeps its bank row in registers (x1.92: P = 48, drift -16 / 2^24 per period)
     const unsigned tol = (1u << (24 - b->up.bits)) / 16;
@@ -91,18 +87,11 @@ extern "C" int dsd446_batch_create(const dsd446_config* cfg, dsd446_batch** out)
   std::vector<float> rows((size_t)b->up.npfb * 16, 0.0f);
   for (unsigned i = 0; i < b->up.npfb; i++)
     for (unsigned k = 0; k < 14; k++) rows[(size_t)i * 16 + k] = b->up.pfb[(size_t)i * 14 + k];
-  if ((rc = b->d_fm.alloc_zero((size_t)b->S * b->fm_cap * 4)) ||
-      (rc = b->d_pfb_up.alloc(rows.size() * 4))) {
-    dsd446_batch_destroy(b);
-    return rc;
-  }
+  if ((rc = b->d_fm.alloc_zero((size_t)b->S * b->fm_cap * 4)) || (rc = b->d_pfb_up.alloc(rows.size() * 4))) return rc;
   cudaMemcpy(b->d_pfb_up.p, rows.data(), rows.size() * 4, cudaMemcpyHostToDevice);
   CUDA_TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking));
-  if (cudaDeviceSynchronize() != cudaSuccess || cudaGetLastError() != cudaSuccess) {
-    dsd446_batch_destroy(b);
-    return fail(PMR446_ECUDA, "CUDA error while setting up the dsd batch");
-  }
-  *out = b;
+  if (cudaDeviceSynchronize() != cudaSuccess || cudaGetLastError() != cudaSuccess) return fail(PMR446_ECUDA, "CUDA error while setting up the dsd batch");
+  *out = b.release();
   return PMR446_OK;
 }
 
@@ -121,6 +110,16 @@ extern "C" int dsd446_batch_reset(dsd446_batch* b) {
   return PMR446_OK;
 }
 
+// The caller's leading dimensions against the counts of a call of n samples (closed form), before any state advances: a
+// rejected call leaves the handle untouched.
+static int check_ld(const dsd446_batch* b, unsigned n, const dsd446_outputs* out) {
+  const long long r1 = b->fe.outputs_after(b->fe.n_in + (long long)n);
+  const long long nz = 2 * ((long long)design::arb_outputs_after((uint64_t)r1, b->up.step) - b->n_z);
+  if ((out->res || out->fm) && r1 - b->fe.n_out > out->res_ld) return fail(PMR446_ERANGE, "res_ld too small");
+  if ((out->audio || out->pcm) && nz > out->out_ld) return fail(PMR446_ERANGE, "out_ld too small");
+  return PMR446_OK;
+}
+
 extern "C" int dsd446_batch_execute_device(dsd446_batch* b, const void* iq, long long iq_stride, unsigned n, const dsd446_outputs* out,
                                            unsigned* ny_out, unsigned* nz_out, void* cuda_stream) {
   if (!b || !out) return fail(PMR446_EINVAL, "null argument");
@@ -130,13 +129,9 @@ extern "C" int dsd446_batch_execute_device(dsd446_batch* b, const void* iq, long
   const int S = b->S;
   int launches = 0;
   const long long r0 = b->fe.n_out;
-  {  // validate against the closed-form counts BEFORE any state advances: a failed call leaves the handle untouched
-    const long long r1p = b->fe.outputs_after(b->fe.n_in + (long long)n);
-    const long long nzp = 2 * ((long long)design::arb_outputs_after((uint64_t)r1p, b->up.step) - b->n_z);
-    if ((out->res || out->fm) && r1p - r0 > out->res_ld) return fail(PMR446_ERANGE, "res_ld too small");
-    if ((out->audio || out->pcm) && nzp > out->out_ld) return fail(PMR446_ERANGE, "out_ld too small");
-  }
-  int rc = b->fe.execute(iq, iq_stride, n, st, &launches);   // src/dsd_in.c:167-168
+  int rc = check_ld(b, n, out);
+  if (rc) return rc;
+  rc = b->fe.execute(iq, iq_stride, n, st, &launches);   // src/dsd_in.c:167-168
   if (rc) return rc;
   const long long r1 = b->fe.n_out, ny = r1 - r0;
   const long long k0 = b->n_z, k1 = (long long)design::arb_outputs_after((uint64_t)r1, b->up.step);
@@ -189,44 +184,27 @@ extern "C" int dsd446_batch_execute(dsd446_batch* b, const void* iq, long long i
   cudaStream_t st = b->own_stream;
   const int S = b->S;
   const size_t bps = (size_t)fmt_bytes_per_sample(b->cfg.in_fmt);
-  const long long in_row = (long long)((b->cfg.max_chunk * bps + 63) / 64 * 64);
+  if ((iq_stride = host_iq_stride(iq_stride, n, bps, S)) < 0) return (int)iq_stride;
   int rc;
+  if ((rc = check_ld(b, n, out))) return rc;
+  const long long in_row = (long long)((b->cfg.max_chunk * bps + 63) / 64 * 64);
   if ((rc = b->d_in.ensure((size_t)S * in_row))) return rc;
-  if (iq_stride < (long long)(n * bps)) {   // a single stream may pass stride 0
-    if (S > 1) return fail(PMR446_EINVAL, "iq_stride smaller than one stream's chunk");
-    iq_stride = (long long)(n * bps);
-  }
   if (n) CUDA_TRY(cudaMemcpy2DAsync(b->d_in.p, in_row, iq, iq_stride, (size_t)n * bps, S, cudaMemcpyHostToDevice, st));
   dsd446_outputs d = *out;
   d.res_ld = b->max_res;
   d.out_ld = b->max_out;
-  int stage_rc = 0;
-  auto stage = [&](const void* host, DevBuf& buf, size_t bytes) -> void* {
-    if (!host) return nullptr;
-    if (int e = buf.ensure(bytes)) { stage_rc = e; return nullptr; }
-    return buf.p;
-  };
-  d.res = (float*)stage(out->res, b->d_res, (size_t)S * d.res_ld * 8);
-  d.fm = (float*)stage(out->fm, b->d_fmout, (size_t)S * d.res_ld * 4);
-  d.audio = (float*)stage(out->audio, b->d_audio, (size_t)S * d.out_ld * 4);
-  d.pcm = (int16_t*)stage(out->pcm, b->d_pcm, (size_t)S * d.out_ld * 2);
-  if (stage_rc) return stage_rc;
-  {  // the caller's leading dimensions, before the state advances
-    const long long r1p = b->fe.outputs_after(b->fe.n_in + (long long)n);
-    const long long nzp = 2 * ((long long)design::arb_outputs_after((uint64_t)r1p, b->up.step) - b->n_z);
-    if ((out->res || out->fm) && r1p - b->fe.n_out > out->res_ld) return fail(PMR446_ERANGE, "res_ld too small");
-    if ((out->audio || out->pcm) && nzp > out->out_ld) return fail(PMR446_ERANGE, "out_ld too small");
-  }
+  Staging stage;
+  d.res = stage(out->res, b->d_res, (size_t)S * d.res_ld * 8);
+  d.fm = stage(out->fm, b->d_fmout, (size_t)S * d.res_ld * 4);
+  d.audio = stage(out->audio, b->d_audio, (size_t)S * d.out_ld * 4);
+  d.pcm = stage(out->pcm, b->d_pcm, (size_t)S * d.out_ld * 2);
+  if (stage.rc) return stage.rc;
   unsigned ny = 0, nz = 0;
-  rc = dsd446_batch_execute_device(b, b->d_in.p, in_row, n, &d, &ny, &nz, st);
-  if (rc) return rc;
-  auto back = [&](void* host, const void* dev, long long hld, long long dld, size_t elt, long long cols) {
-    if (host && cols > 0) cudaMemcpy2DAsync(host, hld * elt, dev, dld * elt, cols * elt, S, cudaMemcpyDeviceToHost, st);
-  };
-  back(out->res, d.res, out->res_ld, d.res_ld, 8, ny);
-  back(out->fm, d.fm, out->res_ld, d.res_ld, 4, ny);
-  back(out->audio, d.audio, out->out_ld, d.out_ld, 4, nz);
-  back(out->pcm, d.pcm, out->out_ld, d.out_ld, 2, nz);
+  if ((rc = dsd446_batch_execute_device(b, b->d_in.p, in_row, n, &d, &ny, &nz, st))) return rc;
+  copy_back(st, out->res, d.res, out->res_ld, d.res_ld, 8, S, 0, ny);
+  copy_back(st, out->fm, d.fm, out->res_ld, d.res_ld, 4, S, 0, ny);
+  copy_back(st, out->audio, d.audio, out->out_ld, d.out_ld, 4, S, 0, nz);
+  copy_back(st, out->pcm, d.pcm, out->out_ld, d.out_ld, 2, S, 0, nz);
   CUDA_TRY(cudaStreamSynchronize(st));
   if (ny_out) *ny_out = ny;
   if (nz_out) *nz_out = nz;

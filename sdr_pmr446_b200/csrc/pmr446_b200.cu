@@ -10,6 +10,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -48,16 +49,13 @@ struct pmr446_batch {
   DevBuf d_demod;
   long long demod_cap = 0;
   // audio
-  DevBuf d_hp, d_lp;
-  int hp_chunks = 0, lp_chunks = 0, hp_delay = 0;
+  DirectAudio au;            // direct-form chain: lpcomp, and audio / pcm when the response does not fit the FFT tile
   DevBuf d_mag;              // [S][max_tiles][16] per-tile sums of |chan| (RSSI)
   int max_tiles = 0;
   long long last_f0 = 0, last_ns = 0;   // frame range of the last execute call (pmr446_batch_gather_channel)
   DevBuf d_out_rssi, d_out_edge;
   int fft_halo = AF_HALO;    // overlap of the FFT audio tile (AF_HALO or AF_HALO_LONG)
   bool fft_audio = false;    // audio / pcm by fast convolution (audio_fft4_kernel); the direct-form kernel serves lpcomp
-  int au_lead = AU_LEAD_MIN; // lead-in of the direct-form kernel's tiles (audio_lead)
-  int de_warm = 0;           // de-emphasis warm-up (deemph_warmup); > 8 selects audio_kernel<true>
   DevBuf d_resp, d_aftw;
   // waterfall
   Waterfall wf;
@@ -97,16 +95,6 @@ extern "C" void pmr446_default_config(pmr446_config* c) {
   c->deemph_a1 = (float)(PMR446_DEEMPH_A1 / PMR446_DEEMPH_A0);
 }
 
-static int upload_padded_taps(const float* h, unsigned n, DevBuf& d, int* chunks) {
-  unsigned padded = (n + 15) / 16 * 16;
-  std::vector<float> t(padded, 0.0f);
-  for (unsigned i = 0; i < n; i++) t[i] = h[i];
-  *chunks = (int)(padded / 16);
-  if (int rc = d.alloc(padded * sizeof(float))) return rc;
-  CUDA_TRY(cudaMemcpy(d.p, t.data(), padded * sizeof(float), cudaMemcpyHostToDevice));
-  return 0;
-}
-
 extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out) {
   if (!cfg || !out) return fail(PMR446_EINVAL, "null argument");
   *out = nullptr;
@@ -115,7 +103,7 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
     return fail(PMR446_EINVAL, "num_channels must be in [2, 4096] and pfb_m in [1, 32]");
   if (int rc = select_device(cfg->device)) return rc;
   cudaGetLastError();   // start from a clean slate: the check at the end only sees errors raised in here
-  pmr446_batch* b = new pmr446_batch();
+  std::unique_ptr<pmr446_batch, int (*)(pmr446_batch*)> b(new pmr446_batch(), pmr446_batch_destroy);   // freed on every early return
   b->cfg = *cfg;
   b->S = cfg->n_streams;
   cudaGetDevice(&b->device);
@@ -129,13 +117,13 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
   int rc = b->fe.init(S, cfg->in_fmt, fs_res / (float)cfg->fs_in, cfg->resamp_as, true, cfg->dc_alpha, cfg->max_chunk,
                       /*extra_hist=*/std::max<long long>(std::max<long long>((long long)M * (2 * cfg->pfb_m + CG_FT + 4), (long long)cfg->waterfall),
                                                          16LL * (CH_FR + CH_HIST + 2)) + 64);   // a call recomputes at most one channelizer tile
-  if (rc) { pmr446_batch_destroy(b); return rc; }
+  if (rc) return rc;
   b->max_res = b->fe.max_out_per_chunk();
   b->max_ns = b->max_res / M + 1;
 
   // channelizer (A.7, A.8)
   std::vector<float> taps = design::pfbch_taps((unsigned)M, cfg->pfb_m, cfg->pfb_as);
-  if ((rc = b->d_pfb_taps.alloc(taps.size() * sizeof(float)))) { pmr446_batch_destroy(b); return rc; }
+  if ((rc = b->d_pfb_taps.alloc(taps.size() * sizeof(float)))) return rc;
   if (b->generic) {
     // the generic kernel walks the branches across lanes: store tap n of all branches contiguously ([n][M])
     const unsigned pp = 2 * cfg->pfb_m;
@@ -155,19 +143,16 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
       if (nn % pr == 0) { b->radix.push_back((int)pr); nn /= pr; }
       else pr++;
     }
-    if (b->radix.size() > 16) { pmr446_batch_destroy(b); return fail(PMR446_EINVAL, "num_channels has more than 16 prime factors"); }
+    if (b->radix.size() > 16) return fail(PMR446_EINVAL, "num_channels has more than 16 prime factors");
     std::vector<float2> tw(M);
     for (int k = 0; k < M; k++) {
       double a = -2.0 * M_PI * (double)k / (double)M;
       tw[k] = make_float2((float)cos(a), (float)sin(a));
     }
-    if ((rc = b->d_tw.alloc((size_t)M * sizeof(float2))) || (rc = b->d_mixed.alloc_zero((size_t)S * b->fe.out_cap * sizeof(float2)))) {
-      pmr446_batch_destroy(b);
-      return rc;
-    }
+    if ((rc = b->d_tw.alloc((size_t)M * sizeof(float2))) || (rc = b->d_mixed.alloc_zero((size_t)S * b->fe.out_cap * sizeof(float2)))) return rc;
     cudaMemcpy(b->d_tw.p, tw.data(), (size_t)M * sizeof(float2), cudaMemcpyHostToDevice);
     const size_t smem = (size_t)M * (3 * sizeof(float2) + CG_FT * sizeof(float));
-    if (smem > (size_t)smem_cap) { pmr446_batch_destroy(b); return fail(PMR446_EINVAL, "num_channels too large for the shared-memory FFT"); }
+    if (smem > (size_t)smem_cap) return fail(PMR446_EINVAL, "num_channels too large for the shared-memory FFT");
     cudaFuncSetAttribute(channelize_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     b->generic_tile = cfg->pfb_m == 13 && channelize_generic_tile_smem(M) <= (size_t)smem_cap;
     if (b->generic_tile)
@@ -175,41 +160,23 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
   }
 
   b->max_tiles = (int)(b->max_ns / CH_TL + 3);
-  if (!b->generic && (rc = b->d_mag.alloc_zero((size_t)S * b->max_tiles * 16 * sizeof(float)))) { pmr446_batch_destroy(b); return rc; }
+  if (!b->generic && (rc = b->d_mag.alloc_zero((size_t)S * b->max_tiles * 16 * sizeof(float)))) return rc;
   // demod ring: history for the audio FIR halo + one chunk
   b->demod_cap = next_pow2(b->max_ns + std::max(AU_MAXHALO + AU_MAXLEAD, AF_N) + 64);
-  if ((rc = b->d_demod.alloc_zero((size_t)S * M * b->demod_cap * sizeof(float)))) { pmr446_batch_destroy(b); return rc; }
+  if ((rc = b->d_demod.alloc_zero((size_t)S * M * b->demod_cap * sizeof(float)))) return rc;
 
-  // audio filters
-  std::vector<float> hp(PMR446_HP_AUDIO_TAPS_LEN), lp(PMR446_LP_AUDIO_TAPS_LEN);
-  pmr446_hp_audio_taps_fill(hp.data());
-  pmr446_lp_audio_taps_fill(lp.data());
-  const float* hpt = cfg->hp_taps ? cfg->hp_taps : hp.data();
-  unsigned hpn = cfg->hp_taps ? cfg->hp_len : (unsigned)hp.size();
-  const float* lpt = cfg->lp_taps ? cfg->lp_taps : lp.data();
-  unsigned lpn = cfg->lp_taps ? cfg->lp_len : (unsigned)lp.size();
-  if (hpn < 1 || hpn > (unsigned)AU_MAXHALO || (hpn & 1) == 0) { pmr446_batch_destroy(b); return fail(PMR446_EINVAL, "hp_len must be odd and <= 383"); }
-  if (lpn < 1 || lpn > (unsigned)AU_LEAD_LP - 16) { pmr446_batch_destroy(b); return fail(PMR446_EINVAL, "lp_len must be <= 112"); }
-  b->hp_delay = (int)(hpn - 1) / 2;  // wdelayf_create((HP_AUDIO_FILT_TAPS - 1) / 2), :447
-  if ((rc = upload_padded_taps(hpt, hpn, b->d_hp, &b->hp_chunks)) || (rc = upload_padded_taps(lpt, lpn, b->d_lp, &b->lp_chunks))) {
-    pmr446_batch_destroy(b);
-    return rc;
-  }
-  // de-emphasis pole: its warm-up sets the direct-form kernel's tile lead-in and the length of its impulse response below
-  b->de_warm = cfg->deemph_fir ? 0 : deemph_warmup(cfg->deemph_a1);
-  b->au_lead = b->de_warm < 0 ? -1 : audio_lead(cfg->lowpass != 0, b->lp_chunks, b->de_warm);
-  if (b->au_lead < 0) {
-    pmr446_batch_destroy(b);
-    return fail(PMR446_EINVAL, "deemph_a1 must satisfy |a1| < 1 with a warm-up that fits the audio tile (|a1| <= 0.977)");
-  }
+  // audio filters; the de-emphasis pole's warm-up also sets the length of its impulse response below
+  if ((rc = b->au.init(*cfg))) return rc;
   // fast-convolution response: hp (x gain) * de-emphasis * optional low-pass, as one impulse response < AF_HALO
   {
-    const unsigned fir_len = hpn + (cfg->lowpass ? lpn - 1 : 0) + (cfg->deemph_fir ? PMR446_FIR_DEEMPH_TAPS_LEN - 1 : 0);
+    const std::vector<float>& hpt = b->au.hp;
+    const std::vector<float>& lpt = b->au.lp;
+    const unsigned fir_len = (unsigned)hpt.size() + (cfg->lowpass ? (unsigned)lpt.size() - 1 : 0) + (cfg->deemph_fir ? PMR446_FIR_DEEMPH_TAPS_LEN - 1 : 0);
     const double a1 = cfg->deemph_a1;
-    const unsigned de_len = (unsigned)std::max(24, b->de_warm);   // the pole's response is cut where it is below 2^-30
+    const unsigned de_len = (unsigned)std::max(24, b->au.de_warm);   // the pole's response is cut where it is below 2^-30
     if (fir_len + de_len <= (unsigned)AF_HALO_LONG) {
       b->fft_halo = fir_len + de_len <= (unsigned)AF_HALO ? AF_HALO : AF_HALO_LONG;
-      std::vector<double> h(hpt, hpt + hpn);
+      std::vector<double> h(hpt.begin(), hpt.end());
       for (auto& x : h) x *= (double)cfg->audio_gain;
       // de-emphasis (A.1): y[n] = b0 x[n] + b1 x[n-1] - a1 y[n-1]
       std::vector<double> de(de_len);
@@ -228,7 +195,7 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
         return z;
       };
       h = conv(h, de);
-      if (cfg->lowpass) h = conv(h, std::vector<double>(lpt, lpt + lpn));
+      if (cfg->lowpass) h = conv(h, std::vector<double>(lpt.begin(), lpt.end()));
       std::vector<float2> resp(AF_N), tw(AF_N);
       for (int k = 0; k < AF_N; k++) {
         const double a = -2.0 * M_PI * (double)k / (double)AF_N;
@@ -245,21 +212,14 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
           }
           resp[k0 * 256 + t] = make_float2((float)(re / AF_N), (float)(im / AF_N));
         }
-      if ((rc = b->d_resp.alloc(AF_N * sizeof(float2))) || (rc = b->d_aftw.alloc(AF_N * sizeof(float2)))) { pmr446_batch_destroy(b); return rc; }
+      if ((rc = b->d_resp.alloc(AF_N * sizeof(float2))) || (rc = b->d_aftw.alloc(AF_N * sizeof(float2)))) return rc;
       cudaMemcpy(b->d_resp.p, resp.data(), AF_N * sizeof(float2), cudaMemcpyHostToDevice);
       cudaMemcpy(b->d_aftw.p, tw.data(), AF_N * sizeof(float2), cudaMemcpyHostToDevice);
       b->fft_audio = true;
     }
   }
-  if (cfg->deemph_fir && !b->fft_audio) {
-    pmr446_batch_destroy(b);
-    return fail(PMR446_EINVAL, "deemph_fir needs the fast-convolution audio path (filters too long for its tile)");
-  }
-  if (cfg->waterfall > 0) {
-    if ((rc = b->wf.init(S, cfg->waterfall))) { pmr446_batch_destroy(b); return rc; }
-  }
-  cudaFuncSetAttribute(audio_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-  cudaFuncSetAttribute(audio_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  if (cfg->deemph_fir && !b->fft_audio) return fail(PMR446_EINVAL, "deemph_fir needs the fast-convolution audio path (filters too long for its tile)");
+  if (cfg->waterfall > 0 && (rc = b->wf.init(S, cfg->waterfall))) return rc;
   cudaFuncSetAttribute(audio_fft4_kernel<AF_HALO>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF4_SMEM_BYTES);
   cudaFuncSetAttribute(audio_fft4_kernel<AF_HALO_LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF4_SMEM_BYTES);
   CUDA_TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking));
@@ -271,11 +231,8 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
     CUDA_TRY(cudaEventCreateWithFlags(&b->ev_free[i], cudaEventDisableTiming));
   }
   // every table upload and attribute call above is synchronous: one check for all of them
-  if (cudaDeviceSynchronize() != cudaSuccess || cudaGetLastError() != cudaSuccess) {
-    pmr446_batch_destroy(b);
-    return fail(PMR446_ECUDA, "CUDA error while setting up the batch");
-  }
-  *out = b;
+  if (cudaDeviceSynchronize() != cudaSuccess || cudaGetLastError() != cudaSuccess) return fail(PMR446_ECUDA, "CUDA error while setting up the batch");
+  *out = b.release();
   return PMR446_OK;
 }
 
@@ -348,9 +305,16 @@ extern "C" int pmr446_batch_reset(pmr446_batch* b) {
   return PMR446_OK;
 }
 
-static size_t audio_smem_bytes() {
-  size_t xn = AU_MAXHALO + AU_SPAN + 16, yn = AU_LEAD_LP + AU_SPAN + 16;
-  return ((xn + xn / 16 + 1) + (yn + yn / 16 + 1) + 384 + 128 + 8) * sizeof(float);
+long long pmr::batch_frames_after(const pmr446_batch* b, unsigned n) {
+  return b->fe.outputs_after(b->fe.n_in + (long long)n) / b->M - b->fe.n_out / b->M;
+}
+
+// The caller's leading dimensions against the counts of a call of n samples (closed form), before any state advances: a
+// rejected call leaves the handle untouched.
+static int check_ld(const pmr446_batch* b, unsigned n, const pmr446_outputs* out) {
+  if (out->res && b->fe.outputs_after(b->fe.n_in + (long long)n) - b->fe.n_out > out->res_ld) return fail(PMR446_ERANGE, "res_ld too small");
+  if ((out->chan || out->demod || out->lpcomp || out->audio || out->pcm) && batch_frames_after(b, n) > out->ld) return fail(PMR446_ERANGE, "ld too small");
+  return PMR446_OK;
 }
 
 extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long long iq_stride, unsigned n, const pmr446_outputs* out,
@@ -362,16 +326,12 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
   const int S = b->S;
   b->launches = 0;
 
-  // ---- validate against the closed-form counts BEFORE any state advances: a failed call leaves the handle untouched ----
+  // ---- validate BEFORE any state advances: a failed call leaves the handle untouched ----------
   const int M = b->M;
-  {
-    const long long r0p = b->fe.n_out, r1p = b->fe.outputs_after(b->fe.n_in + (long long)n);
-    const long long nyp = r1p - r0p, nsp = r1p / M - r0p / M;
-    if (out->res && nyp > out->res_ld) return fail(PMR446_ERANGE, "res_ld too small");
-    if ((out->chan || out->demod || out->lpcomp || out->audio || out->pcm) && nsp > out->ld) return fail(PMR446_ERANGE, "ld too small");
-    if ((out->rssi || out->chan_edge) && b->generic) return fail(PMR446_EINVAL, "rssi / chan_edge outputs need the 16-channel kernel");
-    if (!b->generic && (r1p / M + CH_TL - 1) / CH_TL - r0p / M / CH_TL > b->max_tiles) return fail(PMR446_ERANGE, "internal: tile count exceeds allocation");
-  }
+  if (int rc = check_ld(b, n, out)) return rc;
+  if ((out->rssi || out->chan_edge) && b->generic) return fail(PMR446_EINVAL, "rssi / chan_edge outputs need the 16-channel kernel");
+  const long long tf0 = b->fe.n_out / M, tf1 = tf0 + batch_frames_after(b, n);
+  if (!b->generic && (tf1 + CH_TL - 1) / CH_TL - tf0 / CH_TL > b->max_tiles) return fail(PMR446_ERANGE, "internal: tile count exceeds allocation");
   // ---- front end: [r0, r1) new resampler outputs in fe.out ring ------------------------------
   long long r0 = b->fe.n_out, r1 = 0;
   b->timer.mark(st, TM_START);
@@ -512,34 +472,21 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
     }
     if (fft_now ? out->lpcomp != nullptr : (out->audio || out->pcm || out->lpcomp)) {
       AudioParams ap;
+      memset(&ap, 0, sizeof ap);
       ap.demod = (const float*)b->d_demod.p;
       ap.demod_stride = b->demod_cap;
       ap.demod_mask = b->demod_cap - 1;
       ap.rows = S * M;
-      ap.lead = b->au_lead;
-      const long long own = AU_SPAN - ap.lead;
+      const long long own = AU_SPAN - b->au.lead;
       ap.tile0 = f0 / own;
       ap.tiles = (int)((f1 + own - 1) / own - ap.tile0);
       ap.f0 = f0;
       ap.f1 = f1;
-      ap.row_range = nullptr;
-      ap.lpcomp_ld = 0;
-      ap.hp_taps = (const float*)b->d_hp.p;
-      ap.hp_chunks = b->hp_chunks;
-      ap.hp_delay = b->hp_delay;
-      ap.lp_taps = b->cfg.lowpass ? (const float*)b->d_lp.p : nullptr;
-      ap.lp_chunks = b->lp_chunks;
-      ap.gain = b->cfg.audio_gain;
-      ap.de_b0 = b->cfg.deemph_b0;
-      ap.de_b1 = b->cfg.deemph_b1;
-      ap.de_a1 = b->cfg.deemph_a1;
       ap.audio = fft_now ? nullptr : out->audio;
       ap.pcm = fft_now ? nullptr : out->pcm;
       ap.lpcomp = out->lpcomp;
       ap.out_ld = out->ld;
-      ap.de_warm = b->de_warm;
-      if (b->de_warm > 8) audio_kernel<true><<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, audio_smem_bytes(), st>>>(ap);
-      else audio_kernel<false><<<(unsigned)((long long)ap.rows * ap.tiles), AU_THREADS, audio_smem_bytes(), st>>>(ap);
+      b->au.launch(ap, st);
       b->launches++;
       b->timer.mark(st, TM_AUDIO);
     }
@@ -565,10 +512,9 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
   const int S = b->S, M = b->M;
   const size_t bps = (size_t)fmt_bytes_per_sample(b->cfg.in_fmt);
   const unsigned W = b->cfg.waterfall;
-  if (iq_stride < (long long)(n * bps)) {   // a single stream may pass stride 0
-    if (S > 1) return fail(PMR446_EINVAL, "iq_stride smaller than one stream's chunk");
-    iq_stride = (long long)(n * bps);
-  }
+  if ((iq_stride = host_iq_stride(iq_stride, n, bps, S)) < 0) return (int)iq_stride;
+  int rc;
+  if ((rc = check_ld(b, n, out))) return rc;   // the caller's dimensions, before the first slice advances the state
   // Large chunks are cut in time into sub-chunks so that the host->device copy of sub-chunk k+1 overlaps
   // the kernels of sub-chunk k (all filter state carries across execute_device calls, so the result is the
   // same).  Not done when a waterfall row is requested: asgram produces one row per call (:911-912).
@@ -577,55 +523,38 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
   const unsigned K = (!want_wf && !want_sel && n >= 8u * 65536u) ? 8u : 1u;
   const unsigned sub = K == 1 ? n : ((n + K - 1) / K + 255u) / 256u * 256u;
   const long long pitch = ((long long)(sub ? sub : 1) * (long long)bps + 255) / 256 * 256;
-  int rc;
   for (int i = 0; i < (K > 1 ? 2 : 1); i++)
     if ((rc = b->d_in2[i].ensure((size_t)S * pitch))) return rc;
   pmr446_outputs d = *out;
   const long long ld = b->max_ns, rld = b->max_res;
   d.ld = ld;
   d.res_ld = rld;
-  int stage_rc = 0;   // a failed staging allocation must fail the call, not silently drop the output
-  auto stage = [&](const void* host, DevBuf& buf, size_t bytes) -> void* {
-    if (!host) return nullptr;
-    if (int e = buf.ensure(bytes)) { stage_rc = e; return nullptr; }
-    return buf.p;
-  };
-  d.res = (float*)stage(out->res, b->d_out_res, (size_t)S * rld * 8);
-  d.chan = (float*)stage(out->chan, b->d_out_chan, (size_t)S * M * ld * 8);
-  d.demod = (float*)stage(out->demod, b->d_out_demod, (size_t)S * M * ld * 4);
-  d.lpcomp = (float*)stage(out->lpcomp, b->d_out_lpcomp, (size_t)S * M * ld * 4);
-  d.audio = (float*)stage(out->audio, b->d_out_audio, (size_t)S * M * ld * 4);
-  d.pcm = (int16_t*)stage(out->pcm, b->d_out_pcm, (size_t)S * M * ld * 2);
-  d.ascii = (char*)stage(W ? out->ascii : nullptr, b->d_out_ascii, (size_t)S * W);
-  d.peak = (float*)stage(W ? out->peak : nullptr, b->d_out_peak, (size_t)S * 2 * 4);
-  d.psd = (float*)stage(W ? out->psd : nullptr, b->d_out_psd, (size_t)S * 4 * W * 4);
-  d.rssi = (float*)stage(out->rssi, b->d_out_rssi, (size_t)S * M * 4);
-  d.chan_edge = (float*)stage(out->chan_edge, b->d_out_edge, (size_t)S * M * 2 * 8);
-  if (stage_rc) return stage_rc;
-  {  // the caller's leading dimensions against the closed-form totals, before the first slice advances the state
-    const long long r0p = b->fe.n_out, r1p = b->fe.outputs_after(b->fe.n_in + (long long)n);
-    if (out->res && r1p - r0p > out->res_ld) return fail(PMR446_ERANGE, "res_ld too small");
-    if ((out->chan || out->demod || out->lpcomp || out->audio || out->pcm) && r1p / M - r0p / M > out->ld) return fail(PMR446_ERANGE, "ld too small");
-  }
+  Staging stage;
+  d.res = stage(out->res, b->d_out_res, (size_t)S * rld * 8);
+  d.chan = stage(out->chan, b->d_out_chan, (size_t)S * M * ld * 8);
+  d.demod = stage(out->demod, b->d_out_demod, (size_t)S * M * ld * 4);
+  d.lpcomp = stage(out->lpcomp, b->d_out_lpcomp, (size_t)S * M * ld * 4);
+  d.audio = stage(out->audio, b->d_out_audio, (size_t)S * M * ld * 4);
+  d.pcm = stage(out->pcm, b->d_out_pcm, (size_t)S * M * ld * 2);
+  d.ascii = stage(W ? out->ascii : nullptr, b->d_out_ascii, (size_t)S * W);
+  d.peak = stage(W ? out->peak : nullptr, b->d_out_peak, (size_t)S * 2 * 4);
+  d.psd = stage(W ? out->psd : nullptr, b->d_out_psd, (size_t)S * 4 * W * 4);
+  d.rssi = stage(out->rssi, b->d_out_rssi, (size_t)S * M * 4);
+  d.chan_edge = stage(out->chan_edge, b->d_out_edge, (size_t)S * M * 2 * 8);
+  if (stage.rc) return stage.rc;
   unsigned ny_tot = 0, ns_tot = 0;
   int launches = 0;
   unsigned off = 0;
   // device -> host copies of a column range of every requested output; with time slices they run on their own stream
   // right behind each slice's kernels, i.e. concurrently with the next slices' host -> device copies (PCIe is duplex)
-  auto back = [&](cudaStream_t s2, void* host, const void* dev, long long hld, long long dld, size_t elt, long long rows, long long col0,
-                  long long cols) {
-    if (host && cols > 0)
-      cudaMemcpy2DAsync((char*)host + col0 * elt, hld * elt, (const char*)dev + col0 * elt, dld * elt, cols * elt, rows, cudaMemcpyDeviceToHost, s2);
-  };
   auto back_range = [&](cudaStream_t s2, unsigned y0, unsigned ny_k, unsigned s0, unsigned ns_k) {
-    back(s2, out->res, d.res, out->res_ld, rld, 8, S, y0, ny_k);
-    back(s2, out->chan, d.chan, out->ld, ld, 8, (long long)S * M, s0, ns_k);
-    back(s2, out->demod, d.demod, out->ld, ld, 4, (long long)S * M, s0, ns_k);
-    back(s2, out->lpcomp, d.lpcomp, out->ld, ld, 4, (long long)S * M, s0, ns_k);
-    back(s2, out->audio, d.audio, out->ld, ld, 4, (long long)S * M, s0, ns_k);
-    back(s2, out->pcm, d.pcm, out->ld, ld, 2, (long long)S * M, s0, ns_k);
+    copy_back(s2, out->res, d.res, out->res_ld, rld, 8, S, y0, ny_k);
+    copy_back(s2, out->chan, d.chan, out->ld, ld, 8, (long long)S * M, s0, ns_k);
+    copy_back(s2, out->demod, d.demod, out->ld, ld, 4, (long long)S * M, s0, ns_k);
+    copy_back(s2, out->lpcomp, d.lpcomp, out->ld, ld, 4, (long long)S * M, s0, ns_k);
+    copy_back(s2, out->audio, d.audio, out->ld, ld, 4, (long long)S * M, s0, ns_k);
+    copy_back(s2, out->pcm, d.pcm, out->ld, ld, 2, (long long)S * M, s0, ns_k);
   };
-  const bool any_rows = out->chan || out->demod || out->lpcomp || out->audio || out->pcm;
   for (unsigned k = 0; k == 0 || off < n; k++) {
     const unsigned len = std::min(sub, n - off);
     const int buf = (int)(k & 1u);
@@ -646,11 +575,6 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
     if (rc) return rc;
     launches += b->launches;
     CUDA_TRY(cudaEventRecord(b->ev_free[buf], st));
-    if ((out->res && ny_tot + ny > out->res_ld) || (any_rows && ns_tot + ns > out->ld)) {
-      cudaStreamSynchronize(st);
-      cudaStreamSynchronize(b->out_stream);
-      return fail(PMR446_ERANGE, out->res && ny_tot + ny > out->res_ld ? "res_ld too small" : "ld too small");
-    }
     if (K > 1) {
       CUDA_TRY(cudaEventRecord(b->ev_out, st));
       CUDA_TRY(cudaStreamWaitEvent(b->out_stream, b->ev_out, 0));
@@ -663,12 +587,12 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
   b->launches = launches;
   const unsigned ny = ny_tot, ns = ns_tot;
   if (K == 1) back_range(st, 0, ny, 0, ns);
-  back(st, out->rssi, d.rssi, M, M, 4, S, 0, M);
-  back(st, out->chan_edge, d.chan_edge, 2 * M, 2 * M, 8, S, 0, 2 * M);
+  copy_back(st, out->rssi, d.rssi, M, M, 4, S, 0, M);
+  copy_back(st, out->chan_edge, d.chan_edge, 2 * M, 2 * M, 8, S, 0, 2 * M);
   if (W) {
-    back(st, out->ascii, d.ascii, W, W, 1, S, 0, W);
-    back(st, out->peak, d.peak, 2, 2, 4, S, 0, 2);
-    back(st, out->psd, d.psd, 4 * W, 4 * W, 4, S, 0, 4 * W);
+    copy_back(st, out->ascii, d.ascii, W, W, 1, S, 0, W);
+    copy_back(st, out->peak, d.peak, 2, 2, 4, S, 0, 2);
+    copy_back(st, out->psd, d.psd, 4 * W, 4 * W, 4, S, 0, 4 * W);
   }
   CUDA_TRY(cudaStreamSynchronize(st));
   CUDA_TRY(cudaStreamSynchronize(b->out_stream));

@@ -193,6 +193,24 @@ def test_failed_execute_leaves_state_untouched():
     da.close()
     db.close()
     assert ra["nz"] == rb["nz"] and np.array_equal(ra["pcm"], rb["pcm"])
+    # receiver path
+    xa = chain.PmrReceiver(n_streams=1, fs_in=fs, in_fmt=1, audio_gain=1.0, max_chunk=n)
+    xb = chain.PmrReceiver(n_streams=1, fs_in=fs, in_fmt=1, audio_gain=1.0, max_chunk=n)
+    xa.execute(iq[:, :2 * n])
+    xb.execute(iq[:, :2 * n])
+    from sdr_pmr446_b200._lib import RxOutputs
+    xbad = RxOutputs()
+    audio, pcm = np.zeros((1, 10), np.float32), np.zeros((1, 10), np.int16)
+    xbad.audio, xbad.pcm, xbad.ld = audio.ctypes.data, pcm.ctypes.data, 10
+    rc = lib().pmr446_receiver_execute(xb.h, chunk2.ctypes.data, chunk2.strides[0], n, C.byref(xbad), None)
+    assert rc == ERANGE
+    ra, rb = xa.execute(chunk2), xb.execute(chunk2)
+    xa.close()
+    xb.close()
+    assert ra["ns"] == rb["ns"]
+    for k in chain.PmrReceiver.STATUS_FIELDS:
+        assert np.array_equal(ra[k], rb[k]), k
+    assert np.array_equal(ra["audio"], rb["audio"]) and np.array_equal(ra["pcm"], rb["pcm"])
 
 
 @pytest.mark.parametrize("fs,M,fmt_cu8", [(3200000, 16, True), (1024000, 20, True), (500000, 16, False), (4800000, 16, True)])

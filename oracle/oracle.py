@@ -248,7 +248,7 @@ class RxOracle:
 
     STATUS_FIELDS = ("state", "active_chan", "rssi", "n_audio", "tone_detected", "ctcss_index", "ctcss_freq", "max_power", "events")
 
-    def __init__(self, squelch_level=18.0, channel_mask=2 ** 64 - 1, lock_mode=0, ctcss_block=2441, **chain_kw):
+    def __init__(self, squelch_level=18.0, channel_mask=2 ** 64 - 1, lock_mode=0, ctcss_block=2441, ctcss_dc_alpha=0.0005, **chain_kw):
         self.cfg = RxCfg()
         lib().oracle_rx_default_cfg(C.byref(self.cfg))
         for k, v in chain_kw.items():
@@ -259,6 +259,7 @@ class RxOracle:
         self.cfg.channel_mask = channel_mask
         self.cfg.lock_mode = lock_mode
         self.cfg.ctcss_block = ctcss_block
+        self.cfg.ctcss_dc_alpha = ctcss_dc_alpha
         self.h = lib().oracle_rx_create(C.byref(self.cfg))
         if not self.h:
             raise RuntimeError("oracle_rx_create failed")
@@ -273,12 +274,12 @@ class RxOracle:
     __del__ = close
 
     def execute(self, iq):
-        """One chunk -> dict(status fields, rssi_ch [M], audio, pcm, ctcss_in [n_audio], ctcss_power [38], ns)."""
+        """One chunk -> dict(status fields, rssi_ch [M], chan [M, ns], audio, pcm, ctcss_in [n_audio], ctcss_power [38], ns)."""
         iq = np.ascontiguousarray(iq)
         n = iq.shape[0] // 2 if self.cfg.chain.in_fmt == FMT_CU8 else iq.shape[0]
         ld = self.chan_size
         bufs = {"rssi": np.zeros(self.M, np.float32), "audio": np.zeros(ld, np.float32), "pcm": np.zeros(ld, np.int16),
-                "ctcss_in": np.zeros(ld, np.float32), "ctcss_power": np.zeros(38, np.float32)}
+                "ctcss_in": np.zeros(ld, np.float32), "ctcss_power": np.zeros(38, np.float32), "chan": np.zeros((self.M, ld), np.complex64)}
         out = RxOut()
         out.ld = ld
         for k, v in bufs.items():
@@ -291,6 +292,7 @@ class RxOracle:
         r["ns"] = ns.value
         r["rssi_ch"] = bufs["rssi"]
         r["ctcss_power"] = bufs["ctcss_power"]
+        r["chan"] = bufs["chan"][:, :ns.value]
         for k in ("audio", "pcm", "ctcss_in"):
             r[k] = bufs[k][:st.n_audio]
         return r

@@ -171,7 +171,7 @@ class PmrReceiver:
 
     STATUS_FIELDS = ("state", "active_chan", "rssi", "n_audio", "tone_detected", "ctcss_index", "ctcss_freq", "max_power", "events")
 
-    def __init__(self, squelch_level=18.0, channel_mask=2 ** 64 - 1, lock_mode=0, ctcss_block=2441, **chain_kw):
+    def __init__(self, squelch_level=18.0, channel_mask=2 ** 64 - 1, lock_mode=0, ctcss_block=2441, ctcss_dc_alpha=0.0005, **chain_kw):
         self.cfg = _lib.RxConfig()
         lib().pmr446_rx_default_config(C.byref(self.cfg))
         for k, v in chain_kw.items():
@@ -182,6 +182,7 @@ class PmrReceiver:
         self.cfg.channel_mask = channel_mask
         self.cfg.lock_mode = lock_mode
         self.cfg.ctcss_block = ctcss_block
+        self.cfg.ctcss_dc_alpha = ctcss_dc_alpha
         h = C.c_void_p()
         check(lib().pmr446_receiver_create(C.byref(self.cfg), C.byref(h)), "pmr446_receiver_create")
         self.h = h

@@ -46,3 +46,22 @@ def steady_chunks(rows, carriers, chunk=CHUNK, fs=FS):
         if run >= 3:
             good.append(k)
     return good
+
+
+def ctcss_change():
+    """Channel 5 keyed for the whole capture: 67.0 Hz, then 100.0 Hz from 1.0 s, then no tone from 2.0 s."""
+    return (synth.Carrier(5, 0.2, 800.0, 67.0, t_off=1.0), synth.Carrier(5, 0.2, 800.0, 100.0, t_on=1.0, t_off=2.0),
+            synth.Carrier(5, 0.2, 800.0, 0.0, t_on=2.0))
+
+
+def rx_sizes(n, chunk):
+    """Call sizes covering n input samples: full calls with 0-, 1- and 7-sample calls (and one that completes about one
+    frame) early, while the receiver still scans, and again later, while it is tuned."""
+    sizes = [0, 1, 7, chunk - 3, 83, chunk, 0, chunk - 1]
+    k = 0
+    while sum(sizes) < n:
+        sizes.append(min(chunk - 17 * (k % 3), n - sum(sizes)))
+        if len(sizes) == 14:
+            sizes += [0, 7, 1, 81]
+        k += 1
+    return sizes

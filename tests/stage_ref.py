@@ -29,6 +29,12 @@ liquid-dsp:
               interpolation (rate > 1): the arbitrary resampler first, then the half-band stages from index 0 up, each
               input n giving y[2 n] = x[n - m] (delay branch) and y[2 n + 1] = sum_j hb[g][j] x[n - j] (filter branch;
               resamp2_interp, msresamp2_interp), no scale.
+  receiver    (oracle/receiver.c) rssi = 20 log10(mean |y|) per channel and call; the squelch / selector step and the
+              38-tone Goertzel bank restated bit-exactly in float32 (NumPy rounds every operation and never fuses, the
+              oracle builds with -ffp-contract=off and the kernels use explicitly rounded operations); the selected
+              stream = the active channel's frames of every tuned call, sample 0 of a call discriminated against the last
+              frame of the previous tuned call's then-active channel (0 at start and after a detune); the CTCSS branch's
+              iirfilt_rrrf DC blocker v0 = x - a1 v1, y = v0 - v1 with a1 = fl32(-1 + alpha).
 """
 import numpy as np
 from scipy import signal
@@ -276,3 +282,192 @@ def check_asgram(psd, peak, ascii, psd64, peak64, tol_db):
     near = np.min(np.abs(val[:, None] - edges[None, :]), axis=1) < tol_db
     assert np.all((ascii == asgram_chars(val)) | near)
     return err
+
+
+# ---- receiver (oracle/receiver.c, pmr446_receiver_*) ---------------------------------------------------------------------
+CTCSS_FREQS = np.array([67.0, 71.9, 74.4, 77.0, 79.7, 82.5, 85.4, 88.5, 91.5, 94.8, 97.4, 100.0, 103.5, 107.2, 110.9, 114.8,
+                        118.8, 123.0, 127.3, 131.8, 136.5, 141.3, 146.2, 151.4, 156.7, 162.2, 167.9, 173.8, 179.9, 186.2,
+                        192.8, 203.5, 210.7, 218.1, 225.7, 233.6, 241.8, 250.3], np.float32)   # include/pmr446_taps.h
+EV_TUNED, EV_CHANGED, EV_DETUNED, EV_CTCSS_ACQUIRED, EV_CTCSS_CHANGED, EV_CTCSS_LOST = 1, 2, 4, 8, 16, 32
+_F = np.float32
+
+
+def rssi(chan):
+    """20 log10(mean |y|) of every channel of one call (float64); a call with no frame gives NaN (0 / 0)."""
+    y = np.asarray(chan, np.complex128)
+    if y.shape[-1] == 0:
+        return np.full(y.shape[:-1], np.nan)
+    return 20.0 * np.log10(np.mean(np.abs(y), axis=-1))
+
+
+def ctcss_coef(channel_width=12500):
+    """2 cos(2 pi f / fs_audio) per tone in float32, as pmr446_receiver_create and the oracle form it: the argument is
+    rounded to float32 and cosf of it (correctly rounded here) doubled."""
+    arg = ((2.0 * np.pi * CTCSS_FREQS.astype(np.float64)) / float(channel_width)).astype(np.float32)
+    return (_F(2.0) * np.cos(arg.astype(np.float64)).astype(np.float32)).astype(np.float32)
+
+
+def tone_bank_state():
+    """ctcss_detector_reset: the tone bank's state (u0, u1 and the last block's powers, all float32)."""
+    z = np.zeros(len(CTCSS_FREQS), np.float32)
+    return {"u0": z.copy(), "u1": z.copy(), "power": z.copy(), "max_power": _F(0.0), "index": 0, "samp": 0, "tone": 0}
+
+
+def rx_state():
+    """A receiver's state at creation and after reset (proc_scanning, no channel, ctcss_freq -1)."""
+    return {"state": 0, "active": -1, "rssi": _F(0.0), "ctcss_freq": _F(-1.0), "bank": tone_bank_state()}
+
+
+def squelch_step(state, rssi_ch_f32, cfg):
+    """One call of the squelch / selector state machine on the float32 RSSI of every channel; updates `state` (rx_state())
+    in place and returns the events (1 tuned, 2 channel changed, 4 detuned).  cfg: squelch (float32), mask, lock_mode.
+
+    Bit-exact to squelch_kernel and oracle/receiver.c: the sum over the enabled channels in channel order and
+    top - sum / enabled in float32, the first enabled channel wins ties and -- with every RSSI NaN (a call with no
+    frame) -- counts as the strongest; a NaN spread neither tunes nor detunes; the detune test in double.  A detune
+    clears the discriminator's previous sample (the caller's business: the selected stream restarts from 0) and the tone
+    bank, not the CTCSS DC blocker."""
+    r = np.asarray(rssi_ch_f32, np.float32)
+    best, enabled, top, total = -1, 0, _F(0.0), _F(0.0)
+    for i in range(r.shape[0]):
+        if not (int(cfg["mask"]) >> i) & 1:
+            continue
+        enabled += 1
+        total = _F(total + r[i])
+        if best < 0 or r[i] > top:
+            top, best = r[i], i
+    spread = _F(top - _F(total / _F(enabled)))
+    ev = 0
+    state["rssi"] = spread
+    sq = _F(cfg["squelch"])
+    if state["state"] == 0:
+        if spread > sq:
+            state["active"], state["state"] = best, 1
+            ev |= EV_TUNED
+    else:
+        if cfg["lock_mode"] == 1 and state["active"] != best:
+            state["active"] = best
+            ev |= EV_CHANGED
+        if float(spread) < float(sq) - 5.0:
+            state["active"], state["state"], state["ctcss_freq"] = -1, 0, _F(0.0)
+            state["bank"] = tone_bank_state()
+            ev |= EV_DETUNED
+    return ev
+
+
+def ctcss_bank(x_f32, coef, block, bank):
+    """ctcss_detector_analyze over one call's DC-blocked CTCSS branch (float32), bit-exact to ctcss_kernel: the 38
+    Goertzel recurrences u0 <- (x + coef u0) - u1, and at the end of every `block` samples the powers
+    (u0 u0 + u1 u1) - (coef u0) u1, their float32 sum in tone order over 38, the first strict maximum above 0 (the index is
+    kept when none is) and tone = avg > 120 and max / avg > 10.  Updates `bank` (tone_bank_state()) in place and
+    returns the CTCSS events of the call (8 acquired, 16 code changed, 32 lost)."""
+    x = np.asarray(x_f32, np.float32)
+    coef = np.asarray(coef, np.float32)
+    had_tone, had_code = bank["tone"], bank["index"]
+    u0, u1, samp = bank["u0"].copy(), bank["u1"].copy(), bank["samp"]
+    i, n = 0, x.shape[0]
+    while i < n:
+        e = min(n, i + block - samp)
+        for k in range(i, e):
+            u0, u1 = (x[k] + coef * u0) - u1, u0
+        samp += e - i
+        i = e
+        if samp == block:
+            p = ((u0 * u0) + (u1 * u1)) - ((coef * u0) * u1)
+            bank["power"] = p
+            u0, u1 = np.zeros_like(u0), np.zeros_like(u1)
+            avg = _F(np.cumsum(p, dtype=np.float32)[-1] / _F(len(p)))   # cumsum: sequential, in tone order
+            j = int(np.argmax(p))
+            mx = p[j] if p[j] > 0 else _F(0.0)
+            if p[j] > 0:
+                bank["index"] = j
+            bank["max_power"] = mx
+            bank["tone"] = int(bool(avg > _F(120.0)) and bool(_F(mx / avg) > _F(10.0)))
+            samp = 0
+    bank["u0"], bank["u1"], bank["samp"] = u0, u1, samp
+    ev = 0
+    if bank["tone"]:
+        if not had_tone:
+            ev |= EV_CTCSS_ACQUIRED
+        elif had_code != bank["index"]:
+            ev |= EV_CTCSS_CHANGED
+    elif had_tone:
+        ev |= EV_CTCSS_LOST
+    return ev
+
+
+def selected_stream(chan_calls, active_per_call, kf=0.5, wrong_first=False):
+    """The discriminator output the selected chain sees over a run of calls from a fresh (or reset) receiver, float64.
+
+    chan_calls: per call the channel samples [M][ns] (ns may be 0); active_per_call: the active channel after that call's
+    squelch step (-1 = none).  The active channel's samples of every tuned call, sample 0 of a call discriminated
+    against the last sample of the previous tuned call's then-active channel -- 0 at start and after a detune (a call
+    with no active channel) -- with the component-wise products of `discriminator`, so the sign-of-zero cases match.
+    wrong_first: discriminate sample 0 against the NEW channel's own previous frame instead (what an append that ignores
+    channel changes and resets would play; a self-check of the tests' bounds).  Returns (stream, call_starts)."""
+    parts, starts, pos = [], [], 0
+    prev = 0j
+    own_prev = {}
+    for ch, a in zip(chan_calls, active_per_call):
+        ch = np.asarray(ch, np.complex128)
+        ns = ch.shape[-1]
+        starts.append(pos)
+        if a < 0:
+            prev = 0j
+        elif ns:
+            p0 = own_prev.get(a, 0j) if wrong_first else prev
+            y = ch[a]
+            parts.append(discriminator(np.concatenate([[p0], y])[None, :], kf)[0, 1:])
+            pos += ns
+            prev = y[-1]
+        for c in range(ch.shape[0]):
+            if ns:
+                own_prev[c] = ch[c, -1]
+    return (np.concatenate(parts) if parts else np.zeros(0)), starts
+
+
+def dc_block_real(x, alpha):
+    """iirfilt_rrrf_create_dc_blocker(alpha) in float64: v0 = x - a1 v1, y = v0 - v1, a1 = fl32(-1 + alpha), zero state."""
+    a1 = float(_F(_F(-1.0) + _F(alpha)))
+    return signal.lfilter([1.0, -1.0], [1.0, a1], np.asarray(x, np.float64))
+
+
+def rx_cfg(squelch_level=18.0, channel_mask=2 ** 64 - 1, lock_mode=0, **_):
+    return {"squelch": np.float32(squelch_level), "mask": int(channel_mask), "lock_mode": int(lock_mode)}
+
+
+def same_f32(a, b):
+    """Bitwise equality of float32 values (every NaN equal to every NaN: their payloads are not part of the contract)."""
+    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
+    return a.shape == b.shape and bool(np.all((a.view(np.uint32) == b.view(np.uint32)) | (np.isnan(a) & np.isnan(b))))
+
+
+def replay_rx(rows, rssi_ch, ctcss_in, cfg, block=2441, coef=None):
+    """squelch_step + ctcss_bank over a run of calls from a fresh receiver, fed `rssi_ch[k]` and `ctcss_in[k]` (the
+    implementation's own float32 values).  Yields per call (state dict snapshot, events)."""
+    coef = ctcss_coef() if coef is None else coef
+    st = rx_state()
+    for k in range(len(rows)):
+        ev = squelch_step(st, rssi_ch[k], cfg)
+        if st["active"] >= 0:
+            ev |= ctcss_bank(ctcss_in[k], coef, block, st["bank"])
+            st["ctcss_freq"] = CTCSS_FREQS[st["bank"]["index"]]
+        yield st, ev
+
+
+def check_replay(rows, cfg, block):
+    """The replay of squelch_step / ctcss_bank from the rows' own rssi_ch and ctcss_in reproduces every status field, the
+    events and the Goertzel powers bitwise.  Returns the events seen."""
+    seen = 0
+    rs = [r["rssi_ch"] for r in rows]
+    cs = [r["ctcss_in"][:int(r["n_audio"])] for r in rows]
+    for k, (st, ev) in enumerate(replay_rx(rows, rs, cs, cfg, block)):
+        r, b = rows[k], st["bank"]
+        want = {"state": st["state"], "active_chan": st["active"], "events": ev, "n_audio": r["ns"] if st["active"] >= 0 else 0,
+                "ctcss_index": b["index"], "tone_detected": b["tone"]}
+        for f, v in want.items():
+            assert int(r[f]) == int(v), (k, f, int(r[f]), int(v))
+        for f, v in (("rssi", st["rssi"]), ("max_power", b["max_power"]), ("ctcss_freq", st["ctcss_freq"]), ("ctcss_power", b["power"])):
+            assert same_f32(r[f], v), (k, f, r[f], v)
+        seen |= ev
+    return seen

@@ -290,6 +290,7 @@ def test_selector_taps_rssi_and_edge_samples():
     import torch
     from sdr_pmr446_b200 import chain, synth
     from sdr_pmr446_b200._lib import check, lib
+    from test_gpu_receiver_ref import RSSI_TOL_DB
     fs, S = 2400000, 2
     iq = np.stack([synth.make_cu8(synth.CaptureSpec(fs=float(fs), carriers=synth.rotated_carriers(s)), 500000, 470 + s) for s in range(S)])
     gpu = chain.PmrBatch(n_streams=S, fs_in=fs, in_fmt=1, audio_gain=1.0, max_chunk=240000)
@@ -302,7 +303,7 @@ def test_selector_taps_rssi_and_edge_samples():
             assert np.all(np.isnan(g["rssi"]))
             continue
         want = 20 * np.log10(np.mean(np.abs(g["chan"].astype(np.complex128)), axis=2))
-        assert np.max(np.abs(g["rssi"] - want)) < 1e-3
+        assert np.max(np.abs(g["rssi"] - want)) < RSSI_TOL_DB
         assert np.array_equal(g["chan_edge"][:, :, 0], g["chan"][:, :, 0]) and np.array_equal(g["chan_edge"][:, :, 1], g["chan"][:, :, ns - 1])
         sel = torch.tensor([3, -1], dtype=torch.int32, device="cuda")
         row = torch.full((S, gpu.max_ns), -7.0, dtype=torch.float32, device="cuda")

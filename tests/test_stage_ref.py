@@ -166,3 +166,76 @@ def test_msresamp_interp_matches_oracle(fs, fmt):
     inside = np.abs(au) < 0.999
     assert np.mean(inside) > 0.95
     stage_ref.check_pcm(pcm[inside], au[inside], float(np.max(np.abs(audio - au))))
+
+
+# ---- receiver: squelch / selector, tone bank, RSSI, selected stream ------------------------------------------------------
+RX_CASES = {"keyed_two_calls": ({}, "keyed_two_calls"), "stronger_later_lock_max": ({"lock_mode": 1}, "stronger_later"),
+            "ctcss_change": ({}, "ctcss_change")}
+
+
+def _rx_oracle_rows(case, block=2441, alpha=0.0005):
+    import rx_scenarios as sc
+    from oracle import oracle as orc
+    kw, scen = RX_CASES[case]
+    car = getattr(sc, scen)()
+    iq = sc.capture(car)
+    o = orc.RxOracle(fs_in=sc.FS, in_fmt=1, chunk=sc.CHUNK, audio_gain=1.0, ctcss_block=block, ctcss_dc_alpha=alpha, **kw)
+    rows, p = [], 0
+    for k in sc.rx_sizes(iq.shape[0] // 2, sc.CHUNK):
+        rows.append(o.execute(iq[2 * p:2 * (p + k)]))
+        p += k
+    o.close()
+    return rows, kw
+
+
+@pytest.mark.parametrize("block", [2441, 1, 5000])
+@pytest.mark.parametrize("case", sorted(RX_CASES))
+def test_squelch_and_tone_bank_replay_oracle(case, block):
+    """stage_ref.squelch_step and stage_ref.ctcss_bank replayed from the oracle's own rssi_ch and ctcss_in reproduce its
+    state, active channel, spread, events, tone flag, code, maximum and every Goertzel power bitwise in every call."""
+    rows, kw = _rx_oracle_rows(case, block)
+    seen = stage_ref.check_replay(rows, stage_ref.rx_cfg(**kw), block)
+    assert seen & 1 and (seen & 8 or block == 1)
+    if case == "keyed_two_calls":
+        assert seen & 4
+    if case == "stronger_later_lock_max":
+        assert seen & 2
+    if case == "ctcss_change" and block == 2441:
+        assert seen & 16 and seen & 32
+
+
+# ~3x the float32 oracle's own distance from float64, measured on these three runs: rssi 1.5e-5 dB (a float32 running
+# sum of ~1 221 magnitudes), audio 3.0e-7 relative RMS / 2.9e-6 of the RMS per sample, ctcss_in 3.8e-6 of the
+# discriminator RMS per sample
+RX_RSSI_TOL_DB = 5e-5
+RX_AUDIO_TOL_RMS, RX_AUDIO_TOL_MAX = 1e-6, 1e-5
+RX_CTCSS_TOL = 1.2e-5
+
+
+@pytest.mark.parametrize("case", sorted(RX_CASES))
+def test_receiver_stages_match_oracle(case):
+    """stage_ref.rssi of the oracle's channel samples against its rssi_ch; selected_stream -> stage_ref.audio ->
+    dc_block_real against its audio, s16 and ctcss_in, per sample over everything it played (every call, key-up,
+    detune, retune and channel changes included)."""
+    from liquid_api import reference_taps
+    rows, kw = _rx_oracle_rows(case)
+    d_rssi = 0.0
+    for r in rows:
+        want = stage_ref.rssi(r["chan"])
+        if r["ns"] == 0:
+            assert np.all(np.isnan(r["rssi_ch"])) and np.all(np.isnan(want))
+            continue
+        d_rssi = max(d_rssi, float(np.max(np.abs(r["rssi_ch"] - want))))
+    x, _ = stage_ref.selected_stream([r["chan"] for r in rows], [r["active_chan"] for r in rows])
+    hp, lp = reference_taps()
+    b0, b1, a1 = (np.float32(v) for v in (0.507301437230636, 0.507301437230636, 0.014602874461272194))
+    lpc, au, pcm = stage_ref.audio(x, hp, None, 1.0, b0, b1, a1)
+    audio = np.concatenate([r["audio"] for r in rows])
+    ctin = np.concatenate([r["ctcss_in"] for r in rows])
+    assert audio.shape == au.shape
+    rms, worst = stage_ref.check_res(audio, au, RX_AUDIO_TOL_RMS, RX_AUDIO_TOL_MAX)
+    stage_ref.check_pcm(np.concatenate([r["pcm"] for r in rows]), au, float(np.max(np.abs(audio - au))))
+    ct = stage_ref.dc_block_real(lpc, 0.0005)
+    e_ct = float(np.max(np.abs(ctin - ct)) / np.sqrt(np.mean(x ** 2)))
+    print("MEASURED oracle %s: rssi %.2e dB, audio %.2e rms / %.2e sample, ctcss_in %.2e" % (case, d_rssi, rms, worst, e_ct))
+    assert d_rssi < RX_RSSI_TOL_DB and e_ct < RX_CTCSS_TOL

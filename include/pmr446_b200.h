@@ -78,6 +78,11 @@ typedef struct {
   int deemph_fir;          /* APP_FIR_DEEMPH build of the reference: the 101-tap FIR de-emphasis (:122-135, :458, :896)
                               instead of the one-pole filter; served by the fast-convolution audio kernel only
                               (batch API; composite responses up to 1000 taps) */
+  unsigned dsd_rate;       /* batch API: rate (Hz) of the per-channel DSD feed (dsd_audio / dsd_pcm), 0 = off (default).  Every
+                              channel's discriminator output through msresamp_rrrf_create((float)dsd_rate / channel_width,
+                              resamp_as), as src/dsd_in.c:104,170 does for its one carrier: 48000 feeds DSD.  The plan must be
+                              one arbitrary stage in [1, 2] then one half-band x2 stage with m <= 10 (rates in (2, 4] at 60 dB),
+                              else create() fails with PMR446_EINVAL; the receiver refuses any non-zero value */
 } pmr446_config;
 
 /* Per-call outputs.  Any pointer may be NULL.  For *_execute() these are HOST pointers, for
@@ -100,6 +105,13 @@ typedef struct {
   float *rssi;             /* [n_streams][M] 20 log10(mean |chan|) over this call's ns frames, dB */
   float *chan_edge;        /* [n_streams][M][2] complex: channel sample of this call's first and last frame
                               (what freqdem's r_prime needs when the active channel changes, :866, :881) */
+  /* Per-channel DSD feed, cfg.dsd_rate != 0 only (else requesting it is PMR446_EINVAL): a call that completes frames [F0, F1)
+   * writes 2 (k(F1) - k(F0)) samples per row, k(F) = ceil(F 2^24 / step) resampler outputs, pmr446_batch_last_dsd() of them. */
+  float *dsd_audio;        /* [n_streams][M][dsd_ld] msresamp_rrrf output of the channel's discriminator (dsd_in's out_buf) */
+  int16_t *dsd_pcm;        /* [n_streams][M][dsd_ld] (int16_t)trunc(dsd_audio * 32767) SATURATED at full scale, unlike dsd446_*'s
+                              wrapping cast: an empty channel's discriminator swings to +-1 and the interpolator overshoots it,
+                              which a wrapping cast would turn into full-scale spikes of the wrong sign in DSD's input */
+  long long dsd_ld;        /* samples per row, >= pmr446_batch_max_dsd() covers any call */
 } pmr446_outputs;
 
 typedef struct pmr446_batch pmr446_batch;
@@ -126,14 +138,20 @@ int pmr446_batch_execute_device(pmr446_batch *b, const void *iq, long long iq_st
 int pmr446_batch_gather_channel(pmr446_batch *b, const int *channel, float *demod_out, long long ld, void *cuda_stream);
 /* Kernels launched by the last execute call (for the benchmark's gpu_launches field). */
 int pmr446_batch_last_launches(const pmr446_batch *b);
+/* Largest per-row dsd_audio / dsd_pcm count one call can return (for sizing dsd_ld); 0 with dsd_rate = 0. */
+long long pmr446_batch_max_dsd(const pmr446_batch *b);
+/* dsd_audio / dsd_pcm samples per row the last execute call wrote (summed over the host-buffer call's time slices; 0 when the
+ * call requested neither).  Host state, valid as soon as the call returns, like pmr446_batch_last_launches. */
+long long pmr446_batch_last_dsd(const pmr446_batch *b);
 /* Resets all filter state to stream start (t = 0). */
 int pmr446_batch_reset(pmr446_batch *b);
 /* Per-kernel device timing (CUDA events on the launch stream).  After pmr446_batch_timing(b, 1)
  * every execute call records events around its kernels; pmr446_batch_get_timings() waits for the
  * device and returns, per tag, the accumulated milliseconds and the number of intervals since
  * timing was enabled.  Tags: 1 DC-blocker carry, 2-4 half-band/resampler cascade launches,
- * 5 history save, 6 channelizer+discriminator, 7 audio FIR chain, 8 waterfall, 9 output gathers. */
-#define PMR446_TIMING_TAGS 10
+ * 5 history save, 6 channelizer+discriminator, 7 audio FIR chain, 8 waterfall, 9 output gathers, 10 dsd tap (dsd_audio /
+ * dsd_pcm). */
+#define PMR446_TIMING_TAGS 11
 int pmr446_batch_timing(pmr446_batch *b, int enable);
 int pmr446_batch_get_timings(pmr446_batch *b, double *total_ms, long long *count, int n);
 

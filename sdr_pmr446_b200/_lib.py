@@ -22,14 +22,16 @@ class Config(C.Structure):
                 ("resamp_as", C.c_float), ("dc_alpha", C.c_float), ("kf", C.c_float), ("audio_gain", C.c_float),
                 ("lowpass", C.c_int), ("waterfall", C.c_uint), ("max_chunk", C.c_uint),
                 ("hp_taps", C.c_void_p), ("hp_len", C.c_uint), ("lp_taps", C.c_void_p), ("lp_len", C.c_uint),
-                ("deemph_b0", C.c_float), ("deemph_b1", C.c_float), ("deemph_a1", C.c_float), ("deemph_fir", C.c_int)]
+                ("deemph_b0", C.c_float), ("deemph_b1", C.c_float), ("deemph_a1", C.c_float), ("deemph_fir", C.c_int),
+                ("dsd_rate", C.c_uint)]
 
 
 class Outputs(C.Structure):
     """pmr446_outputs (include/pmr446_b200.h)."""
     _fields_ = [("res", C.c_void_p), ("res_ld", C.c_longlong), ("chan", C.c_void_p), ("demod", C.c_void_p),
                 ("lpcomp", C.c_void_p), ("audio", C.c_void_p), ("pcm", C.c_void_p), ("ld", C.c_longlong),
-                ("ascii", C.c_void_p), ("peak", C.c_void_p), ("psd", C.c_void_p), ("rssi", C.c_void_p), ("chan_edge", C.c_void_p)]
+                ("ascii", C.c_void_p), ("peak", C.c_void_p), ("psd", C.c_void_p), ("rssi", C.c_void_p), ("chan_edge", C.c_void_p),
+                ("dsd_audio", C.c_void_p), ("dsd_pcm", C.c_void_p), ("dsd_ld", C.c_longlong)]
 
 
 class RxConfig(C.Structure):
@@ -67,7 +69,7 @@ class DsdOutputs(C.Structure):
 EXPORTS = [
     "pmr446_default_config", "pmr446_batch_create", "pmr446_batch_destroy", "pmr446_batch_max_res",
     "pmr446_batch_max_ns", "pmr446_batch_execute", "pmr446_batch_execute_device", "pmr446_batch_last_launches",
-    "pmr446_batch_gather_channel",
+    "pmr446_batch_gather_channel", "pmr446_batch_max_dsd", "pmr446_batch_last_dsd",
     "pmr446_batch_reset", "pmr446_last_error", "pmr446_host_alloc", "pmr446_host_free", "pmr446_measure_fp32_peak", "pmr446_batch_timing",
     "pmr446_batch_get_timings",
     "pmr446_rx_default_config", "pmr446_receiver_create", "pmr446_receiver_destroy", "pmr446_receiver_max_ns",
@@ -108,6 +110,10 @@ def lib():
         L.pmr446_batch_execute_device.argtypes = [C.c_void_p, C.c_void_p, C.c_longlong, C.c_uint, C.POINTER(Outputs),
                                                   C.POINTER(C.c_uint), C.POINTER(C.c_uint), C.c_void_p]
         L.pmr446_batch_last_launches.argtypes = [C.c_void_p]
+        L.pmr446_batch_max_dsd.argtypes = [C.c_void_p]
+        L.pmr446_batch_max_dsd.restype = C.c_longlong
+        L.pmr446_batch_last_dsd.argtypes = [C.c_void_p]
+        L.pmr446_batch_last_dsd.restype = C.c_longlong
         L.pmr446_batch_gather_channel.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]
         L.pmr446_batch_reset.argtypes = [C.c_void_p]
         L.pmr446_last_error.restype = C.c_char_p

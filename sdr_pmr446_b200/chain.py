@@ -16,6 +16,7 @@ from . import _lib
 from ._lib import FMT_CF32, FMT_CS8, FMT_CS16, FMT_CU8, Config, Outputs, bytes_per_sample, check, lib  # noqa: F401 (formats re-exported)
 
 PMR_OUTPUTS = ("res", "chan", "demod", "lpcomp", "audio", "pcm")
+DSD_OUTPUTS = ("dsd_audio", "dsd_pcm")   # per-channel DSD feed, PmrBatch(dsd_rate=48000)
 
 
 def _samples(iq, bps):
@@ -49,6 +50,7 @@ class PmrBatch:
         self.M = self.cfg.num_channels
         self.max_res = lib().pmr446_batch_max_res(self.h)
         self.max_ns = lib().pmr446_batch_max_ns(self.h)
+        self.max_dsd = lib().pmr446_batch_max_dsd(self.h)
         self.bytes_per_sample = bytes_per_sample(self.cfg.in_fmt)
 
     def close(self):
@@ -68,8 +70,13 @@ class PmrBatch:
     def last_launches(self):
         return lib().pmr446_batch_last_launches(self.h)
 
+    @property
+    def last_dsd(self):
+        """dsd_audio / dsd_pcm samples per row the last execute call wrote."""
+        return lib().pmr446_batch_last_dsd(self.h)
+
     TIMING_TAGS = ("start", "dc_carry", "cascade0", "cascade1", "cascade2", "hist_save", "channelize", "audio", "waterfall",
-                   "gather")
+                   "gather", "dsd")
 
     def timing(self, enable=True):
         check(lib().pmr446_batch_timing(self.h, int(enable)), "pmr446_batch_timing")
@@ -112,6 +119,11 @@ class PmrBatch:
             bufs["rssi"] = np.zeros((S, M), np.float32)
         if "chan_edge" in want:
             bufs["chan_edge"] = np.zeros((S, M, 2), np.complex64)
+        out.dsd_ld = self.max_dsd
+        if "dsd_audio" in want:
+            bufs["dsd_audio"] = np.zeros((S, M, self.max_dsd), np.float32)
+        if "dsd_pcm" in want:
+            bufs["dsd_pcm"] = np.zeros((S, M, self.max_dsd), np.int16)
         for k, v in bufs.items():
             setattr(out, k, v.ctypes.data)
         ny, ns = C.c_uint(0), C.c_uint(0)
@@ -121,6 +133,8 @@ class PmrBatch:
         for k, v in bufs.items():
             if k == "res":
                 r[k] = v[:, :ny.value]
+            elif k in DSD_OUTPUTS:
+                r[k] = v[:, :, :self.last_dsd]
             elif k in ("chan", "demod", "lpcomp", "audio", "pcm"):
                 r[k] = v[:, :, :ns.value]
             else:
@@ -147,12 +161,14 @@ class PmrBatch:
     # ---- device buffers (torch tensors are only used as device memory + stream handles) ---------
     def execute_device(self, iq, n, outputs, stream_ptr=None):
         """iq: torch CUDA tensor [S, row] (uint8 or complex64/float32 view); outputs: dict name ->
-        torch CUDA tensor laid out as in include/pmr446_b200.h plus 'ld'/'res_ld'.  Asynchronous."""
+        torch CUDA tensor laid out as in include/pmr446_b200.h plus 'ld'/'res_ld'/'dsd_ld'.  Asynchronous; the DSD feed's
+        count per row is last_dsd once the call returns."""
         import torch
         out = Outputs()
         out.ld = int(outputs.get("ld", self.max_ns))
         out.res_ld = int(outputs.get("res_ld", self.max_res))
-        for k in ("res", "chan", "demod", "lpcomp", "audio", "pcm", "ascii", "peak", "psd", "rssi", "chan_edge"):
+        out.dsd_ld = int(outputs.get("dsd_ld", self.max_dsd))
+        for k in ("res", "chan", "demod", "lpcomp", "audio", "pcm", "ascii", "peak", "psd", "rssi", "chan_edge") + DSD_OUTPUTS:
             t = outputs.get(k)
             if t is not None:
                 setattr(out, k, t.data_ptr())

@@ -169,7 +169,7 @@ __global__ void hist_update_kernel(SrcView v, T* dst, long long dst_stride_elts,
 // Optional per-kernel timing with CUDA events recorded on the launch stream (bench.py's roofline).
 // mark(tag) closes the interval since the previous mark and attributes it to `tag`.
 enum { TM_START = 0, TM_DC = 1, TM_CASCADE0 = 2, TM_CASCADE1 = 3, TM_CASCADE2 = 4, TM_HIST = 5, TM_CHANNELIZE = 6, TM_AUDIO = 7,
-       TM_WATERFALL = 8, TM_GATHER = 9, TM_NTAGS = 10 };
+       TM_WATERFALL = 8, TM_GATHER = 9, TM_DSD = 10, TM_NTAGS = 11 };
 struct Timer {
   bool enabled = false;
   std::vector<cudaEvent_t> ev;

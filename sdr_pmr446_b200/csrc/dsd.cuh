@@ -8,6 +8,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "audio_fft.cuh"   // pcm_sat
+
 namespace pmr {
 
 // fm[n] = arg(conj(x[n-1]) x[n]) * ref, n in [n0, n1); x[-1] = 0
@@ -127,20 +129,23 @@ static __global__ void __launch_bounds__(256) dsd_interp_kernel(DsdInterpParams 
 // ---- dsd_backend_kernel: the arbitrary resampler, the half-band interpolator and the s16 cast in ONE launch (batched dsd path) ----
 // dsd_arb_kernel gathers a 64-byte filter-bank row per OUTPUT (lanes of a warp hit ~25 different rows: 16-25 L1 wavefronts per
 // 128-bit load; 0.32 ms per 1024-stream second for 24.6 M outputs) and hands z to dsd_interp_kernel through a ring in HBM (0.17 ms,
-// one output pair per thread).  Here a block owns KB consecutive resampler outputs of one stream:
+// one output pair per thread).  Here a block owns KB consecutive resampler outputs of one row (a dsd_in stream, or one (stream,
+// channel) row of the batch chain's discriminator ring for its per-channel DSD feed):
 //  phase 1: thread (j, g) computes outputs ks + j + P (g + G n), n = 0, 1, ...  P is the (near-)period of the phase sequence found on
 //   the host (x1.92 = 48/25: P = 48, after which the 24-bit phase has moved by -16/2^24), so a thread's bank row changes once in
 //   ~4000 outputs and its 14 taps stay in REGISTERS; the input window comes from shared memory (lanes read neighbouring words).  The
 //   2m - 1 outputs in front of the block are recomputed from the discriminator ring instead of being read back: no z ring at all.
 //  phase 2: out[2k] = z[k - m], out[2k + 1] = sum_j h[j] z[k - j] from shared memory, float / s16 pair stores.
-// Same operations in the same order as the two kernels it replaces (bit-identical results).
+// Same operations in the same order as the two kernels it replaces (bit-identical results).  The s16 cast wraps like dsd_in's
+// (SAT = false) or saturates (SAT = true, pcm_sat: the batch chain's DSD feed).
 constexpr int DSB_T = 192;                 // threads per block
 constexpr int DSB_KB = 1536;               // resampler outputs per block (3072 output samples)
 constexpr int DSB_HIST = 19;               // 2 m - 1 for the largest half-band (m = 10)
 constexpr int DSB_XS = DSB_KB + DSB_HIST + 32;   // staged inputs: rate >= 1 means at most one input per output, + 13 of filter history
 struct DsdBackendParams {
-  const float* fm;           // discriminator ring [n_streams][fm_stride]
+  const float* fm;           // discriminator ring [rows][fm_stride]
   long long fm_stride, fm_mask;
+  int tiles;                 // blocks per row: block b serves row b / tiles (rows folded into gridDim.x: no 65535-row limit)
   long long k0, k1;          // resampler outputs of this call
   unsigned step;             // 2^24 / rate of the arbitrary stage, in [2^23, 2^24]
   int bits;                  // log2(number of bank rows)
@@ -148,23 +153,33 @@ struct DsdBackendParams {
   const float* pfb;          // [rows][16] bank, newest tap first
   int m;                     // half-band semi-length
   float hb[20];
-  float* audio;              // optional [n_streams][out_ld]
-  short* pcm;                // optional [n_streams][out_ld]
+  float* audio;              // optional [rows][out_ld]
+  short* pcm;                // optional [rows][out_ld]
   long long out_ld;
 };
-template <int M>   // half-band semi-length known at compile time (unrolled taps from the constant bank), 0 = use p.m
+// (Near-)period P <= DSB_T of the arbitrary stage's phase sequence: after P outputs the 24-bit phase is back within 1/16 of a bank
+// row, so a thread that computes outputs k, k + P, k + 2P, ... keeps its bank row in registers (x1.92: P = 48, drift -16 / 2^24).
+inline int dsd_arb_period(unsigned step, unsigned bits) {
+  const unsigned tol = (1u << (24 - bits)) / 16;
+  for (int P = 1; P <= DSB_T; P++) {
+    const unsigned r = (unsigned)(((unsigned long long)P * step) & 0xffffffu);
+    if (r <= tol || (1u << 24) - r <= tol) return P;
+  }
+  return 32;
+}
+template <int M, bool SAT>   // M: half-band semi-length known at compile time (unrolled taps from the constant bank), 0 = use p.m
 static __global__ void __launch_bounds__(DSB_T) dsd_backend_kernel(DsdBackendParams p) {
   __shared__ float xs[DSB_XS];
   __shared__ float zs[DSB_KB + DSB_HIST];
-  const int s = blockIdx.y;
-  const long long kb = p.k0 + (long long)blockIdx.x * DSB_KB;
+  const long long s = blockIdx.x / p.tiles;
+  const long long kb = p.k0 + (long long)(blockIdx.x % p.tiles) * DSB_KB;
   if (kb >= p.k1) return;
   const long long kend = kb + DSB_KB < p.k1 ? kb + DSB_KB : p.k1;
   const int m = M ? M : p.m;
   const int hist = 2 * m - 1;
   const long long ks = kb - hist;                       // first z this block needs (z[k < 0] = 0)
   const long long kf = ks > 0 ? ks : 0;
-  const float* f = p.fm + (long long)s * p.fm_stride;
+  const float* f = p.fm + s * p.fm_stride;
   const long long i_first = (long long)(((unsigned long long)kf * p.step) >> 24) - 13;
   const long long i_last = (long long)(((unsigned long long)(kend - 1) * p.step) >> 24);
   const int count = (int)(i_last - i_first + 1);        // <= KB + hist + 14 for step <= 2^24 (checked on the host)
@@ -211,13 +226,13 @@ static __global__ void __launch_bounds__(DSB_T) dsd_backend_kernel(DsdBackendPar
     } else {
       for (int j = 0; j < 2 * m; j++) y1 = fmaf(p.hb[j], q[-j], y1);
     }
-    const long long o = (long long)s * p.out_ld + 2 * (k - p.k0);
+    const long long o = s * p.out_ld + 2 * (k - p.k0);
     if (p.audio) {
       p.audio[o] = y0;
       p.audio[o + 1] = y1;
     }
     if (p.pcm) {
-      const short a = (short)__float2int_rz(y0 * 32767.0f), b = (short)__float2int_rz(y1 * 32767.0f);
+      const short a = SAT ? pcm_sat(y0) : (short)__float2int_rz(y0 * 32767.0f), b = SAT ? pcm_sat(y1) : (short)__float2int_rz(y1 * 32767.0f);
       if (((o | (long long)(uintptr_t)p.pcm >> 1) & 1) == 0) {
         *(short2*)(p.pcm + o) = make_short2(a, b);
       } else {

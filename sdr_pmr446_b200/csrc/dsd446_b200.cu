@@ -71,15 +71,7 @@ extern "C" int dsd446_batch_create(const dsd446_config* cfg, dsd446_batch** out)
   if (!b->up.interp || b->up.stages != 1 || b->up.sub_len != 14 || b->up.m[0] > 10)
     return fail(PMR446_EINVAL, "up-sampler plan not built: need one half-band stage after the arbitrary resampler (2 < rate <= 4)");
   if (b->up.step < (1u << 23) || b->up.step > (1u << 24)) return fail(PMR446_EINVAL, "up-sampler plan not built: arbitrary stage outside (1, 2]");
-  {  // smallest P <= DSB_T after which the 24-bit phase is back within 1/16 of a bank row: a thread that computes outputs k, k + P,
-     // k + 2P, ... keeps its bank row in registers (x1.92: P = 48, drift -16 / 2^24 per period)
-    const unsigned tol = (1u << (24 - b->up.bits)) / 16;
-    b->arb_period = 32;
-    for (int P = 1; P <= DSB_T; P++) {
-      const unsigned r = (unsigned)(((unsigned long long)P * b->up.step) & 0xffffffu);
-      if (r <= tol || (1u << 24) - r <= tol) { b->arb_period = P; break; }
-    }
-  }
+  b->arb_period = dsd_arb_period(b->up.step, b->up.bits);
   b->max_res = b->fe.max_out_per_chunk();
   const long long max_z = (long long)design::arb_outputs_after((uint64_t)b->max_res, b->up.step) + 2;
   b->max_out = 2 * max_z;
@@ -163,9 +155,10 @@ extern "C" int dsd446_batch_execute_device(dsd446_batch* b, const void* iq, long
     bp.audio = out->audio;
     bp.pcm = out->pcm;
     bp.out_ld = out->out_ld;
-    dim3 g((unsigned)((k1 - k0 + DSB_KB - 1) / DSB_KB), S);
-    if (bp.m == 10) dsd_backend_kernel<10><<<g, DSB_T, 0, st>>>(bp);   // the reference's 60 dB plan
-    else dsd_backend_kernel<0><<<g, DSB_T, 0, st>>>(bp);
+    bp.tiles = (int)((k1 - k0 + DSB_KB - 1) / DSB_KB);
+    const unsigned g = (unsigned)((long long)bp.tiles * S);
+    if (bp.m == 10) dsd_backend_kernel<10, false><<<g, DSB_T, 0, st>>>(bp);   // the reference's 60 dB plan
+    else dsd_backend_kernel<0, false><<<g, DSB_T, 0, st>>>(bp);
     launches++;
   }
   b->launches = launches;

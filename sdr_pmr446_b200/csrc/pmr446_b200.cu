@@ -24,6 +24,7 @@
 #include "common_host.hpp"
 #include "frontend_host.hpp"
 #include "design.hpp"
+#include "dsd.cuh"
 #include "frontend.cuh"
 #include "spectrum.cuh"
 
@@ -59,8 +60,14 @@ struct pmr446_batch {
   DevBuf d_resp, d_aftw;
   // waterfall
   Waterfall wf;
+  // per-channel DSD feed (cfg.dsd_rate != 0): msresamp_rrrf over every discriminator row, no state of its own
+  design::MsresampPlan dsd;
+  DevBuf d_dsd_pfb;          // [npfb][16] bank rows of the arbitrary stage
+  int dsd_period = 32;       // (near-)period of its phase sequence (dsd_backend_kernel)
+  long long max_dsd = 0, last_dsd = 0;
   // staging for the host-buffer call
-  DevBuf d_in2[2], d_out_res, d_out_chan, d_out_demod, d_out_lpcomp, d_out_audio, d_out_pcm, d_out_ascii, d_out_peak, d_out_psd;
+  DevBuf d_in2[2], d_out_res, d_out_chan, d_out_demod, d_out_lpcomp, d_out_audio, d_out_pcm, d_out_ascii, d_out_peak, d_out_psd, d_out_dsd_audio,
+      d_out_dsd_pcm;
   long long max_res = 0, max_ns = 0;
   cudaStream_t own_stream = nullptr, copy_stream = nullptr, out_stream = nullptr;
   cudaEvent_t ev_out = nullptr;
@@ -164,6 +171,23 @@ extern "C" int pmr446_batch_create(const pmr446_config* cfg, pmr446_batch** out)
   // demod ring: history for the audio FIR halo + one chunk
   b->demod_cap = next_pow2(b->max_ns + std::max(AU_MAXHALO + AU_MAXLEAD, AF_N) + 64);
   if ((rc = b->d_demod.alloc_zero((size_t)S * M * b->demod_cap * sizeof(float)))) return rc;
+  if (cfg->dsd_rate) {
+    // the plan and its checks of dsd446_batch_create (src/dsd_in.c:104)
+    b->dsd = design::msresamp_plan((float)cfg->dsd_rate / cfg->channel_width, cfg->resamp_as);
+    if (!b->dsd.interp || b->dsd.stages != 1 || b->dsd.sub_len != 14 || b->dsd.m[0] > 10)
+      return fail(PMR446_EINVAL, "dsd_rate: need one half-band stage after the arbitrary resampler (2 < dsd_rate / channel_width <= 4)");
+    if (b->dsd.step < (1u << 23) || b->dsd.step > (1u << 24)) return fail(PMR446_EINVAL, "dsd_rate: arbitrary stage outside [1, 2]");
+    // a call's first output reaches back 2 m - 1 outputs and 13 taps: at most 13 + 2 m frames behind its first frame
+    if (b->demod_cap < b->max_ns + 13 + 2 * (long long)b->dsd.m[0] + 1) return fail(PMR446_EINVAL, "internal: discriminator ring too short for dsd_rate");
+    b->max_dsd = 2 * ((long long)design::arb_outputs_after((uint64_t)b->max_ns, b->dsd.step) + 1);
+    b->dsd_period = dsd_arb_period(b->dsd.step, b->dsd.bits);
+    if ((b->max_dsd / 2 + DSB_KB - 1) / DSB_KB * (long long)S * M > 0x7fffffffLL) return fail(PMR446_EINVAL, "dsd_rate: too many rows for one launch");
+    std::vector<float> rows((size_t)b->dsd.npfb * 16, 0.0f);
+    for (unsigned i = 0; i < b->dsd.npfb; i++)
+      for (unsigned k = 0; k < 14; k++) rows[(size_t)i * 16 + k] = b->dsd.pfb[(size_t)i * 14 + k];
+    if ((rc = b->d_dsd_pfb.alloc(rows.size() * 4))) return rc;
+    cudaMemcpy(b->d_dsd_pfb.p, rows.data(), rows.size() * 4, cudaMemcpyHostToDevice);
+  }
 
   // audio filters; the de-emphasis pole's warm-up also sets the length of its impulse response below
   if ((rc = b->au.init(*cfg))) return rc;
@@ -255,6 +279,8 @@ extern "C" int pmr446_batch_destroy(pmr446_batch* b) {
 extern "C" long long pmr446_batch_max_res(const pmr446_batch* b) { return b ? b->max_res : 0; }
 extern "C" long long pmr446_batch_max_ns(const pmr446_batch* b) { return b ? b->max_ns : 0; }
 extern "C" int pmr446_batch_last_launches(const pmr446_batch* b) { return b ? b->launches : 0; }
+extern "C" long long pmr446_batch_max_dsd(const pmr446_batch* b) { return b ? b->max_dsd : 0; }
+extern "C" long long pmr446_batch_last_dsd(const pmr446_batch* b) { return b ? b->last_dsd : 0; }
 
 static __global__ void gather_channel_kernel(const float* ring, long long stride, long long mask, int M, long long f0, long long ns, const int* channel,
                                              float* out, long long ld) {
@@ -309,11 +335,19 @@ long long pmr::batch_frames_after(const pmr446_batch* b, unsigned n) {
   return b->fe.outputs_after(b->fe.n_in + (long long)n) / b->M - b->fe.n_out / b->M;
 }
 
+// Resampler outputs of the DSD feed once frames [0, F) exist; a call completing [F0, F1) owns [k(F0), k(F1)).
+static long long dsd_outputs_after(const pmr446_batch* b, long long F) { return (long long)design::arb_outputs_after((uint64_t)F, b->dsd.step); }
+
 // The caller's leading dimensions against the counts of a call of n samples (closed form), before any state advances: a
 // rejected call leaves the handle untouched.
 static int check_ld(const pmr446_batch* b, unsigned n, const pmr446_outputs* out) {
   if (out->res && b->fe.outputs_after(b->fe.n_in + (long long)n) - b->fe.n_out > out->res_ld) return fail(PMR446_ERANGE, "res_ld too small");
   if ((out->chan || out->demod || out->lpcomp || out->audio || out->pcm) && batch_frames_after(b, n) > out->ld) return fail(PMR446_ERANGE, "ld too small");
+  if (out->dsd_audio || out->dsd_pcm) {
+    if (!b->cfg.dsd_rate) return fail(PMR446_EINVAL, "dsd_audio / dsd_pcm need dsd_rate != 0");
+    const long long f0 = b->fe.n_out / b->M, f1 = f0 + batch_frames_after(b, n);
+    if (2 * (dsd_outputs_after(b, f1) - dsd_outputs_after(b, f0)) > out->dsd_ld) return fail(PMR446_ERANGE, "dsd_ld too small");
+  }
   return PMR446_OK;
 }
 
@@ -325,6 +359,7 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
   cudaStream_t st = (cudaStream_t)cuda_stream;
   const int S = b->S;
   b->launches = 0;
+  b->last_dsd = 0;
 
   // ---- validate BEFORE any state advances: a failed call leaves the handle untouched ----------
   const int M = b->M;
@@ -491,6 +526,37 @@ extern "C" int pmr446_batch_execute_device(pmr446_batch* b, const void* iq, long
       b->timer.mark(st, TM_AUDIO);
     }
   }
+  // ---- per-channel DSD feed: msresamp_rrrf (src/dsd_in.c:170-175) over every discriminator row -------------------------------
+  if (ns > 0 && (out->dsd_audio || out->dsd_pcm)) {
+    const long long k0 = dsd_outputs_after(b, f0), k1 = dsd_outputs_after(b, f1);
+    if (k1 > k0) {
+      // dsd_in's back end over every (stream, channel) row of the discriminator ring, s16 saturated
+      DsdBackendParams bp;
+      memset(&bp, 0, sizeof bp);
+      bp.fm = (const float*)b->d_demod.p;
+      bp.fm_stride = b->demod_cap;
+      bp.fm_mask = b->demod_cap - 1;
+      bp.k0 = k0;
+      bp.k1 = k1;
+      bp.step = b->dsd.step;
+      bp.bits = (int)b->dsd.bits;
+      bp.period = b->dsd_period;
+      bp.groups = DSB_T / b->dsd_period;
+      bp.pfb = (const float*)b->d_dsd_pfb.p;
+      bp.m = (int)b->dsd.m[0];
+      for (size_t j = 0; j < b->dsd.hb[0].size() && j < 20; j++) bp.hb[j] = b->dsd.hb[0][j];
+      bp.audio = out->dsd_audio;
+      bp.pcm = out->dsd_pcm;
+      bp.out_ld = out->dsd_ld;
+      bp.tiles = (int)((k1 - k0 + DSB_KB - 1) / DSB_KB);
+      const unsigned g = (unsigned)((long long)bp.tiles * S * M);
+      if (bp.m == 10) dsd_backend_kernel<10, true><<<g, DSB_T, 0, st>>>(bp);   // the 60 dB plan
+      else dsd_backend_kernel<0, true><<<g, DSB_T, 0, st>>>(bp);
+      b->launches++;
+      b->timer.mark(st, TM_DSD);
+    }
+    b->last_dsd = 2 * (k1 - k0);
+  }
   // ---- waterfall on the un-mixed resampler output of this chunk (:910-913) -------------------
   if (b->cfg.waterfall > 0 && (out->ascii || out->peak || out->psd)) {
     rc = b->wf.execute((const float2*)b->fe.out.p, b->fe.out_cap, r0, ny, out->ascii, out->peak, out->psd, st, &b->launches);
@@ -541,19 +607,26 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
   d.psd = stage(W ? out->psd : nullptr, b->d_out_psd, (size_t)S * 4 * W * 4);
   d.rssi = stage(out->rssi, b->d_out_rssi, (size_t)S * M * 4);
   d.chan_edge = stage(out->chan_edge, b->d_out_edge, (size_t)S * M * 2 * 8);
+  const long long dld = b->max_dsd;
+  d.dsd_ld = dld;
+  d.dsd_audio = stage(out->dsd_audio, b->d_out_dsd_audio, (size_t)S * M * dld * 4);
+  d.dsd_pcm = stage(out->dsd_pcm, b->d_out_dsd_pcm, (size_t)S * M * dld * 2);
   if (stage.rc) return stage.rc;
   unsigned ny_tot = 0, ns_tot = 0;
+  long long dsd_tot = 0;
   int launches = 0;
   unsigned off = 0;
   // device -> host copies of a column range of every requested output; with time slices they run on their own stream
   // right behind each slice's kernels, i.e. concurrently with the next slices' host -> device copies (PCIe is duplex)
-  auto back_range = [&](cudaStream_t s2, unsigned y0, unsigned ny_k, unsigned s0, unsigned ns_k) {
+  auto back_range = [&](cudaStream_t s2, unsigned y0, unsigned ny_k, unsigned s0, unsigned ns_k, long long d0, long long nd_k) {
     copy_back(s2, out->res, d.res, out->res_ld, rld, 8, S, y0, ny_k);
     copy_back(s2, out->chan, d.chan, out->ld, ld, 8, (long long)S * M, s0, ns_k);
     copy_back(s2, out->demod, d.demod, out->ld, ld, 4, (long long)S * M, s0, ns_k);
     copy_back(s2, out->lpcomp, d.lpcomp, out->ld, ld, 4, (long long)S * M, s0, ns_k);
     copy_back(s2, out->audio, d.audio, out->ld, ld, 4, (long long)S * M, s0, ns_k);
     copy_back(s2, out->pcm, d.pcm, out->ld, ld, 2, (long long)S * M, s0, ns_k);
+    copy_back(s2, out->dsd_audio, d.dsd_audio, out->dsd_ld, dld, 4, (long long)S * M, d0, nd_k);
+    copy_back(s2, out->dsd_pcm, d.dsd_pcm, out->dsd_ld, dld, 2, (long long)S * M, d0, nd_k);
   };
   for (unsigned k = 0; k == 0 || off < n; k++) {
     const unsigned len = std::min(sub, n - off);
@@ -570,6 +643,8 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
     if (dk.lpcomp) dk.lpcomp += ns_tot;
     if (dk.audio) dk.audio += ns_tot;
     if (dk.pcm) dk.pcm += ns_tot;
+    if (dk.dsd_audio) dk.dsd_audio += dsd_tot;   // a slice's columns start where the previous slices' k(F) left off
+    if (dk.dsd_pcm) dk.dsd_pcm += dsd_tot;
     unsigned ny = 0, ns = 0;
     rc = pmr446_batch_execute_device(b, b->d_in2[buf].p, pitch, len, &dk, &ny, &ns, st);
     if (rc) return rc;
@@ -578,15 +653,17 @@ extern "C" int pmr446_batch_execute(pmr446_batch* b, const void* iq, long long i
     if (K > 1) {
       CUDA_TRY(cudaEventRecord(b->ev_out, st));
       CUDA_TRY(cudaStreamWaitEvent(b->out_stream, b->ev_out, 0));
-      back_range(b->out_stream, ny_tot, ny, ns_tot, ns);
+      back_range(b->out_stream, ny_tot, ny, ns_tot, ns, dsd_tot, b->last_dsd);
     }
     ny_tot += ny;
     ns_tot += ns;
+    dsd_tot += b->last_dsd;
     off += len;
   }
   b->launches = launches;
+  b->last_dsd = dsd_tot;
   const unsigned ny = ny_tot, ns = ns_tot;
-  if (K == 1) back_range(st, 0, ny, 0, ns);
+  if (K == 1) back_range(st, 0, ny, 0, ns, 0, dsd_tot);
   copy_back(st, out->rssi, d.rssi, M, M, 4, S, 0, M);
   copy_back(st, out->chan_edge, d.chan_edge, 2 * M, 2 * M, 8, S, 0, 2 * M);
   if (W) {

@@ -60,6 +60,7 @@ extern "C" int pmr446_receiver_create(const pmr446_rx_config* cfg, pmr446_receiv
   if ((cfg->channel_mask & all) == 0) return fail(PMR446_EINVAL, "channel_mask enables no channel");   // :725
   if (cfg->ctcss_block < 1) return fail(PMR446_EINVAL, "ctcss_block must be positive");
   if (cfg->chain.deemph_fir) return fail(PMR446_EINVAL, "the receiver runs the direct-form audio chain: deemph_fir is not available");
+  if (cfg->chain.dsd_rate) return fail(PMR446_EINVAL, "the receiver has no per-channel DSD feed: dsd_rate must be 0");
   pmr446_batch* batch = nullptr;
   int rc = pmr446_batch_create(&cfg->chain, &batch);
   if (rc) return rc;
